@@ -211,5 +211,7 @@ def accumulators(device) -> torch.Tensor:
 
 
 def f32c(t):
-    """contiguous fp32 view/copy (the reference forces boxes to fp32, structures/boxes.py:21)."""
-    return t.detach().to(torch.float32).contiguous()
+    """contiguous fp32 view/copy (the reference forces boxes to fp32, structures/boxes.py:21), 16-byte aligned as the
+    box kernels require: a view can be contiguous and still start inside a row, e.g. rois[:, 1:5] of a single roi."""
+    t = t.detach().to(torch.float32).contiguous()
+    return t if t.data_ptr() % 16 == 0 else t.clone()

@@ -413,7 +413,8 @@ def rpn_losses(anchors: torch.Tensor, pred_logits: torch.Tensor, gt_labels: torc
     loc = dense_box_regression_loss(anchors, pred_deltas, gt_boxes, pos, weights, scale_clamp,
                                     box_reg_loss_type, smooth_l1_beta)
     valid = gt_labels >= 0
-    obj = F.binary_cross_entropy_with_logits(pred_logits[valid], gt_labels[valid].to(torch.float32), reduction="sum")
+    # targets in the logits' dtype: with fp32 targets, BCE-with-logits computes a float64 run in fp32
+    obj = F.binary_cross_entropy_with_logits(pred_logits[valid], gt_labels[valid].to(pred_logits.dtype), reduction="sum")
     norm = batch_size_per_image * n
     return {"cls_loss": obj / norm * loss_weight[0], "loc_loss": loc / norm * loss_weight[1],
             "num_pos": int(pos.sum()), "num_neg": int((gt_labels == 0).sum())}
@@ -563,9 +564,10 @@ def yolo_loss(head: torch.Tensor, labels: torch.Tensor, matched: torch.Tensor, g
     for i in range(n):
         lab = labels[i]
         valid = lab >= 0
-        wgt = torch.where(lab == 1, torch.ones(()), torch.full((), lambda_noobj))
+        # weights and BCE targets in the head's dtype, so that a float64 run is float64 throughout
+        wgt = torch.where(lab == 1, torch.ones((), dtype=head.dtype), torch.full((), lambda_noobj, dtype=head.dtype))
         obj = obj + (wgt[valid] * F.binary_cross_entropy_with_logits(
-            t[i, valid, 4], lab[valid].float(), reduction="none")).sum()
+            t[i, valid, 4], lab[valid].to(head.dtype), reduction="none")).sum()
         p = torch.nonzero(lab == 1, as_tuple=True)[0]
         if p.numel() == 0:
             continue
@@ -581,6 +583,6 @@ def yolo_loss(head: torch.Tensor, labels: torch.Tensor, matched: torch.Tensor, g
         tp = t[i, p]
         loc = loc + ((torch.sigmoid(tp[:, 0]) - xs) ** 2 + (torch.sigmoid(tp[:, 1]) - ys) ** 2
                      + (tp[:, 2] - tw_t) ** 2 + (tp[:, 3] - th_t) ** 2).sum()
-        onehot = F.one_hot(gc, C).float()
+        onehot = F.one_hot(gc, C).to(head.dtype)
         cls = cls + F.binary_cross_entropy_with_logits(cl[i, cell], onehot, reduction="sum")
     return {"loc_loss": loc * lambda_coord / norm, "obj_loss": obj / norm, "cls_loss": cls / norm}

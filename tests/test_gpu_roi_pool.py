@@ -100,6 +100,18 @@ def test_roi_align_single_level_and_edges(det):
         det.ROIPooler([0.25], 0, 7, "Bilinear")
 
 
+def test_roi_align_single_roi(det):
+    """One roi: rois[:, 1:5] is then a contiguous view that starts 4 bytes into the row; the boxes handed to the kernel
+    must still be 16-byte aligned."""
+    g = gen(13)
+    feat = torch.randn(1, 5, 16, 16, generator=g)
+    rois = torch.tensor([[0, 3.0, 2.0, 40.0, 50.0]])
+    ra = det.ROIAlign((3, 4), 0.25, 0, True)
+    got = ra(feat.cuda(), rois.cuda())
+    torch.testing.assert_close(got.cpu(), torchvision.ops.roi_align(feat, rois, (3, 4), 0.25, 0, True), rtol=1e-5,
+                               atol=1e-5)
+
+
 @pytest.mark.parametrize("ptype,sampling_ratio", [("ROIAlignV2", 0), ("ROIAlign", 2)])
 def test_roi_pooler_backward_matches_torchvision_cpu(det, ptype, sampling_ratio):
     """Gradients w.r.t. every pyramid level against autograd through torchvision's CPU roi_align (atomics: 1e-5)."""

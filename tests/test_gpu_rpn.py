@@ -23,30 +23,74 @@ def O():
     return ref_torch
 
 
-def _heads(n, img, g, scale=1.0):
-    obj = [torch.randn(n, 3, img // s, img // s, generator=g) for s in STRIDES]
-    dlt = [torch.randn(n, 12, img // s, img // s, generator=g) * scale for s in STRIDES]
+def _heads(n, img, g, scale=1.0, a=3):
+    obj = [torch.randn(n, a, img // s, img // s, generator=g) for s in STRIDES]
+    dlt = [torch.randn(n, 4 * a, img // s, img // s, generator=g) * scale for s in STRIDES]
     return obj, dlt
 
 
-def _oracle_decode(O, obj, dlt, img, weights=(1.0, 1.0, 1.0, 1.0)):
-    cells = [O.cell_anchors(s, RATIOS[0]) for s in SIZES]
+def _oracle_decode(O, obj, dlt, img, weights=(1.0, 1.0, 1.0, 1.0), sizes=SIZES, ratios=RATIOS):
+    ratios = ratios * len(sizes) if len(ratios) == 1 else ratios
+    cells = [O.cell_anchors(s, r) for s, r in zip(sizes, ratios)]
     anchors = O.grid_anchors([(img // s, img // s) for s in STRIDES], STRIDES, cells, 0.0)
     lg, dl = zip(*[O.head_to_hwa(o, d) for o, d in zip(obj, dlt)])
     props = O.decode_proposals(anchors, list(dl), weights)
     return anchors, list(lg), list(dl), props
 
 
-@pytest.mark.parametrize("img", [448, 224])
-def test_decode_heads_matches_oracle(det, O, img):
-    g = gen(img)
-    obj, dlt = _heads(3, img, g, 0.5)
-    rpn = det.RegionProposalNetwork(STRIDES, SIZES, RATIOS)
-    logits, boxes, sizes = rpn.decode_heads([o.cuda() for o in obj], [d.cuda() for d in dlt])
-    anchors, lg, dl, props = _oracle_decode(O, obj, dlt, img)
-    assert sizes == [a.shape[0] for a in anchors]
-    if img == 448:
-        assert sum(sizes) == 50127
+RPN_FLAT_MAX_A = 4  # kRpnFlatMaxA, csrc/box_ops.cu:278
+
+
+def rpn_decode_launches(a, level_hw):
+    """The launches det_rpn_decode makes (box_ops.cu:541-556, :521-528): one flat launch for the whole pyramid when
+    a <= RPN_FLAT_MAX_A, else one det_rpn_decode_level launch per level, with 16-byte loads ("vec") when the level's
+    planes are whole 16-byte tiles and scalar loads otherwise (aligned heads assumed, as torch allocates them)."""
+    if a <= RPN_FLAT_MAX_A:
+        return ["flat"]
+    return ["vec" if (h * w) % 4 == 0 else "scalar" for h, w in level_hw]
+
+
+_ANCHOR_SETS = {  # anchors per position: (sizes per level, ratios)
+    1: (SIZES, [[1.0]]),
+    2: (SIZES, [[0.5, 2.0]]),
+    4: ([[s[0], s[0] * 1.5] for s in SIZES], [[0.5, 2.0]]),
+    9: ([[s[0], s[0] * 1.26, s[0] * 1.59] for s in SIZES], RATIOS),
+}
+
+
+@pytest.mark.parametrize("img,a,weights", [
+    pytest.param(448, 3, (1.0, 1.0, 1.0, 1.0), id="448"),
+    pytest.param(224, 3, (1.0, 1.0, 1.0, 1.0), id="224"),
+    pytest.param(224, 1, (10.0, 10.0, 5.0, 5.0), id="224-a1"),
+    pytest.param(224, 2, (10.0, 10.0, 5.0, 5.0), id="224-a2"),
+    pytest.param(448, 4, (10.0, 10.0, 5.0, 5.0), id="448-a4"),
+    pytest.param(448, 9, (10.0, 10.0, 5.0, 5.0), id="448-a9"),
+])
+def test_decode_heads_matches_oracle(det, O, img, a, weights):
+    """a = 3 (the reference's anchors) and other anchor sets: a <= 4 decodes the pyramid in one flat launch, a = 9
+    (three sizes x three ratios) falls back to one launch per level (vec and scalar forms).  With box weights
+    (10, 10, 5, 5) some width / height deltas exceed scale_clamp."""
+    sizes, ratios = _ANCHOR_SETS[a] if a != 3 else (SIZES, RATIOS)
+    launches = rpn_decode_launches(a, [(img // s, img // s) for s in STRIDES])
+    if a <= RPN_FLAT_MAX_A:
+        assert launches == ["flat"]
+    else:
+        assert {"vec", "scalar"} <= set(launches)
+    g = gen(img + (0 if a == 3 else 100 * a))
+    obj, dlt = _heads(3, img, g, 0.5 if weights[2] == 1.0 else 4.0, a)
+    rpn = det.RegionProposalNetwork(STRIDES, sizes, ratios, box2box_weights=weights)
+    if weights[2] != 1.0:
+        for d in dlt:  # beyond scale_clamp (log(1000/16) = 4.14 after dividing by 5), both signs of dx / dy
+            d[:, 2::4, ::3, ::2] = 30.0
+            d[:, 3::4, 1::3, ::2] = 25.0
+            d[:, 0::4, ::2, 1::3] *= -3.0
+        assert any(float(d[:, 2::4].max()) / weights[2] > rpn.box2box_transform.scale_clamp for d in dlt)
+    logits, boxes, lsz = rpn.decode_heads([o.cuda() for o in obj], [d.cuda() for d in dlt])
+    anchors, lg, dl, props = _oracle_decode(O, obj, dlt, img, weights, sizes, ratios)
+    assert lsz == [x.shape[0] for x in anchors]
+    assert sum(lsz) == a * sum((img // s) ** 2 for s in STRIDES)
+    if img == 448 and a == 3:
+        assert sum(lsz) == 50127
     assert torch.equal(logits.cpu(), torch.cat(lg, 1))          # pure layout change: bit-exact
     assert_boxes_close(boxes.cpu(), torch.cat(props, 1), rtol=1e-5)
 
