@@ -33,6 +33,13 @@ extern "C" {
 
 #define DET_ABI_VERSION 3
 
+/* element type of a detection head passed to the *_typed entry points.  A 16-bit head is widened to fp32 as it is
+ * loaded (exact) and then takes the fp32 path's instructions: every output is bit-identical to the fp32 entry point
+ * fed the same head converted to fp32.  Outputs keep their documented dtypes. */
+#define DET_DTYPE_F32 0
+#define DET_DTYPE_BF16 1
+#define DET_DTYPE_F16 2
+
 #if defined(__GNUC__)
 #define DET_API __attribute__((visibility("default")))
 #else
@@ -105,6 +112,13 @@ typedef struct det_rpn_level {
 DET_API int det_rpn_decode(const det_rpn_level_t* levels_host, int num_levels, int n, int a, float offset, float wx, float wy,
                    float ww, float wh, float scale_clamp, float* logits_out, float* boxes_out, int64_t out_img_stride,
                    void* stream);
+/* det_rpn_decode on a head of element type head_dtype (DET_DTYPE_*): the objectness and deltas pointers of every level
+ * point at elements of that type (the `reserved` field stays unread).  A level streams with vector loads when h*w % 4 == 0
+ * and both planes are aligned to 4 elements; others ride along with scalar loads.  Unknown head_dtype: DET_ERR_BAD_ARG.
+ * det_rpn_decode is this call with DET_DTYPE_F32. */
+DET_API int det_rpn_decode_typed(const det_rpn_level_t* levels_host, int num_levels, int n, int a, float offset, float wx,
+                         float wy, float ww, float wh, float scale_clamp, float* logits_out, float* boxes_out,
+                         int64_t out_img_stride, int head_dtype, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------
  * (3) batched, category-partitioned NMS -- replaces batched_nms, python/src/utils.py:96 (and through it
@@ -162,6 +176,15 @@ DET_API int det_yolo_decode_nms_i32(const float* head, int n, int s, int b, int 
                             float* dense_boxes, float* dense_conf, float* dense_scores, int64_t max_det,
                             int32_t* det_flat32, float* det_boxes, float* det_scores, int32_t* det_count, void* stream);
 
+/* both of the above for a head of element type head_dtype (DET_DTYPE_*), aligned to 4 elements: det_flat is int64
+ * (index_bytes 8) or int32 (index_bytes 4).  Unknown head_dtype or index_bytes: DET_ERR_BAD_ARG.  det_yolo_decode_nms
+ * and det_yolo_decode_nms_i32 are this call with DET_DTYPE_F32. */
+DET_API int det_yolo_decode_nms_typed(const void* head, int head_dtype, int n, int s, int b, int c, int img_h, int img_w,
+                              const float* priors, float scale_clamp, int clip, float score_thresh,
+                              double iou_threshold, int mode, float* dense_boxes, float* dense_conf, float* dense_scores,
+                              int64_t max_det, void* det_flat, int index_bytes, float* det_boxes, float* det_scores,
+                              int32_t* det_count, void* stream);
+
 /* dense anchor head (YOLOv3-style, NCHW): head (n, a*(5+c), h, w) -> boxes (n,h*w*a,4), best score, best class.
  * anchors_wh (a,2) device.  Output slots as in det_rpn_decode_level. */
 DET_API int det_dense_decode_level(const float* head, int n, int a, int c, int h, int w, int stride, const float* anchors_wh,
@@ -180,6 +203,13 @@ typedef struct det_dense_level {
 } det_dense_level_t;
 DET_API int det_dense_decode(const det_dense_level_t* levels_host, int num_levels, int n, int a, int c, float scale_clamp,
                      float* boxes_out, float* score_out, int64_t* class_out, int64_t out_img_stride, void* stream);
+/* det_dense_decode on a head of element type head_dtype (DET_DTYPE_*): every level's `head` points at elements of that
+ * type (the `reserved` field stays unread).  The one-launch path needs every level h*w % 4 == 0 and heads aligned to 4
+ * elements; otherwise each level takes its own launch (scalar loads where needed) -- same results.  Unknown
+ * head_dtype: DET_ERR_BAD_ARG.  det_dense_decode is this call with DET_DTYPE_F32. */
+DET_API int det_dense_decode_typed(const det_dense_level_t* levels_host, int num_levels, int n, int a, int c,
+                           float scale_clamp, float* boxes_out, float* score_out, int64_t* class_out,
+                           int64_t out_img_stride, int head_dtype, void* stream);
 
 /* Dense anchor head as a detector runs it (BASELINE configs[3]): decode -> score > score_thresh -> per-class NMS ->
  * top max_det, two launches for the whole batch and no dense output.  Specification: oracle/ref_torch.py
@@ -204,6 +234,14 @@ DET_API int det_dense_detect(const det_dense_level_t* levels_host, int num_level
                      float score_thresh, double iou_threshold, int mode, int gate, int64_t cand_cap, int64_t max_det,
                      int64_t* det_idx, float* det_boxes, float* det_scores, int64_t* det_classes, int32_t* det_count,
                      int32_t* overflow_flag, void* workspace, int64_t workspace_bytes, void* stream);
+/* det_dense_detect on a head of element type head_dtype (DET_DTYPE_*), as in det_dense_decode_typed.  Limits: every level
+ * h*w % 4 == 0 and heads aligned to 4 elements (else DET_ERR_UNSUPPORTED).  Unknown head_dtype: DET_ERR_BAD_ARG.
+ * det_dense_detect is this call with DET_DTYPE_F32. */
+DET_API int det_dense_detect_typed(const det_dense_level_t* levels_host, int num_levels, int n, int a, int c,
+                           float scale_clamp, float score_thresh, double iou_threshold, int mode, int gate,
+                           int64_t cand_cap, int64_t max_det, int64_t* det_idx, float* det_boxes, float* det_scores,
+                           int64_t* det_classes, int32_t* det_count, int32_t* overflow_flag, void* workspace,
+                           int64_t workspace_bytes, int head_dtype, void* stream);
 
 /* Row-ordered candidate compaction and the final gather of the UNFUSED detector path (det_dense_decode ->
  * det_threshold_compact -> det_nms_batched -> det_gather_detections): the exact route for images that overflow

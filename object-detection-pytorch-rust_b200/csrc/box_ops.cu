@@ -210,9 +210,9 @@ __global__ void grid_anchors_kernel(const float4* __restrict__ cell, int a, int 
 // ------------------------------------------------------------------------------------------------
 constexpr int kMaxCellAnchors = 16;
 
-template <int V>
+template <int V, typename T = float>
 __global__ void __launch_bounds__(256)
-rpn_decode_level_kernel(const float* __restrict__ obj, const float* __restrict__ deltas, int n, int a, int h, int w,
+rpn_decode_level_kernel(const T* __restrict__ obj, const T* __restrict__ deltas, int n, int a, int h, int w,
                         int stride, float offset, const float4* __restrict__ cell, CodecWeights wt,
                         float scale_clamp, float* __restrict__ logits_out, float4* __restrict__ boxes_out,
                         int64_t out_img_stride, int64_t out_offset) {
@@ -225,8 +225,8 @@ rpn_decode_level_kernel(const float* __restrict__ obj, const float* __restrict__
     const int img = blockIdx.y;
     if (g >= groups) return;
     const int64_t p0 = g * V;
-    const float* obj_img = obj + (int64_t)img * a * hw;
-    const float* del_img = deltas + (int64_t)img * a * 4 * hw;
+    const T* obj_img = obj + (int64_t)img * a * hw;
+    const T* del_img = deltas + (int64_t)img * a * 4 * hw;
     float* lo = logits_out + (int64_t)img * out_img_stride + out_offset;
     float4* bo = boxes_out + (int64_t)img * out_img_stride + out_offset;
     float sx[V], sy[V];
@@ -239,17 +239,18 @@ rpn_decode_level_kernel(const float* __restrict__ obj, const float* __restrict__
     for (int ai = 0; ai < a; ++ai) {
         float lg[V], d[4][V];
         if (V == 4) {
-            const float4 l4 = ld_stream(reinterpret_cast<const float4*>(obj_img + ai * hw + p0));
+            using HV = typename Head<T>::vec;
+            const float4 l4 = ld4_stream<T>(reinterpret_cast<const HV*>(obj_img + ai * hw + p0));
             lg[0] = l4.x; lg[1] = l4.y; lg[2] = l4.z; lg[3] = l4.w;
 #pragma unroll
             for (int c = 0; c < 4; ++c) {
-                const float4 q = ld_stream(reinterpret_cast<const float4*>(del_img + (ai * 4 + c) * hw + p0));
+                const float4 q = ld4_stream<T>(reinterpret_cast<const HV*>(del_img + (ai * 4 + c) * hw + p0));
                 d[c][0] = q.x; d[c][1] = q.y; d[c][2] = q.z; d[c][3] = q.w;
             }
         } else {
-            lg[0] = ld_stream(obj_img + ai * hw + p0);
+            lg[0] = ld1_stream(obj_img + ai * hw + p0);
 #pragma unroll
-            for (int c = 0; c < 4; ++c) d[c][0] = ld_stream(del_img + (ai * 4 + c) * hw + p0);
+            for (int c = 0; c < 4; ++c) d[c][0] = ld1_stream(del_img + (ai * 4 + c) * hw + p0);
         }
         const float4 ca = s_cell[ai];
 #pragma unroll
@@ -280,11 +281,11 @@ constexpr int kRpnTilePos = 128;
 constexpr int kRpnFlatWarps = 8;
 
 struct RpnLevelDev {
-    const float* obj;
-    const float* deltas;
+    const void* obj;     // elements of the kernel's head type T
+    const void* deltas;
     const float4* cell;
     int w, hw, tiles;  // tiles of 128 positions per image
-    int stride, vec;   // vec: planes are whole 16-byte tiles (hw % 4 == 0, aligned heads)
+    int stride, vec;   // vec: planes are whole 4-element vectors (hw % 4 == 0, heads aligned to 4 elements)
     int64_t out_offset;
 };
 
@@ -299,7 +300,9 @@ struct RpnFlatArgs {
     float4* boxes_out;
 };
 
+template <typename T = float>
 __global__ void __launch_bounds__(kRpnFlatWarps * 32) rpn_decode_flat_kernel(const __grid_constant__ RpnFlatArgs g) {
+    using HV = typename Head<T>::vec;
     extern __shared__ __align__(16) unsigned char rpn_smem[];
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const long long tile = (long long)blockIdx.x * kRpnFlatWarps + wid;
@@ -318,8 +321,8 @@ __global__ void __launch_bounds__(kRpnFlatWarps * 32) rpn_decode_flat_kernel(con
                    (size_t)wid * kRpnTilePos * A;
     const int p0 = pos0 + lane * 4;
     if (lane * 4 < npos) {  // vec levels (hw % 4 == 0): a lane's 4 positions are all inside or all outside
-        const float* obj_img = L.obj + (int64_t)img * A * L.hw + p0;
-        const float* del_img = L.deltas + (int64_t)img * A * 4 * L.hw + p0;
+        const T* obj_img = static_cast<const T*>(L.obj) + (int64_t)img * A * L.hw + p0;
+        const T* del_img = static_cast<const T*>(L.deltas) + (int64_t)img * A * 4 * L.hw + p0;
         float sx[4], sy[4];
 #pragma unroll
         for (int v = 0; v < 4; ++v) {
@@ -330,23 +333,23 @@ __global__ void __launch_bounds__(kRpnFlatWarps * 32) rpn_decode_flat_kernel(con
         for (int ai = 0; ai < A; ++ai) {
             float4 l4, q[4];
             if (L.vec) {
-                l4 = ld_stream(reinterpret_cast<const float4*>(obj_img + (int64_t)ai * L.hw));
+                l4 = ld4_stream<T>(reinterpret_cast<const HV*>(obj_img + (int64_t)ai * L.hw));
 #pragma unroll
-                for (int c = 0; c < 4; ++c) q[c] = ld_stream(reinterpret_cast<const float4*>(del_img + (int64_t)(ai * 4 + c) * L.hw));
+                for (int c = 0; c < 4; ++c) q[c] = ld4_stream<T>(reinterpret_cast<const HV*>(del_img + (int64_t)(ai * 4 + c) * L.hw));
             } else {
                 // a level whose planes are not 16-byte tiles (h*w not a multiple of 4, e.g. the 7x7 level of a 448^2
                 // pyramid, or an unaligned view): scalar loads, positions past the plane read as 0 and are never written
-                auto ld4 = [&](const float* pl) {
+                auto ld4s = [&](const T* pl) {
                     float4 r = make_float4(0.f, 0.f, 0.f, 0.f);
-                    if (p0 + 0 < L.hw) r.x = pl[0];
-                    if (p0 + 1 < L.hw) r.y = pl[1];
-                    if (p0 + 2 < L.hw) r.z = pl[2];
-                    if (p0 + 3 < L.hw) r.w = pl[3];
+                    if (p0 + 0 < L.hw) r.x = ld1(pl + 0);
+                    if (p0 + 1 < L.hw) r.y = ld1(pl + 1);
+                    if (p0 + 2 < L.hw) r.z = ld1(pl + 2);
+                    if (p0 + 3 < L.hw) r.w = ld1(pl + 3);
                     return r;
                 };
-                l4 = ld4(obj_img + (int64_t)ai * L.hw);
+                l4 = ld4s(obj_img + (int64_t)ai * L.hw);
 #pragma unroll
-                for (int c = 0; c < 4; ++c) q[c] = ld4(del_img + (int64_t)(ai * 4 + c) * L.hw);
+                for (int c = 0; c < 4; ++c) q[c] = ld4s(del_img + (int64_t)(ai * 4 + c) * L.hw);
             }
             const float lg[4] = {l4.x, l4.y, l4.z, l4.w};
             const float d0[4] = {q[0].x, q[0].y, q[0].z, q[0].w}, d1[4] = {q[1].x, q[1].y, q[1].z, q[1].w};
@@ -500,10 +503,15 @@ int det_grid_anchors(const float* cell_anchors, int a, int h, int w, int stride,
     return DET_OK;
 }
 
-int det_rpn_decode_level(const float* objectness, const float* deltas, int n, int a, int h, int w, int stride,
-                         float offset, const float* cell_anchors, float wx, float wy, float ww, float wh,
-                         float scale_clamp, float* logits_out, float* boxes_out, int64_t out_img_stride,
-                         int64_t out_offset, void* stream) {
+}  // extern "C"
+
+// The entry points below have C linkage through their declarations in det_b200.h; the per-type implementations
+// between them are C++ templates.
+template <typename T>
+static int rpn_decode_level_t(const T* objectness, const T* deltas, int n, int a, int h, int w, int stride,
+                              float offset, const float* cell_anchors, float wx, float wy, float ww, float wh,
+                              float scale_clamp, float* logits_out, float* boxes_out, int64_t out_img_stride,
+                              int64_t out_offset, void* stream) {
     DET_CHECK_ARG(n >= 0 && a >= 1 && a <= kMaxCellAnchors && h >= 0 && w >= 0, "bad size (a <= 16)");
     const int64_t hw = (int64_t)h * w;
     if (n == 0 || hw == 0) return DET_OK;
@@ -518,23 +526,32 @@ int det_rpn_decode_level(const float* objectness, const float* deltas, int n, in
     auto cell = reinterpret_cast<const float4*>(cell_anchors);
     auto bo = reinterpret_cast<float4*>(boxes_out);
     cudaStream_t st = as_stream(stream);
-    const bool vec = (hw % 4 == 0) && aligned16(objectness) && aligned16(deltas);
+    const bool vec = (hw % 4 == 0) && aligned_to(objectness, 4 * sizeof(T)) && aligned_to(deltas, 4 * sizeof(T));
     if (vec) {
         dim3 grid((unsigned)((hw / 4 + 255) / 256), (unsigned)n);
-        rpn_decode_level_kernel<4><<<grid, 256, 0, st>>>(objectness, deltas, n, a, h, w, stride, offset, cell, wt,
+        rpn_decode_level_kernel<4, T><<<grid, 256, 0, st>>>(objectness, deltas, n, a, h, w, stride, offset, cell, wt,
                                                          scale_clamp, logits_out, bo, out_img_stride, out_offset);
     } else {
         dim3 grid((unsigned)((hw + 255) / 256), (unsigned)n);
-        rpn_decode_level_kernel<1><<<grid, 256, 0, st>>>(objectness, deltas, n, a, h, w, stride, offset, cell, wt,
+        rpn_decode_level_kernel<1, T><<<grid, 256, 0, st>>>(objectness, deltas, n, a, h, w, stride, offset, cell, wt,
                                                          scale_clamp, logits_out, bo, out_img_stride, out_offset);
     }
     DET_LAUNCH_OK("rpn_decode_level_kernel");
     return DET_OK;
 }
 
-int det_rpn_decode(const det_rpn_level_t* levels_host, int num_levels, int n, int a, float offset, float wx, float wy,
-                   float ww, float wh, float scale_clamp, float* logits_out, float* boxes_out, int64_t out_img_stride,
-                   void* stream) {
+int det_rpn_decode_level(const float* objectness, const float* deltas, int n, int a, int h, int w, int stride,
+                         float offset, const float* cell_anchors, float wx, float wy, float ww, float wh,
+                         float scale_clamp, float* logits_out, float* boxes_out, int64_t out_img_stride,
+                         int64_t out_offset, void* stream) {
+    return rpn_decode_level_t<float>(objectness, deltas, n, a, h, w, stride, offset, cell_anchors, wx, wy, ww, wh,
+                                     scale_clamp, logits_out, boxes_out, out_img_stride, out_offset, stream);
+}
+
+template <typename T>
+static int rpn_decode_t(const det_rpn_level_t* levels_host, int num_levels, int n, int a, float offset, float wx, float wy,
+                        float ww, float wh, float scale_clamp, float* logits_out, float* boxes_out, int64_t out_img_stride,
+                        void* stream) {
     DET_CHECK_ARG(num_levels >= 0 && n >= 0 && a >= 1 && a <= kMaxCellAnchors, "bad size (a <= 16)");
     if (num_levels == 0 || n == 0) return DET_OK;
     DET_CHECK_ARG(levels_host && logits_out && boxes_out, "null pointer");
@@ -551,9 +568,10 @@ int det_rpn_decode(const det_rpn_level_t* levels_host, int num_levels, int n, in
         DET_CHECK_ARG(out_img_stride >= L.out_offset + hw * a, "output slot out of range");
         // (levels whose planes are not 16-byte tiles ride along with scalar loads: they are the small ones)
         const bool flat = flat_ok && f.num_levels < kRpnFlatMaxLevels && hw < (1ll << 30) && aligned16(L.cell_anchors);
-        const bool vec_ok = hw % 4 == 0 && aligned16(L.objectness) && aligned16(L.deltas);
+        const bool vec_ok = hw % 4 == 0 && aligned_to(L.objectness, 4 * sizeof(T)) && aligned_to(L.deltas, 4 * sizeof(T));
         if (!flat) {  // this level takes its own launch: same results
-            const int rc = det_rpn_decode_level(L.objectness, L.deltas, n, a, L.h, L.w, L.stride, offset, L.cell_anchors, wx,
+            const int rc = rpn_decode_level_t<T>(reinterpret_cast<const T*>(L.objectness),
+                                                 reinterpret_cast<const T*>(L.deltas), n, a, L.h, L.w, L.stride, offset, L.cell_anchors, wx,
                                                 wy, ww, wh, scale_clamp, logits_out, boxes_out, out_img_stride,
                                                 L.out_offset, stream);
             if (rc != DET_OK) return rc;
@@ -577,11 +595,23 @@ int det_rpn_decode(const det_rpn_level_t* levels_host, int num_levels, int n, in
     const long long blocks = (tb + kRpnFlatWarps - 1) / kRpnFlatWarps;
     DET_CHECK_ARG(blocks < (1ll << 31), "too many positions");
     const size_t smem = (size_t)kRpnFlatWarps * kRpnTilePos * a * (sizeof(float4) + sizeof(float));
-    cudaError_t e = cudaFuncSetAttribute(rpn_decode_flat_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(rpn_decode_flat_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(rpn_decode_flat_kernel)");
-    rpn_decode_flat_kernel<<<(unsigned)blocks, kRpnFlatWarps * 32, smem, as_stream(stream)>>>(f);
+    rpn_decode_flat_kernel<T><<<(unsigned)blocks, kRpnFlatWarps * 32, smem, as_stream(stream)>>>(f);
     DET_LAUNCH_OK("rpn_decode_flat_kernel");
     return DET_OK;
 }
 
-}  // extern "C"
+int det_rpn_decode(const det_rpn_level_t* levels_host, int num_levels, int n, int a, float offset, float wx, float wy,
+                   float ww, float wh, float scale_clamp, float* logits_out, float* boxes_out, int64_t out_img_stride,
+                   void* stream) {
+    return rpn_decode_t<float>(levels_host, num_levels, n, a, offset, wx, wy, ww, wh, scale_clamp, logits_out, boxes_out,
+                               out_img_stride, stream);
+}
+
+int det_rpn_decode_typed(const det_rpn_level_t* levels_host, int num_levels, int n, int a, float offset, float wx,
+                         float wy, float ww, float wh, float scale_clamp, float* logits_out, float* boxes_out,
+                         int64_t out_img_stride, int head_dtype, void* stream) {
+    DET_HEAD_DISPATCH(head_dtype, rpn_decode_t, levels_host, num_levels, n, a, offset, wx, wy, ww, wh, scale_clamp,
+                      logits_out, boxes_out, out_img_stride, stream);
+}

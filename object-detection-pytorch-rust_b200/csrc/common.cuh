@@ -3,6 +3,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <math.h>
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include "../../include/det_b200.h"
 
 namespace det {
@@ -27,7 +29,21 @@ int cuda_fail(cudaError_t e, const char* what);
 
 static inline cudaStream_t as_stream(void* s) { return reinterpret_cast<cudaStream_t>(s); }
 static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+static inline bool aligned_to(const void* p, unsigned bytes) { return (reinterpret_cast<uintptr_t>(p) & (bytes - 1u)) == 0; }
 int sm_count();
+
+// calls FN<T>(args...) with T the element type named by DET_DTYPE_* `dtype`; an unknown code is DET_ERR_BAD_ARG before
+// any CUDA call
+#define DET_HEAD_DISPATCH(dtype, FN, ...)                                               \
+    do {                                                                                \
+        switch (dtype) {                                                                \
+            case DET_DTYPE_F32: return FN<float>(__VA_ARGS__);                          \
+            case DET_DTYPE_BF16: return FN<__nv_bfloat16>(__VA_ARGS__);                 \
+            case DET_DTYPE_F16: return FN<__half>(__VA_ARGS__);                         \
+        }                                                                               \
+        det::set_error("bad argument: unknown head_dtype %d", (int)(dtype));            \
+        return DET_ERR_BAD_ARG;                                                         \
+    } while (0)
 
 // largest float f with (double)f <= thr: then for every float v, ((double)v > thr) == (v > f).
 // torchvision's CPU NMS compares the fp32 IoU against a *double* threshold.
@@ -88,6 +104,47 @@ __device__ __forceinline__ void st_stream(float4* p, float4 v) { __stcs(p, v); }
 __device__ __forceinline__ void st_stream(float* p, float v) { __stcs(p, v); }
 __device__ __forceinline__ float4 ld_stream(const float4* p) { return __ldcs(p); }
 __device__ __forceinline__ float ld_stream(const float* p) { return __ldcs(p); }
+
+// ---- head element types (DET_DTYPE_*): a bf16 or fp16 head is widened to fp32 as it is loaded -- exact -- and the
+// kernels then run the same fp32 instructions as for an fp32 head.  Head<T>::vec holds 4 consecutive elements (16 bytes
+// for fp32, 8 bytes for the 16-bit types; the element at the lower address is in the low half of each 32-bit word).
+template <typename T> struct Head;
+template <> struct Head<float> {
+    using vec = float4;
+    static __device__ __forceinline__ float4 f32(const float4 v) { return v; }
+    static __device__ __forceinline__ float f32(const float x) { return x; }
+};
+template <> struct Head<__nv_bfloat16> {
+    using vec = uint2;
+    static __device__ __forceinline__ float f32(const unsigned short b) { return __bfloat162float(__ushort_as_bfloat16(b)); }
+    static __device__ __forceinline__ float f32(const __nv_bfloat16 x) { return __bfloat162float(x); }
+    static __device__ __forceinline__ float4 f32(const uint2 v) {
+        return make_float4(f32((unsigned short)(v.x & 0xffffu)), f32((unsigned short)(v.x >> 16)),
+                           f32((unsigned short)(v.y & 0xffffu)), f32((unsigned short)(v.y >> 16)));
+    }
+};
+template <> struct Head<__half> {
+    using vec = uint2;
+    static __device__ __forceinline__ float f32(const unsigned short b) { return __half2float(__ushort_as_half(b)); }
+    static __device__ __forceinline__ float f32(const __half x) { return __half2float(x); }
+    static __device__ __forceinline__ float4 f32(const uint2 v) {
+        return make_float4(f32((unsigned short)(v.x & 0xffffu)), f32((unsigned short)(v.x >> 16)),
+                           f32((unsigned short)(v.y & 0xffffu)), f32((unsigned short)(v.y >> 16)));
+    }
+};
+// 4 consecutive head elements as fp32: streaming (read-once) and plain (re-read) forms
+template <typename T>
+__device__ __forceinline__ float4 ld4_stream(const typename Head<T>::vec* p) { return Head<T>::f32(__ldcs(p)); }
+template <typename T>
+__device__ __forceinline__ float4 ld4(const typename Head<T>::vec* p) { return Head<T>::f32(*p); }
+// one head element as fp32
+__device__ __forceinline__ float ld1_stream(const float* p) { return __ldcs(p); }
+template <typename T>
+__device__ __forceinline__ float ld1_stream(const T* p) {
+    return Head<T>::f32(__ldcs(reinterpret_cast<const unsigned short*>(p)));
+}
+template <typename T>
+__device__ __forceinline__ float ld1(const T* p) { return Head<T>::f32(*p); }
 
 __device__ __forceinline__ float box_area(const float4 b) { return (b.z - b.x) * (b.w - b.y); }
 

@@ -33,7 +33,7 @@ constexpr int kMaxLevels = 8;
 constexpr int kModeDense = 0, kModeSelect = 1, kModeSelectGated = 2;
 
 struct DenseLevelDev {
-    const float* head;
+    const void* head;  // elements of the kernel's head type T
     const float2* anchors_wh;
     int w, hw;
     float stride;
@@ -65,8 +65,9 @@ struct FlatArgs {
     int32_t* overflow_flag;  // cleared here (first thread of the grid); the NMS kernel behind this one sets it
 };
 
-template <int MODE, int TH = kFlatThreads>
+template <int MODE, int TH = kFlatThreads, typename T = float>
 __global__ void __launch_bounds__(TH) dense_decode_flat_kernel(const __grid_constant__ FlatArgs g) {
+    using V = typename Head<T>::vec;  // 4 positions of one plane: 16 bytes (fp32) or 8 bytes (bf16 / fp16)
     if (MODE != kModeDense) {
         pdl_trigger();  // det_dense_detect: the NMS kernel's CTAs may move in as SM slots free up
         if (blockIdx.x == 0 && threadIdx.x == 0 && g.overflow_flag) *g.overflow_flag = 0;
@@ -88,11 +89,11 @@ __global__ void __launch_bounds__(TH) dense_decode_flat_kernel(const __grid_cons
     const int grp = (int)(local % groups);
     const int ia = (int)(local / groups);  // image * A + anchor
     const int img = ia / A, ai = ia - img * A;
-    const int plane4 = groups;  // float4 stride between planes
-    const float4* pl = reinterpret_cast<const float4*>(L.head + (int64_t)ia * nch * L.hw) + grp;
-    const float4* pk = pl + (int64_t)5 * plane4;
+    const int plane4 = groups;  // stride between planes, in 4-element vectors
+    const V* pl = reinterpret_cast<const V*>(static_cast<const T*>(L.head) + (int64_t)ia * nch * L.hw) + grp;
+    const V* pk = pl + (int64_t)5 * plane4;
     if (MODE == kModeSelectGated && active) {
-        const float4 q = ld_stream(pl + (int64_t)4 * plane4);
+        const float4 q = ld4_stream<T>(pl + (int64_t)4 * plane4);
         const float thr = g.score_thresh;
         // `!(x > thr)` also holds for NaN: a NaN objectness gives a NaN score, which is no candidate either
         if (!(sigmoidf_dd(q.x) > thr) && !(sigmoidf_dd(q.y) > thr) && !(sigmoidf_dd(q.z) > thr) &&
@@ -108,7 +109,7 @@ __global__ void __launch_bounds__(TH) dense_decode_flat_kernel(const __grid_cons
         for (; k + 8 <= C; k += 8) {
             float4 q[8];
 #pragma unroll
-            for (int i = 0; i < 8; ++i) q[i] = ld_stream(pk + (int64_t)(k + i) * plane4);
+            for (int i = 0; i < 8; ++i) q[i] = ld4_stream<T>(pk + (int64_t)(k + i) * plane4);
 #pragma unroll
             for (int i = 0; i < 8; ++i) {
                 bidx[0] = (q[i].x > best[0]) ? k + i : bidx[0]; best[0] = max_nan(best[0], q[i].x);
@@ -118,7 +119,7 @@ __global__ void __launch_bounds__(TH) dense_decode_flat_kernel(const __grid_cons
             }
         }
         for (; k < C; ++k) {
-            const float4 q = ld_stream(pk + (int64_t)k * plane4);
+            const float4 q = ld4_stream<T>(pk + (int64_t)k * plane4);
             bidx[0] = (q.x > best[0]) ? k : bidx[0]; best[0] = max_nan(best[0], q.x);
             bidx[1] = (q.y > best[1]) ? k : bidx[1]; best[1] = max_nan(best[1], q.y);
             bidx[2] = (q.z > best[2]) ? k : bidx[2]; best[2] = max_nan(best[2], q.z);
@@ -129,7 +130,7 @@ __global__ void __launch_bounds__(TH) dense_decode_flat_kernel(const __grid_cons
         if (best[0] != best[0] || best[1] != best[1] || best[2] != best[2] || best[3] != best[3]) {
             bool found[4] = {false, false, false, false};
             for (int j = 0; j < C; ++j) {
-                const float4 q4 = pk[(int64_t)j * plane4];
+                const float4 q4 = ld4<T>(pk + (int64_t)j * plane4);
                 const float q[4] = {q4.x, q4.y, q4.z, q4.w};
 #pragma unroll
                 for (int v = 0; v < 4; ++v)
@@ -142,7 +143,7 @@ __global__ void __launch_bounds__(TH) dense_decode_flat_kernel(const __grid_cons
         float t[5][4];  // box logits last: they would only occupy registers during the class loop
 #pragma unroll
         for (int j = 0; j < 5; ++j) {
-            const float4 q = ld_stream(pl + (int64_t)j * plane4);
+            const float4 q = ld4_stream<T>(pl + (int64_t)j * plane4);
             t[j][0] = q.x; t[j][1] = q.y; t[j][2] = q.z; t[j][3] = q.w;
         }
         const float2 awh = L.anchors_wh[ai];
@@ -213,9 +214,9 @@ __global__ void __launch_bounds__(TH) dense_decode_flat_kernel(const __grid_cons
 }
 
 // ---- fallback for levels whose h*w is not a multiple of 4 (or an unaligned head): one thread per position, scalar loads
-template <int V>
+template <int V, typename T = float>
 __global__ void __launch_bounds__(256)
-dense_decode_level_kernel(const float* __restrict__ head, int a, int c, int h, int w, float stride,
+dense_decode_level_kernel(const T* __restrict__ head, int a, int c, int h, int w, float stride,
                           const float2* __restrict__ anchors_wh, float scale_clamp, float4* __restrict__ boxes_out,
                           float* __restrict__ score_out, int64_t* __restrict__ class_out, int64_t out_img_stride,
                           int64_t out_offset) {
@@ -234,15 +235,15 @@ dense_decode_level_kernel(const float* __restrict__ head, int a, int c, int h, i
     }
     const int64_t obase = (int64_t)img * out_img_stride + out_offset;
     for (int ai = 0; ai < a; ++ai) {
-        const float* pl = head + ((int64_t)(img * a + ai) * nch) * hw + p0;
+        const T* pl = head + ((int64_t)(img * a + ai) * nch) * hw + p0;
         float t[5][V];
 #pragma unroll
         for (int k = 0; k < 5; ++k) {
             if (V == 4) {
-                const float4 q = ld_stream(reinterpret_cast<const float4*>(pl + k * hw));
+                const float4 q = ld4_stream<T>(reinterpret_cast<const typename Head<T>::vec*>(pl + k * hw));
                 t[k][0] = q.x; t[k][1] = q.y; t[k][2] = q.z; t[k][3] = q.w;
             } else {
-                t[k][0] = ld_stream(pl + k * hw);
+                t[k][0] = ld1_stream(pl + k * hw);
             }
         }
         float best[V];
@@ -257,10 +258,10 @@ dense_decode_level_kernel(const float* __restrict__ head, int a, int c, int h, i
         for (int k = 0; k < c; ++k) {
             float q[V];
             if (V == 4) {
-                const float4 q4 = ld_stream(reinterpret_cast<const float4*>(pl + (int64_t)(5 + k) * hw));
+                const float4 q4 = ld4_stream<T>(reinterpret_cast<const typename Head<T>::vec*>(pl + (int64_t)(5 + k) * hw));
                 q[0] = q4.x; q[1] = q4.y; q[2] = q4.z; q[3] = q4.w;
             } else {
-                q[0] = ld_stream(pl + (int64_t)(5 + k) * hw);
+                q[0] = ld1_stream(pl + (int64_t)(5 + k) * hw);
             }
 #pragma unroll
             for (int v = 0; v < V; ++v) {
@@ -394,17 +395,21 @@ static int launch_detect_nms(const SelectArgs& sel, int n, float thr_f, int mode
                                          det_count, overflow_flag, st);
 }
 
-extern "C" {
-
 #ifdef DET_DEBUG_PHASES
+extern "C" {
 __attribute__((visibility("default"))) int det_debug_read_phases_dense(long long* out_host) {
     return cudaMemcpyFromSymbol(out_host, det::g_phase_clock, sizeof(long long) * 32) == cudaSuccess ? 0 : -4;
 }
 __attribute__((visibility("default"))) int det_debug_read_phase_blocks_dense(long long* out_host) {
     return cudaMemcpyFromSymbol(out_host, det::g_phase_block, sizeof(long long) * 64 * 16) == cudaSuccess ? 0 : -4;
 }
+}  // extern "C"
 #endif
 
+// The entry points below have C linkage through their declarations in det_b200.h; the per-type implementations
+// between them are C++ templates.
+
+template <typename T>
 static int launch_flat(const det_dense_level_t* levels_host, int num_levels, int n, int a, int c, float scale_clamp,
                        float* boxes_out, float* score_out, int64_t* class_out, int64_t out_img_stride, cudaStream_t st,
                        const SelectArgs* sel = nullptr) {
@@ -438,26 +443,31 @@ static int launch_flat(const det_dense_level_t* levels_host, int num_levels, int
     const long long blocks = (tb + th - 1) / th;
     DET_CHECK_ARG(blocks < (1ll << 31), "too many positions");
     if (!sel) {
-        if (th == 256) dense_decode_flat_kernel<kModeDense, 256><<<(unsigned)blocks, 256, 0, st>>>(f);
-        else if (th == 512) dense_decode_flat_kernel<kModeDense, 512><<<(unsigned)blocks, 512, 0, st>>>(f);
-        else dense_decode_flat_kernel<kModeDense><<<(unsigned)blocks, kFlatThreads, 0, st>>>(f);
+        if (th == 256) dense_decode_flat_kernel<kModeDense, 256, T><<<(unsigned)blocks, 256, 0, st>>>(f);
+        else if (th == 512) dense_decode_flat_kernel<kModeDense, 512, T><<<(unsigned)blocks, 512, 0, st>>>(f);
+        else dense_decode_flat_kernel<kModeDense, kFlatThreads, T><<<(unsigned)blocks, kFlatThreads, 0, st>>>(f);
     } else if (sel->mode == kModeSelectGated) {
-        dense_decode_flat_kernel<kModeSelectGated><<<(unsigned)blocks, kFlatThreads, 0, st>>>(f);
+        dense_decode_flat_kernel<kModeSelectGated, kFlatThreads, T><<<(unsigned)blocks, kFlatThreads, 0, st>>>(f);
     } else {
-        if (th == 256) dense_decode_flat_kernel<kModeSelect, 256><<<(unsigned)blocks, 256, 0, st>>>(f);
-        else if (th == 512) dense_decode_flat_kernel<kModeSelect, 512><<<(unsigned)blocks, 512, 0, st>>>(f);
-        else dense_decode_flat_kernel<kModeSelect><<<(unsigned)blocks, kFlatThreads, 0, st>>>(f);
+        if (th == 256) dense_decode_flat_kernel<kModeSelect, 256, T><<<(unsigned)blocks, 256, 0, st>>>(f);
+        else if (th == 512) dense_decode_flat_kernel<kModeSelect, 512, T><<<(unsigned)blocks, 512, 0, st>>>(f);
+        else dense_decode_flat_kernel<kModeSelect, kFlatThreads, T><<<(unsigned)blocks, kFlatThreads, 0, st>>>(f);
     }
     DET_LAUNCH_OK("dense_decode_flat_kernel");
     return DET_OK;
 }
 
 
-static bool level_is_flat(const float* head, int64_t hw) { return hw % 4 == 0 && aligned16(head) && hw < (1ll << 30); }
+// the one-launch kernel reads 4 positions of a plane per vector load: whole vectors per plane, head aligned to 4 elements
+template <typename T>
+static bool level_is_flat(const void* head, int64_t hw) {
+    return hw % 4 == 0 && aligned_to(head, 4 * sizeof(T)) && hw < (1ll << 30);
+}
 
-int det_dense_decode_level(const float* head, int n, int a, int c, int h, int w, int stride, const float* anchors_wh,
-                           float scale_clamp, float* boxes_out, float* score_out, int64_t* class_out,
-                           int64_t out_img_stride, int64_t out_offset, void* stream) {
+template <typename T>
+static int dense_decode_level_t(const T* head, int n, int a, int c, int h, int w, int stride, const float* anchors_wh,
+                                float scale_clamp, float* boxes_out, float* score_out, int64_t* class_out,
+                                int64_t out_img_stride, int64_t out_offset, void* stream) {
     DET_CHECK_ARG(n >= 0 && a >= 1 && c >= 0 && h >= 0 && w >= 0, "bad size");
     const int64_t hw = (int64_t)h * w;
     if (n == 0 || hw == 0) return DET_OK;
@@ -469,13 +479,13 @@ int det_dense_decode_level(const float* head, int n, int a, int c, int h, int w,
         return DET_ERR_ALIGN;
     }
     cudaStream_t st = as_stream(stream);
-    if (level_is_flat(head, hw)) {
+    if (level_is_flat<T>(head, hw)) {
         det_dense_level_t L;
-        L.head = head; L.anchors_wh = anchors_wh; L.h = h; L.w = w; L.stride = stride; L.reserved = 0; L.out_offset = out_offset;
-        return launch_flat(&L, 1, n, a, c, scale_clamp, boxes_out, score_out, class_out, out_img_stride, st);
+        L.head = reinterpret_cast<const float*>(head); L.anchors_wh = anchors_wh; L.h = h; L.w = w; L.stride = stride; L.reserved = 0; L.out_offset = out_offset;
+        return launch_flat<T>(&L, 1, n, a, c, scale_clamp, boxes_out, score_out, class_out, out_img_stride, st);
     }
     dim3 grid((unsigned)((hw + 255) / 256), (unsigned)n);
-    dense_decode_level_kernel<1><<<grid, 256, 0, st>>>(head, a, c, h, w, (float)stride,
+    dense_decode_level_kernel<1, T><<<grid, 256, 0, st>>>(head, a, c, h, w, (float)stride,
                                                        reinterpret_cast<const float2*>(anchors_wh), scale_clamp,
                                                        reinterpret_cast<float4*>(boxes_out), score_out, class_out,
                                                        out_img_stride, out_offset);
@@ -483,8 +493,16 @@ int det_dense_decode_level(const float* head, int n, int a, int c, int h, int w,
     return DET_OK;
 }
 
-int det_dense_decode(const det_dense_level_t* levels_host, int num_levels, int n, int a, int c, float scale_clamp,
-                     float* boxes_out, float* score_out, int64_t* class_out, int64_t out_img_stride, void* stream) {
+int det_dense_decode_level(const float* head, int n, int a, int c, int h, int w, int stride, const float* anchors_wh,
+                           float scale_clamp, float* boxes_out, float* score_out, int64_t* class_out,
+                           int64_t out_img_stride, int64_t out_offset, void* stream) {
+    return dense_decode_level_t<float>(head, n, a, c, h, w, stride, anchors_wh, scale_clamp, boxes_out, score_out,
+                                       class_out, out_img_stride, out_offset, stream);
+}
+
+template <typename T>
+static int dense_decode_t(const det_dense_level_t* levels_host, int num_levels, int n, int a, int c, float scale_clamp,
+                          float* boxes_out, float* score_out, int64_t* class_out, int64_t out_img_stride, void* stream) {
     DET_CHECK_ARG(num_levels >= 0 && n >= 0 && a >= 1 && c >= 0, "bad size");
     if (num_levels == 0 || n == 0) return DET_OK;
     DET_CHECK_ARG(levels_host && boxes_out && score_out && class_out, "null pointer");
@@ -493,18 +511,32 @@ int det_dense_decode(const det_dense_level_t* levels_host, int num_levels, int n
     for (int l = 0; l < num_levels; ++l) {
         const det_dense_level_t& L = levels_host[l];
         DET_CHECK_ARG(L.head && L.anchors_wh && L.h >= 0 && L.w >= 0 && L.out_offset >= 0, "bad level");
-        flat_ok = flat_ok && level_is_flat(L.head, (int64_t)L.h * L.w);
+        flat_ok = flat_ok && level_is_flat<T>(L.head, (int64_t)L.h * L.w);
     }
-    if (flat_ok)  // every level streams with 16-byte loads: one launch for the whole pyramid
-        return launch_flat(levels_host, num_levels, n, a, c, scale_clamp, boxes_out, score_out, class_out, out_img_stride,
+    if (flat_ok)  // every level streams with vector loads: one launch for the whole pyramid
+        return launch_flat<T>(levels_host, num_levels, n, a, c, scale_clamp, boxes_out, score_out, class_out, out_img_stride,
                            as_stream(stream));
     for (int l = 0; l < num_levels; ++l) {
         const det_dense_level_t& L = levels_host[l];
-        const int rc = det_dense_decode_level(L.head, n, a, c, L.h, L.w, L.stride, L.anchors_wh, scale_clamp, boxes_out,
-                                              score_out, class_out, out_img_stride, L.out_offset, stream);
+        const int rc = dense_decode_level_t<T>(reinterpret_cast<const T*>(L.head), n, a, c, L.h, L.w, L.stride,
+                                               L.anchors_wh, scale_clamp, boxes_out, score_out, class_out, out_img_stride,
+                                               L.out_offset, stream);
         if (rc != DET_OK) return rc;
     }
     return DET_OK;
+}
+
+int det_dense_decode(const det_dense_level_t* levels_host, int num_levels, int n, int a, int c, float scale_clamp,
+                     float* boxes_out, float* score_out, int64_t* class_out, int64_t out_img_stride, void* stream) {
+    return dense_decode_t<float>(levels_host, num_levels, n, a, c, scale_clamp, boxes_out, score_out, class_out,
+                                 out_img_stride, stream);
+}
+
+int det_dense_decode_typed(const det_dense_level_t* levels_host, int num_levels, int n, int a, int c, float scale_clamp,
+                           float* boxes_out, float* score_out, int64_t* class_out, int64_t out_img_stride,
+                           int head_dtype, void* stream) {
+    DET_HEAD_DISPATCH(head_dtype, dense_decode_t, levels_host, num_levels, n, a, c, scale_clamp, boxes_out, score_out,
+                      class_out, out_img_stride, stream);
 }
 
 int64_t det_dense_detect_workspace_bytes(int n, int64_t cand_cap) {
@@ -514,10 +546,12 @@ int64_t det_dense_detect_workspace_bytes(int n, int64_t cand_cap) {
 
 int64_t det_dense_detect_counter_bytes(int n) { return n <= 0 ? 0 : (int64_t)n * kCountStride * 4; }
 
-int det_dense_detect(const det_dense_level_t* levels_host, int num_levels, int n, int a, int c, float scale_clamp,
-                     float score_thresh, double iou_threshold, int mode, int gate, int64_t cand_cap, int64_t max_det,
-                     int64_t* det_idx, float* det_boxes, float* det_scores, int64_t* det_classes, int32_t* det_count,
-                     int32_t* overflow_flag, void* workspace, int64_t workspace_bytes, void* stream) {
+template <typename T>
+static int dense_detect_t(const det_dense_level_t* levels_host, int num_levels, int n, int a, int c, float scale_clamp,
+                          float score_thresh, double iou_threshold, int mode, int gate, int64_t cand_cap, int64_t max_det,
+                          int64_t* det_idx, float* det_boxes, float* det_scores, int64_t* det_classes,
+                          int32_t* det_count, int32_t* overflow_flag, void* workspace, int64_t workspace_bytes,
+                          void* stream) {
     DET_CHECK_ARG(num_levels >= 0 && n >= 0 && a >= 1 && c >= 0, "bad size");
     DET_CHECK_ARG(mode >= DET_NMS_AUTO && mode <= DET_NMS_OFFSET_TRICK, "unknown mode");
     DET_CHECK_ARG(cand_cap >= 1 && cand_cap <= 4096, "cand_cap must be in [1, 4096]");
@@ -535,8 +569,9 @@ int det_dense_detect(const det_dense_level_t* levels_host, int num_levels, int n
     for (int l = 0; l < num_levels; ++l) {
         const det_dense_level_t& L = levels_host[l];
         DET_CHECK_ARG(L.head && L.anchors_wh && L.h >= 0 && L.w >= 0 && L.out_offset >= 0, "bad level");
-        if (!level_is_flat(L.head, (int64_t)L.h * L.w)) {
-            set_error("det_dense_detect needs h*w %% 4 == 0 and 16-byte aligned heads (level %d: %d x %d)", l, L.h, L.w);
+        if (!level_is_flat<T>(L.head, (int64_t)L.h * L.w)) {
+            set_error("det_dense_detect needs h*w %% 4 == 0 and heads aligned to 4 elements (level %d: %d x %d)", l, L.h,
+                      L.w);
             return DET_ERR_UNSUPPORTED;
         }
         rows = L.out_offset + (int64_t)L.h * L.w * a > rows ? L.out_offset + (int64_t)L.h * L.w * a : rows;
@@ -573,7 +608,7 @@ int det_dense_detect(const det_dense_level_t* levels_host, int num_levels, int n
         cudaError_t e = cudaMemsetAsync(sel.cand_count, 0, sizeof(int32_t) * (size_t)n * kCountStride, st);
         if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync");
     }
-    int rc = launch_flat(levels_host, num_levels, n, a, c, scale_clamp, nullptr, nullptr, nullptr, rows, st, &sel);
+    int rc = launch_flat<T>(levels_host, num_levels, n, a, c, scale_clamp, nullptr, nullptr, nullptr, rows, st, &sel);
     if (rc != DET_OK) return rc;
     const float thr_f = float_threshold_below(iou_threshold);
     if (cand_cap <= 1024)
@@ -584,6 +619,25 @@ int det_dense_detect(const det_dense_level_t* levels_host, int num_levels, int n
                                        det_count, overflow_flag, st);
     return launch_detect_nms<4096>(sel, n, thr_f, mode, max_det, det_idx, det_boxes, det_scores, det_classes, det_count,
                                    overflow_flag, st);
+}
+
+int det_dense_detect(const det_dense_level_t* levels_host, int num_levels, int n, int a, int c, float scale_clamp,
+                     float score_thresh, double iou_threshold, int mode, int gate, int64_t cand_cap, int64_t max_det,
+                     int64_t* det_idx, float* det_boxes, float* det_scores, int64_t* det_classes, int32_t* det_count,
+                     int32_t* overflow_flag, void* workspace, int64_t workspace_bytes, void* stream) {
+    return dense_detect_t<float>(levels_host, num_levels, n, a, c, scale_clamp, score_thresh, iou_threshold, mode, gate,
+                                 cand_cap, max_det, det_idx, det_boxes, det_scores, det_classes, det_count, overflow_flag,
+                                 workspace, workspace_bytes, stream);
+}
+
+int det_dense_detect_typed(const det_dense_level_t* levels_host, int num_levels, int n, int a, int c, float scale_clamp,
+                           float score_thresh, double iou_threshold, int mode, int gate, int64_t cand_cap,
+                           int64_t max_det, int64_t* det_idx, float* det_boxes, float* det_scores,
+                           int64_t* det_classes, int32_t* det_count, int32_t* overflow_flag, void* workspace,
+                           int64_t workspace_bytes, int head_dtype, void* stream) {
+    DET_HEAD_DISPATCH(head_dtype, dense_detect_t, levels_host, num_levels, n, a, c, scale_clamp, score_thresh,
+                      iou_threshold, mode, gate, cand_cap, max_det, det_idx, det_boxes, det_scores, det_classes, det_count,
+                      overflow_flag, workspace, workspace_bytes, stream);
 }
 
 int det_threshold_compact(const float* boxes, const float* scores, const int64_t* classes, int n, int64_t r,
@@ -621,5 +675,3 @@ int det_gather_detections(const int64_t* keep, const int32_t* keep_counts, int n
     DET_LAUNCH_OK("gather_detections_kernel");
     return DET_OK;
 }
-
-}  // extern "C"

@@ -27,9 +27,9 @@ constexpr int kYoloThreads = 512;
 constexpr int kYoloMaxPred = 1024;
 constexpr int kYoloMaxHead = 6144;
 
-template <int CAP>
+template <int CAP, typename HT = float>
 __global__ void __launch_bounds__(kYoloThreads, 2)
-yolo_decode_nms_kernel(const float* __restrict__ head, const float2* __restrict__ priors, YoloParams prm,
+yolo_decode_nms_kernel(const HT* __restrict__ head, const float2* __restrict__ priors, YoloParams prm,
                        float4* __restrict__ dense_boxes, float* __restrict__ dense_conf,
                        float* __restrict__ dense_scores, int64_t* __restrict__ det_flat,
                        float4* __restrict__ det_boxes, float* __restrict__ det_scores,
@@ -49,18 +49,18 @@ yolo_decode_nms_kernel(const float* __restrict__ head, const float2* __restrict_
     const int img = blockIdx.x;
 
     DET_MARK(0);
-    // ---- stage this image's logits: 16-byte coalesced loads over the aligned interior of its span
+    // ---- stage this image's logits: coalesced 4-element loads over the aligned interior of its span, widened to fp32
     const int64_t g0 = (int64_t)img * S2 * ch, g1 = g0 + (int64_t)S2 * ch;
-    const float4* head4 = reinterpret_cast<const float4*>(head);
+    const typename Head<HT>::vec* head4 = reinterpret_cast<const typename Head<HT>::vec*>(head);
     for (int64_t v = (g0 >> 2) + tid; v < ((g1 + 3) >> 2); v += T) {
         const int64_t base = v << 2;
         if (base >= g0 && base + 4 <= g1) {
-            const float4 q = ld_stream(head4 + v);
+            const float4 q = ld4_stream<HT>(head4 + v);
             float* d = hs + (base - g0);
             d[0] = q.x; d[1] = q.y; d[2] = q.z; d[3] = q.w;
         } else {
             for (int e = 0; e < 4; ++e)
-                if (base + e >= g0 && base + e < g1) hs[base + e - g0] = ld_stream(head + base + e);
+                if (base + e >= g0 && base + e < g1) hs[base + e - g0] = ld1_stream(head + base + e);
         }
     }
     __syncthreads();
@@ -173,33 +173,33 @@ yolo_decode_nms_kernel(const float* __restrict__ head, const float2* __restrict_
     DET_MARK(15);
 }
 
-template <int CAP>
-static int launch_yolo(const float* head, const float* priors, const YoloParams& prm, float* dense_boxes,
+template <int CAP, typename T>
+static int launch_yolo(const T* head, const float* priors, const YoloParams& prm, float* dense_boxes,
                        float* dense_conf, float* dense_scores, int64_t* det_flat, float* det_boxes, float* det_scores,
                        int32_t* det_count, cudaStream_t st) {
     const int S2 = prm.s * prm.s, ch = prm.b * 5 + prm.c, P = S2 * prm.b;
     size_t smem = ((sizeof(SmallSmem<CAP, kYoloThreads>) + 15) / 16) * 16;
     smem += sizeof(float4) * P + sizeof(float) * CAP + sizeof(float) * ((S2 * ch + 3) & ~3) + sizeof(uint32_t) * CAP;
-    cudaError_t e = cudaFuncSetAttribute(yolo_decode_nms_kernel<CAP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(yolo_decode_nms_kernel<CAP, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(yolo_decode_nms_kernel)");
-    yolo_decode_nms_kernel<CAP><<<prm.n, kYoloThreads, smem, st>>>(
+    yolo_decode_nms_kernel<CAP, T><<<prm.n, kYoloThreads, smem, st>>>(
         head, reinterpret_cast<const float2*>(priors), prm, reinterpret_cast<float4*>(dense_boxes), dense_conf,
         dense_scores, det_flat, reinterpret_cast<float4*>(det_boxes), det_scores, det_count);
     DET_LAUNCH_OK("yolo_decode_nms_kernel");
     return DET_OK;
 }
 
-template <int MAXT, int MINB, int CS, int CB, int CC>
-static int launch_yolo_fast(const float* head, const float* priors, const YoloParams& prm, float* dense_boxes,
+template <int MAXT, int MINB, int CS, int CB, int CC, typename T>
+static int launch_yolo_fast(const T* head, const float* priors, const YoloParams& prm, float* dense_boxes,
                             float* dense_conf, float* dense_scores, int64_t* det_flat, float* det_boxes,
                             float* det_scores, int32_t* det_count, cudaStream_t st) {
     const int S2 = prm.s * prm.s, ch = prm.b * 5 + prm.c, P = S2 * prm.b;
     const FastLayout lay(S2, ch, P, prm.c);
     const int warps = prm.c > kFastMinWarps ? prm.c : kFastMinWarps;
-    cudaError_t e = cudaFuncSetAttribute(yolo_fast_kernel<MAXT, MINB, CS, CB, CC>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)lay.bytes);
+    cudaError_t e = cudaFuncSetAttribute(yolo_fast_kernel<MAXT, MINB, CS, CB, CC, T>,
+                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lay.bytes);
     if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(yolo_fast_kernel)");
-    e = launch_pdl(yolo_fast_kernel<MAXT, MINB, CS, CB, CC>, dim3(prm.n), dim3(warps * 32), lay.bytes, st, head,
+    e = launch_pdl(yolo_fast_kernel<MAXT, MINB, CS, CB, CC, T>, dim3(prm.n), dim3(warps * 32), lay.bytes, st, head,
                    reinterpret_cast<const float2*>(priors), prm, reinterpret_cast<float4*>(dense_boxes), dense_conf,
                    dense_scores, det_flat, reinterpret_cast<float4*>(det_boxes), det_scores, det_count);
     if (e != cudaSuccess) return cuda_fail(e, "yolo_fast_kernel");
@@ -216,9 +216,10 @@ extern "C" __attribute__((visibility("default"))) int det_debug_read_phases(long
 }
 #endif
 
-extern "C" {
-
-static int yolo_decode_nms_impl(const float* head, int n, int s, int b, int c, int img_h, int img_w, const float* priors,
+// The entry points below have C linkage through their declarations in det_b200.h; the per-type implementation is a C++
+// template.
+template <typename T>
+static int yolo_decode_nms_impl(const void* head_v, int n, int s, int b, int c, int img_h, int img_w, const float* priors,
                                 float scale_clamp, int clip, float score_thresh, double iou_threshold, int mode,
                                 float* dense_boxes, float* dense_conf, float* dense_scores, int64_t max_det,
                                 int64_t* det_flat, float* det_boxes, float* det_scores, int32_t* det_count, void* stream,
@@ -226,15 +227,16 @@ static int yolo_decode_nms_impl(const float* head, int n, int s, int b, int c, i
     DET_CHECK_ARG(n >= 0 && s >= 1 && b >= 1 && c >= 1 && max_det >= 1, "bad size");
     DET_CHECK_ARG(mode >= DET_NMS_AUTO && mode <= DET_NMS_OFFSET_TRICK, "unknown mode");
     if (n == 0) return DET_OK;
-    DET_CHECK_ARG(head && priors && det_flat && det_count, "null pointer");
+    DET_CHECK_ARG(head_v && priors && det_flat && det_count, "null pointer");
+    const T* head = static_cast<const T*>(head_v);
     const int64_t P = (int64_t)s * s * b, PC = P * c, HS = (int64_t)s * s * (b * 5 + c);
     if (P > kYoloMaxPred || PC > 4096 || HS > kYoloMaxHead || c > 1024) {
         set_error("grid head too large for the fused kernel (limits: s*s*b <= 1024, s*s*b*c <= 4096, "
                   "s*s*(5b+c) <= 6144); use det_dense_decode_level + det_nms_batched");
         return DET_ERR_UNSUPPORTED;
     }
-    if (!aligned16(head) || (dense_boxes && !aligned16(dense_boxes)) || (det_boxes && !aligned16(det_boxes))) {
-        set_error("head / box outputs must be 16-byte aligned");
+    if (!aligned_to(head, 4 * sizeof(T)) || (dense_boxes && !aligned16(dense_boxes)) || (det_boxes && !aligned16(det_boxes))) {
+        set_error("head must be aligned to 4 elements, box outputs to 16 bytes");
         return DET_ERR_ALIGN;
     }
     YoloParams prm;
@@ -265,18 +267,27 @@ int det_yolo_decode_nms(const float* head, int n, int s, int b, int c, int img_h
                         float scale_clamp, int clip, float score_thresh, double iou_threshold, int mode,
                         float* dense_boxes, float* dense_conf, float* dense_scores, int64_t max_det,
                         int64_t* det_flat, float* det_boxes, float* det_scores, int32_t* det_count, void* stream) {
-    return yolo_decode_nms_impl(head, n, s, b, c, img_h, img_w, priors, scale_clamp, clip, score_thresh, iou_threshold, mode,
-                                dense_boxes, dense_conf, dense_scores, max_det, det_flat, det_boxes, det_scores, det_count,
-                                stream, 0);
+    return yolo_decode_nms_impl<float>(head, n, s, b, c, img_h, img_w, priors, scale_clamp, clip, score_thresh,
+                                       iou_threshold, mode, dense_boxes, dense_conf, dense_scores, max_det, det_flat,
+                                       det_boxes, det_scores, det_count, stream, 0);
 }
 
 int det_yolo_decode_nms_i32(const float* head, int n, int s, int b, int c, int img_h, int img_w, const float* priors,
                             float scale_clamp, int clip, float score_thresh, double iou_threshold, int mode,
                             float* dense_boxes, float* dense_conf, float* dense_scores, int64_t max_det,
                             int32_t* det_flat32, float* det_boxes, float* det_scores, int32_t* det_count, void* stream) {
-    return yolo_decode_nms_impl(head, n, s, b, c, img_h, img_w, priors, scale_clamp, clip, score_thresh, iou_threshold, mode,
-                                dense_boxes, dense_conf, dense_scores, max_det, reinterpret_cast<int64_t*>(det_flat32),
-                                det_boxes, det_scores, det_count, stream, 1);
+    return yolo_decode_nms_impl<float>(head, n, s, b, c, img_h, img_w, priors, scale_clamp, clip, score_thresh,
+                                       iou_threshold, mode, dense_boxes, dense_conf, dense_scores, max_det,
+                                       reinterpret_cast<int64_t*>(det_flat32), det_boxes, det_scores, det_count, stream, 1);
 }
 
-}  // extern "C"
+int det_yolo_decode_nms_typed(const void* head, int head_dtype, int n, int s, int b, int c, int img_h, int img_w,
+                              const float* priors, float scale_clamp, int clip, float score_thresh, double iou_threshold,
+                              int mode, float* dense_boxes, float* dense_conf, float* dense_scores, int64_t max_det,
+                              void* det_flat, int index_bytes, float* det_boxes, float* det_scores, int32_t* det_count,
+                              void* stream) {
+    DET_CHECK_ARG(index_bytes == 8 || index_bytes == 4, "index_bytes must be 8 or 4");
+    DET_HEAD_DISPATCH(head_dtype, yolo_decode_nms_impl, head, n, s, b, c, img_h, img_w, priors, scale_clamp, clip,
+                      score_thresh, iou_threshold, mode, dense_boxes, dense_conf, dense_scores, max_det,
+                      static_cast<int64_t*>(det_flat), det_boxes, det_scores, det_count, stream, index_bytes == 4 ? 1 : 0);
+}

@@ -3,7 +3,7 @@
 //
 // One CTA per image, ONE WARP PER CLASS.  A class has at most 128 candidates (one per predictor), so every
 // per-class step fits a warp and needs no block barrier:
-//   A  stage the image's logits (16-byte loads), sigmoid the conf / class logits in place, decode the boxes
+//   A  stage the image's logits (16-byte loads; 8-byte loads of a bf16 / fp16 head, widened to fp32 on load), sigmoid the conf / class logits in place, decode the boxes
 //   B  scores conf x class for the warp's class, threshold, class count, score histogram; one thread per predictor
 //      gathers the coordinate statistics torchvision's offset trick needs
 //   T  tier cut: only the first max_det kept detections (global score order) are output and a box can only be
@@ -71,9 +71,9 @@ __device__ __forceinline__ int score_shift(unsigned base) {
     return 0x3F800000u > base ? max(0, 32 - __clz(0x3F800000u - base) - 8) : 0;
 }
 
-template <int MAXT, int MINB, int CS, int CB, int CC>
+template <int MAXT, int MINB, int CS, int CB, int CC, typename HT = float>
 __global__ void __launch_bounds__(MAXT, MINB)
-yolo_fast_kernel(const float* __restrict__ head, const float2* __restrict__ priors, YoloParams prm,
+yolo_fast_kernel(const HT* __restrict__ head, const float2* __restrict__ priors, YoloParams prm,
                  float4* __restrict__ dense_boxes, float* __restrict__ dense_conf, float* __restrict__ dense_scores,
                  int64_t* __restrict__ det_flat, float4* __restrict__ det_boxes, float* __restrict__ det_scores,
                  int32_t* __restrict__ det_count) {
@@ -117,7 +117,7 @@ yolo_fast_kernel(const float* __restrict__ head, const float2* __restrict__ prio
     // transformed on its way into shared memory -- sigmoid for tx, ty, conf and the class logits, exp(min(t, clamp)) for
     // tw, th -- so nothing is staged raw and the box assembly below is a handful of multiply-adds
     const int64_t g0 = (int64_t)img * S2 * ch, g1 = g0 + (int64_t)S2 * ch;
-    const float4* head4 = reinterpret_cast<const float4*>(head);
+    const typename Head<HT>::vec* head4 = reinterpret_cast<const typename Head<HT>::vec*>(head);  // 4 elements per load
     auto activate = [&](int e, float x) -> float {  // e = element index inside the image (cell-major, channel-minor)
         const int cell = e / ch, k = e - cell * ch;
         if (k < B * 5) {
@@ -133,12 +133,12 @@ yolo_fast_kernel(const float* __restrict__ head, const float2* __restrict__ prio
         const int64_t base = v << 2;
         const int e0 = (int)(base - g0);
         if (base >= g0 && base + 4 <= g1) {
-            const float4 q = ld_stream(head4 + v);
+            const float4 q = ld4_stream<HT>(head4 + v);
             float* d = hs + e0;
             d[0] = activate(e0, q.x); d[1] = activate(e0 + 1, q.y); d[2] = activate(e0 + 2, q.z); d[3] = activate(e0 + 3, q.w);
         } else {
             for (int e = 0; e < 4; ++e)
-                if (base + e >= g0 && base + e < g1) hs[e0 + e] = activate(e0 + e, ld_stream(head + base + e));
+                if (base + e >= g0 && base + e < g1) hs[e0 + e] = activate(e0 + e, ld1_stream(head + base + e));
         }
     }
     __syncthreads();

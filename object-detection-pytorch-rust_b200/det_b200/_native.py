@@ -33,6 +33,7 @@ PROTOTYPES = {
     "det_rpn_decode_level": (c_i, [c_p, c_p, c_i, c_i, c_i, c_i, c_i, c_f, c_p, c_f, c_f, c_f, c_f, c_f, c_p, c_p,
                                    c_l, c_l, c_p]),
     "det_rpn_decode": (c_i, [c_p, c_i, c_i, c_i, c_f, c_f, c_f, c_f, c_f, c_f, c_p, c_p, c_l, c_p]),
+    "det_rpn_decode_typed": (c_i, [c_p, c_i, c_i, c_i, c_f, c_f, c_f, c_f, c_f, c_f, c_p, c_p, c_l, c_i, c_p]),
     "det_nms_workspace_bytes": (c_l, [c_i, c_l]),
     "det_nms_batched": (c_i, [c_p, c_p, c_p, c_p, c_i, c_l, c_d, c_i, c_l, c_p, c_p, c_p, c_l, c_p]),
     "det_rpn_proposals_workspace_bytes": (c_l, [c_i, c_l]),
@@ -42,12 +43,17 @@ PROTOTYPES = {
                                   c_p, c_p, c_p, c_p, c_p]),
     "det_yolo_decode_nms_i32": (c_i, [c_p, c_i, c_i, c_i, c_i, c_i, c_i, c_p, c_f, c_i, c_f, c_d, c_i, c_p, c_p, c_p, c_l,
                                       c_p, c_p, c_p, c_p, c_p]),
+    "det_yolo_decode_nms_typed": (c_i, [c_p, c_i, c_i, c_i, c_i, c_i, c_i, c_i, c_p, c_f, c_i, c_f, c_d, c_i, c_p, c_p,
+                                        c_p, c_l, c_p, c_i, c_p, c_p, c_p, c_p]),
     "det_dense_decode_level": (c_i, [c_p, c_i, c_i, c_i, c_i, c_i, c_i, c_p, c_f, c_p, c_p, c_p, c_l, c_l, c_p]),
     "det_dense_decode": (c_i, [c_p, c_i, c_i, c_i, c_i, c_f, c_p, c_p, c_p, c_l, c_p]),
+    "det_dense_decode_typed": (c_i, [c_p, c_i, c_i, c_i, c_i, c_f, c_p, c_p, c_p, c_l, c_i, c_p]),
     "det_dense_detect_workspace_bytes": (c_l, [c_i, c_l]),
     "det_dense_detect_counter_bytes": (c_l, [c_i]),
     "det_dense_detect": (c_i, [c_p, c_i, c_i, c_i, c_i, c_f, c_f, c_d, c_i, c_i, c_l, c_l, c_p, c_p, c_p, c_p, c_p, c_p,
                                c_p, c_l, c_p]),
+    "det_dense_detect_typed": (c_i, [c_p, c_i, c_i, c_i, c_i, c_f, c_f, c_d, c_i, c_i, c_l, c_l, c_p, c_p, c_p, c_p, c_p,
+                                     c_p, c_p, c_l, c_i, c_p]),
     "det_threshold_compact": (c_i, [c_p, c_p, c_p, c_i, c_l, c_f, c_l, c_p, c_p, c_p, c_p, c_p, c_p]),
     "det_gather_detections": (c_i, [c_p, c_p, c_i, c_l, c_p, c_p, c_p, c_p, c_l, c_p, c_p, c_p, c_p, c_p]),
     "det_peer_sums_publish": (c_i, [c_p, c_i, c_i, c_i, c_p, c_i, c_i, ctypes.c_uint32, c_p]),
@@ -215,3 +221,23 @@ def f32c(t):
     box kernels require: a view can be contiguous and still start inside a row, e.g. rois[:, 1:5] of a single roi."""
     t = t.detach().to(torch.float32).contiguous()
     return t if t.data_ptr() % 16 == 0 else t.clone()
+
+
+# DET_DTYPE_* of include/det_b200.h: head element types the decode kernels read natively (widened to fp32 on load)
+DTYPE_CODES = {torch.float32: 0, torch.bfloat16: 1, torch.float16: 2}
+
+
+def heads_c(tensors):
+    """(list of head tensors, DET_DTYPE_* code) for the *_typed entry points.  When every tensor is fp32, bf16 or fp16
+    and they all share that dtype, each is kept in it -- contiguous and 16-byte aligned, copied only where it is not --
+    so a 16-bit head is read as it is (no fp32 copy; the result is bit-identical to the fp32 path on h.float()).
+    Anything else (fp64, mixed dtypes) goes through f32c, code 0."""
+    tensors = list(tensors)
+    dts = {t.dtype for t in tensors}
+    if len(dts) != 1 or next(iter(dts)) not in DTYPE_CODES:
+        return [f32c(t) for t in tensors], 0
+    out = []
+    for t in tensors:
+        t = t.detach().contiguous()
+        out.append(t if t.data_ptr() % 16 == 0 else t.clone())
+    return out, DTYPE_CODES[tensors[0].dtype]

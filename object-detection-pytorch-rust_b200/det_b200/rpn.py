@@ -134,7 +134,9 @@ class RegionProposalNetwork:
     # ------------------------------------------------------------------ decode
     def decode_heads(self, pred_objectness: List[torch.Tensor], pred_deltas: List[torch.Tensor]):
         """Conv-layout head outputs, per level (N,A,Hi,Wi) and (N,A*4,Hi,Wi) -> logits (N,R), proposals (N,R,4) with all
-        levels concatenated in (level,h,w,a) order; anchors are synthesised in the kernel (rpn.py:270-284 + :330-348)."""
+        levels concatenated in (level,h,w,a) order; anchors are synthesised in the kernel (rpn.py:270-284 + :330-348).
+        bf16 / fp16 heads (objectness and deltas of every level one dtype) are read as they are: bit-identical to the
+        fp32 heads h.float()."""
         N.require_cuda(*pred_objectness, *pred_deltas)
         dev = pred_objectness[0].device
         n = pred_objectness[0].shape[0]
@@ -144,7 +146,9 @@ class RegionProposalNetwork:
         logits = torch.empty((n, R), dtype=torch.float32, device=dev)
         boxes = torch.empty((n, R, 4), dtype=torch.float32, device=dev)
         w = self.box2box_transform.weights
-        ocs, dcs = [N.f32c(o) for o in pred_objectness], [N.f32c(d) for d in pred_deltas]
+        nl = len(pred_objectness)
+        hcs, code = N.heads_c(list(pred_objectness) + list(pred_deltas))
+        ocs, dcs = hcs[:nl], hcs[nl:]
         na = ocs[0].shape[1]
         if all(o.shape[1] == na for o in ocs):  # one launch for the whole pyramid (det_rpn_decode)
             lv = (N.RpnLevel * len(ocs))()
@@ -155,18 +159,23 @@ class RegionProposalNetwork:
                 lv[i].h, lv[i].w, lv[i].stride, lv[i].reserved, lv[i].out_offset = oc.shape[2], oc.shape[3], int(stride), 0, off
                 off += sz
             with torch.cuda.device(dev):
-                N.call("det_rpn_decode", ctypes.cast(lv, ctypes.c_void_p), len(ocs), n, na,
+                N.call("det_rpn_decode_typed", ctypes.cast(lv, ctypes.c_void_p), len(ocs), n, na,
                        float(self.anchor_generator.offset), *w, self.box2box_transform.scale_clamp, N.ptr(logits),
-                       N.ptr(boxes), R, N.stream())
+                       N.ptr(boxes), R, code, N.stream())
             return logits, boxes, sizes
         off = 0
         with torch.cuda.device(dev):
             for oc, dc, cell, stride, sz in zip(ocs, dcs, cells, self.anchor_generator.strides, sizes):
                 a, h, wd = oc.shape[1], oc.shape[2], oc.shape[3]
                 assert dc.shape[1] == a * 4 and a == cell.shape[0]
-                N.call("det_rpn_decode_level", N.ptr(oc), N.ptr(dc), n, a, h, wd, int(stride),
-                       float(self.anchor_generator.offset), N.ptr(cell), *w, self.box2box_transform.scale_clamp,
-                       N.ptr(logits), N.ptr(boxes), R, off, N.stream())
+                if code == 0:
+                    N.call("det_rpn_decode_level", N.ptr(oc), N.ptr(dc), n, a, h, wd, int(stride),
+                           float(self.anchor_generator.offset), N.ptr(cell), *w, self.box2box_transform.scale_clamp,
+                           N.ptr(logits), N.ptr(boxes), R, off, N.stream())
+                else:  # a 16-bit level: the typed entry point with this one level
+                    lv = N.RpnLevel(oc.data_ptr(), dc.data_ptr(), cell.data_ptr(), h, wd, int(stride), 0, off)
+                    N.call("det_rpn_decode_typed", ctypes.byref(lv), 1, n, a, float(self.anchor_generator.offset), *w,
+                           self.box2box_transform.scale_clamp, N.ptr(logits), N.ptr(boxes), R, code, N.stream())
                 off += sz
         return logits, boxes, sizes
 
@@ -362,7 +371,8 @@ class RegionProposalNetwork:
         ranks (normaliser = batch_size_per_image * that, rpn.py:238)."""
         N.require_cuda(anchors, logits, deltas)
         at = N.f32c(anchors)
-        lg, dl = logits.contiguous(), deltas.contiguous()
+        # the loss kernel reads fp32: a 16-bit head (forward(training) sends those here) is converted, autograd-connected
+        lg, dl = logits.float().contiguous(), deltas.float().contiguous()
         n_norm = lg.shape[0] if num_images_global is None else int(num_images_global)
         if with_grads:
             gl, gd = torch.empty_like(lg), torch.empty_like(dl)

@@ -50,9 +50,10 @@ class YoloGridHead:
         count (N) int32) with K = max_det padding, by descending score; one launch, no host synchronisation.
         With return_dense the decoded boxes/conf/scores of every predictor are written too.
         `out` may carry a dict returned by an earlier call with the same shapes to reuse its buffers.
-        index_dtype=torch.int32 writes the same `flat` values as 32-bit integers (det_yolo_decode_nms_i32)."""
+        index_dtype=torch.int32 writes the same `flat` values as 32-bit integers (det_yolo_decode_nms_i32).
+        A bf16 / fp16 head is read as it is (det_yolo_decode_nms_typed): the results are bit-identical to head.float()."""
         N.require_cuda(head)
-        h = N.f32c(head)
+        (h,), code = N.heads_c([head])
         n = h.shape[0]
         assert tuple(h.shape[1:]) == (self.S, self.S, self.B * 5 + self.C), h.shape
         P, C = self.num_predictors, self.C
@@ -70,12 +71,12 @@ class YoloGridHead:
         assert out["flat"].dtype in (torch.int64, torch.int32)
         if n:
             with torch.cuda.device(dev):
-                N.call("det_yolo_decode_nms" if out["flat"].dtype == torch.int64 else "det_yolo_decode_nms_i32",
-                       N.ptr(h), n, self.S, self.B, C, self.image_size[0], self.image_size[1],
-                       N.ptr(self.priors_on(dev)), self.scale_clamp, int(self.clip), float(score_thresh),
-                       float(iou_thresh), int(mode), N.ptr(out.get("dense_boxes")), N.ptr(out.get("dense_conf")),
-                       N.ptr(out.get("dense_scores")), max_det, N.ptr(out["flat"]), N.ptr(out["boxes"]),
-                       N.ptr(out["scores"]), N.ptr(out["count"]), N.stream())
+                N.call("det_yolo_decode_nms_typed", N.ptr(h), code, n, self.S, self.B, C, self.image_size[0],
+                       self.image_size[1], N.ptr(self.priors_on(dev)), self.scale_clamp, int(self.clip),
+                       float(score_thresh), float(iou_thresh), int(mode), N.ptr(out.get("dense_boxes")),
+                       N.ptr(out.get("dense_conf")), N.ptr(out.get("dense_scores")), max_det, N.ptr(out["flat"]),
+                       out["flat"].element_size(), N.ptr(out["boxes"]), N.ptr(out["scores"]), N.ptr(out["count"]),
+                       N.stream())
         return out
 
     def decode(self, head: torch.Tensor):
@@ -89,24 +90,27 @@ class YoloHostPipeline:
     buffers, its own stream and a CUDA graph [H2D copy -> det_yolo_decode_nms -> D2H copy].  Slots run on different
     streams, so the upload of batch i+1, the kernel of batch i and the download of batch i-1 overlap (separate copy
     engines per direction).  The producer writes a batch into ``input(slot)`` (pinned), calls ``launch(slot)`` and
-    later ``wait(slot)`` -> dict of pinned host views (flat, boxes, scores, count).  No per-step allocation."""
+    later ``wait(slot)`` -> dict of pinned host views (flat, boxes, scores, count).  No per-step allocation.
+    input_dtype torch.bfloat16 / torch.float16: the host and device inputs are 16-bit and the kernel reads them as they
+    are -- half the upload bytes, results bit-identical to the fp32 head holding the same values."""
 
     def __init__(self, head: "YoloGridHead", batch: int, score_thresh: float = 0.25, iou_thresh: float = 0.5,
                  max_det: int = 300, depth: int = 3, device=None, mode: int = MODE_AUTO, use_graph: bool = True,
-                 index_dtype: torch.dtype = torch.int64):
+                 index_dtype: torch.dtype = torch.int64, input_dtype: torch.dtype = torch.float32):
         dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         self.head, self.batch, self.depth, self.device = head, int(batch), int(depth), dev
         self.args = (float(score_thresh), float(iou_thresh), int(max_det), int(mode))
         shape = (self.batch, head.S, head.S, head.B * 5 + head.C)
         k = int(max_det)
         assert index_dtype in (torch.int64, torch.int32)
+        assert input_dtype in N.DTYPE_CODES, f"input_dtype must be one of {list(N.DTYPE_CODES)}"
         self.index_dtype = index_dtype  # int32: the same indices, 4 bytes less per detection on the PCIe download
         isz = 8 if index_dtype == torch.int64 else 4
         # one output blob per slot so the download is a single copy: [flat i64/i32 | boxes f32x4 | scores f32 | count i32]
         self._sizes = (self.batch * k * isz, self.batch * k * 16, self.batch * k * 4, self.batch * 4)
         nbytes = sum(self._sizes)
-        self.h_in = [torch.empty(shape, dtype=torch.float32).pin_memory() for _ in range(depth)]
-        self.d_in = [torch.empty(shape, dtype=torch.float32, device=dev) for _ in range(depth)]
+        self.h_in = [torch.empty(shape, dtype=input_dtype).pin_memory() for _ in range(depth)]
+        self.d_in = [torch.empty(shape, dtype=input_dtype, device=dev) for _ in range(depth)]
         self.d_blob = [torch.empty((nbytes,), dtype=torch.uint8, device=dev) for _ in range(depth)]
         self.h_blob = [torch.empty((nbytes,), dtype=torch.uint8).pin_memory() for _ in range(depth)]
         self.d_out = [self._views(b, k) for b in self.d_blob]
@@ -114,7 +118,7 @@ class YoloHostPipeline:
         self.streams = [torch.cuda.Stream(device=dev) for _ in range(depth)]
         self.done = [torch.cuda.Event() for _ in range(depth)]
         self.graphs = [None] * depth
-        self.h2d_bytes = self.h_in[0].numel() * 4
+        self.h2d_bytes = self.h_in[0].numel() * self.h_in[0].element_size()
         self.d2h_bytes = nbytes
         if use_graph:
             for s in range(depth):
@@ -313,7 +317,8 @@ class DenseAnchorHead:
         return self._dev[k]
 
     def decode(self, heads: List[torch.Tensor], out=None):
-        """-> boxes (N,R,4), scores (N,R), classes (N,R) int64 with all levels concatenated, order (level,h,w,a)."""
+        """-> boxes (N,R,4), scores (N,R), classes (N,R) int64 with all levels concatenated, order (level,h,w,a).
+        bf16 / fp16 heads (all levels one dtype) are read as they are: bit-identical to the fp32 heads h.float()."""
         N.require_cuda(*heads)
         dev = heads[0].device
         n = heads[0].shape[0]
@@ -325,36 +330,30 @@ class DenseAnchorHead:
                    torch.empty((n, R), dtype=torch.int64, device=dev))
         boxes, scores, classes = out
         anchors = self._anchors_on(dev)
-        hcs = [N.f32c(h) for h in heads]
+        hcs, code = N.heads_c(heads)
         na = anchors[0].shape[0]
         if all(a.shape[0] == na for a in anchors):  # one persistent launch for the whole pyramid
-            lv = (N.DenseLevel * len(hcs))()
-            off = 0
-            for i, (hc, a, s, sz) in enumerate(zip(hcs, anchors, self.strides, sizes)):
-                assert hc.shape[1] == na * (5 + self.C), hc.shape
-                lv[i].head, lv[i].anchors_wh = hc.data_ptr(), a.data_ptr()
-                lv[i].h, lv[i].w, lv[i].stride, lv[i].reserved, lv[i].out_offset = hc.shape[2], hc.shape[3], s, 0, off
-                off += sz
+            lv = self._level_array(hcs, anchors, na)
             with torch.cuda.device(dev):
-                N.call("det_dense_decode", ctypes.cast(lv, ctypes.c_void_p), len(hcs), n, na, self.C, self.scale_clamp,
-                       N.ptr(boxes), N.ptr(scores), N.ptr(classes), R, N.stream())
+                N.call("det_dense_decode_typed", ctypes.cast(lv, ctypes.c_void_p), len(hcs), n, na, self.C,
+                       self.scale_clamp, N.ptr(boxes), N.ptr(scores), N.ptr(classes), R, code, N.stream())
             return boxes, scores, classes
         off = 0
         with torch.cuda.device(dev):
             for hc, a, s, sz in zip(hcs, anchors, self.strides, sizes):
                 assert hc.shape[1] == a.shape[0] * (5 + self.C), hc.shape
-                N.call("det_dense_decode_level", N.ptr(hc), n, a.shape[0], self.C, hc.shape[2], hc.shape[3], s,
-                       N.ptr(a), self.scale_clamp, N.ptr(boxes), N.ptr(scores), N.ptr(classes), R, off, N.stream())
+                if code == 0:
+                    N.call("det_dense_decode_level", N.ptr(hc), n, a.shape[0], self.C, hc.shape[2], hc.shape[3], s,
+                           N.ptr(a), self.scale_clamp, N.ptr(boxes), N.ptr(scores), N.ptr(classes), R, off, N.stream())
+                else:  # a 16-bit level: the typed entry point with this one level
+                    lv = N.DenseLevel(hc.data_ptr(), a.data_ptr(), hc.shape[2], hc.shape[3], s, 0, off)
+                    N.call("det_dense_decode_typed", ctypes.byref(lv), 1, n, a.shape[0], self.C, self.scale_clamp,
+                           N.ptr(boxes), N.ptr(scores), N.ptr(classes), R, code, N.stream())
                 off += sz
         return boxes, scores, classes
 
-    def _levels(self, heads: List[torch.Tensor]):
-        """(det_dense_level_t array, contiguous heads, n, A, R) for heads that share the anchor count."""
-        dev = heads[0].device
-        anchors = self._anchors_on(dev)
-        hcs = [N.f32c(h) for h in heads]
-        na = anchors[0].shape[0]
-        assert all(a.shape[0] == na for a in anchors), "levels must share the anchor count"
+    def _level_array(self, hcs, anchors, na):
+        """det_dense_level_t array over prepared heads that share the anchor count `na`."""
         lv = (N.DenseLevel * len(hcs))()
         off = 0
         for i, (hc, a, s) in enumerate(zip(hcs, anchors, self.strides)):
@@ -362,7 +361,19 @@ class DenseAnchorHead:
             lv[i].head, lv[i].anchors_wh = hc.data_ptr(), a.data_ptr()
             lv[i].h, lv[i].w, lv[i].stride, lv[i].reserved, lv[i].out_offset = hc.shape[2], hc.shape[3], s, 0, off
             off += hc.shape[2] * hc.shape[3] * na
-        return lv, hcs, heads[0].shape[0], na, off
+        return lv
+
+    def _levels(self, heads: List[torch.Tensor], typed: bool = False):
+        """(det_dense_level_t array, contiguous heads, n, A, R) for heads that share the anchor count; the heads are fp32
+        (f32c).  typed=True: bf16 / fp16 heads are kept as they are (N.heads_c) and the DET_DTYPE_* code is appended."""
+        dev = heads[0].device
+        anchors = self._anchors_on(dev)
+        hcs, code = N.heads_c(heads) if typed else ([N.f32c(h) for h in heads], 0)
+        na = anchors[0].shape[0]
+        assert all(a.shape[0] == na for a in anchors), "levels must share the anchor count"
+        lv = self._level_array(hcs, anchors, na)
+        res = (lv, hcs, heads[0].shape[0], na, sum(h.shape[2] * h.shape[3] * na for h in hcs))
+        return res + (code,) if typed else res
 
     def fused_ok(self, heads: List[torch.Tensor]) -> bool:
         """det_dense_detect's documented limits: equal anchor counts, every level h*w % 4 == 0."""
@@ -379,7 +390,8 @@ class DenseAnchorHead:
 
         cand_cap (<= 4096) bounds the per-image candidate list.  With check=True (one 4-byte read-back) an image that
         overflows it -- or a pyramid outside det_dense_detect's limits -- is redone exactly by the unfused GPU path
-        (decode + det_nms_batched); with check=False overflowing images carry count = -1 and `overflow` is set."""
+        (decode + det_nms_batched); with check=False overflowing images carry count = -1 and `overflow` is set.
+        bf16 / fp16 heads (all levels one dtype) are read as they are, on both routes: bit-identical to h.float()."""
         N.require_cuda(*heads)
         dev = heads[0].device
         n = heads[0].shape[0]
@@ -395,7 +407,7 @@ class DenseAnchorHead:
                    "overflow": torch.empty((1,), dtype=torch.int32, device=dev)}
         if n == 0:
             return out
-        lv, hcs, _, na, _ = self._levels(heads)
+        lv, hcs, _, na, _, code = self._levels(heads, typed=True)
         wsb = N.fn("det_dense_detect_workspace_bytes")(n, int(cand_cap))
         flags = 1 if gate else 0
         if isinstance(workspace, DenseDetectWorkspace):
@@ -404,10 +416,10 @@ class DenseAnchorHead:
         elif workspace is None or workspace.numel() < wsb:
             workspace = torch.empty((wsb,), dtype=torch.uint8, device=dev)
         with torch.cuda.device(dev):
-            N.call("det_dense_detect", ctypes.cast(lv, ctypes.c_void_p), len(hcs), n, na, self.C, self.scale_clamp,
-                   float(score_thresh), float(iou_thresh), int(mode), flags, int(cand_cap), max_det,
+            N.call("det_dense_detect_typed", ctypes.cast(lv, ctypes.c_void_p), len(hcs), n, na, self.C,
+                   self.scale_clamp, float(score_thresh), float(iou_thresh), int(mode), flags, int(cand_cap), max_det,
                    N.ptr(out["idx"]), N.ptr(out["boxes"]), N.ptr(out["scores"]), N.ptr(out["classes"]),
-                   N.ptr(out["count"]), N.ptr(out["overflow"]), N.ptr(workspace), wsb, N.stream())
+                   N.ptr(out["count"]), N.ptr(out["overflow"]), N.ptr(workspace), wsb, code, N.stream())
         if check and int(out["overflow"].item()) != 0:
             return self._detect_thresholded_unfused(heads, score_thresh, iou_thresh, max_det, mode)
         return out
