@@ -396,19 +396,38 @@ DET_API int det_yolo_loss(const float* head, const int8_t* labels, const int64_t
                   const float* upstream, float* accumulators, float* sums_out, float* grad_head, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------
- * (next tier, SURVEY 8f rank 2) FPN level assignment + ROIAlign over a feature pyramid -- replaces
+ * (next tier, SURVEY 8f rank 2) FPN level assignment + ROIAlign / ROIPool over a feature pyramid -- replaces
  *      assign_boxes_to_levels / ROIPooler.forward / ROIAlign.forward,
- *      python/src/models/modules/roi_poolers.py:103-131, :269-331, :55-72 (torchvision.ops.roi_align underneath).
- *      det_roi_align_levels_backward: levels' `data` are the GRADIENT buffers (n, c, h, w), zeroed by the caller and
- *      accumulated into with atomics; grad_out (m, c, out_h, out_w).
+ *      python/src/models/modules/roi_poolers.py:103-131, :269-331, :55-72 (torchvision.ops.roi_align underneath),
+ *      and the ROIPool pooler type, roi_poolers.py:224-231 (torchvision.ops.roi_pool underneath).
  *      det_roi_levels: level_out[i] = clamp(floor(canonical_level + log2(sqrt(area_i)/canonical_box_size + 1e-8)),
  *      min_level, max_level) - min_level, boxes (m,4).
- *      det_roi_align_levels: every box samples the level `level[i]` (NULL when num_levels == 1) of image
- *      batch_index[i]; level l: data (n, c, h, w) device fp32, spatial_scale = 1/stride.  out (m, c, out_h, out_w).
- *      sampling_ratio <= 0: ceil(roi / bins) samples per bin; aligned != 0: half-pixel shift (ROIAlignV2).
+ *      Every pooling entry: box i (boxes (m,4) fp32, 16-byte aligned) samples the level `level[i]` (int64; NULL when
+ *      num_levels == 1) of image batch_index[i] (int32); level l: data (n, c, h, w) contiguous, spatial_scale =
+ *      1/stride.  out / grad_out (m, c, out_h, out_w).  m == 0 returns DET_OK without reading any pointer.
+ *
+ *      Feature dtypes (feat_dtype / grad_dtype = DET_DTYPE_*; all levels and the output share it): every element is
+ *      widened to fp32 on load, the arithmetic is fp32, and the output is rounded once to the feature dtype
+ *      (__float2bfloat16_rn / __float2half_rn).  So a bf16 / fp16 result is bit-identical to the fp32 call on the
+ *      widened features followed by torch's .to(dtype) -- torchvision's autocast rule for roi_align / roi_pool.  An
+ *      unknown dtype: DET_ERR_BAD_ARG before any CUDA call.  Gradients always accumulate into fp32 buffers.
+ *
+ *      det_roi_align_levels_typed: torchvision roi_align; sampling_ratio <= 0: ceil(roi / bins) samples per bin;
+ *      aligned != 0: half-pixel shift (ROIAlignV2).  det_roi_align_levels is this call with DET_DTYPE_F32.
+ *      det_roi_align_levels_backward_typed: levels' `data` are the fp32 GRADIENT buffers (n, c, h, w), zeroed by the
+ *      caller and accumulated into with atomics; grad_out of grad_dtype.  det_roi_align_levels_backward is this call
+ *      with DET_DTYPE_F32.
+ *      det_roi_pool_levels: torchvision roi_pool (max pooling).  start = round(x * spatial_scale) in fp32, halves away
+ *      from zero; roi size max(end - start + 1, 1); bin p of an axis covers [floor(p * bin), ceil((p + 1) * bin)) +
+ *      start, clamped to [0, h] / [0, w].  An empty bin outputs 0; otherwise the max, scanned rows then columns with a
+ *      strict `>` from -FLT_MAX (first maximum wins, NaN never taken; a bin of NaN / -inf gives -FLT_MAX, -inf in 16
+ *      bit).  argmax (m, c, out_h, out_w) int32 = h*W + w inside the box's level plane, -1 when nothing was taken; NULL:
+ *      not written (inference).  sampling_ratio and aligned do not apply.  Every level needs h*w < 2^31.
+ *      det_roi_pool_levels_backward: grad level[batch_index[i]][c][argmax] += grad_out for every argmax >= 0, fp32
+ *      atomics into the zeroed fp32 gradient buffers `grad_levels_host[l].data`; argmax from the forward.
  * ---------------------------------------------------------------------------------------------------------- */
 typedef struct det_feature_level {
-    const float* data;
+    const float* data;  /* the *_typed and pool entries: elements of their feat_dtype, cast to this pointer type */
     int32_t h, w;
     float spatial_scale;
     int32_t reserved;
@@ -418,10 +437,26 @@ DET_API int det_roi_levels(const float* boxes, int64_t m, int min_level, int max
 DET_API int det_roi_align_levels(const det_feature_level_t* levels_host, int num_levels, int n, int c, const float* boxes,
                          const int32_t* batch_index, const int64_t* level, int64_t m, int out_h, int out_w,
                          int sampling_ratio, int aligned, float* out, void* stream);
+DET_API int det_roi_align_levels_typed(const det_feature_level_t* levels_host, int num_levels, int n, int c,
+                                       const float* boxes, const int32_t* batch_index, const int64_t* level, int64_t m,
+                                       int out_h, int out_w, int sampling_ratio, int aligned, void* out, int feat_dtype,
+                                       void* stream);
 DET_API int det_roi_align_levels_backward(const det_feature_level_t* grad_levels_host, int num_levels, int n, int c,
                                   const float* boxes, const int32_t* batch_index, const int64_t* level, int64_t m,
                                   int out_h, int out_w, int sampling_ratio, int aligned, const float* grad_out,
                                   void* stream);
+DET_API int det_roi_align_levels_backward_typed(const det_feature_level_t* grad_levels_host, int num_levels, int n,
+                                                int c, const float* boxes, const int32_t* batch_index,
+                                                const int64_t* level, int64_t m, int out_h, int out_w,
+                                                int sampling_ratio, int aligned, const void* grad_out, int grad_dtype,
+                                                void* stream);
+DET_API int det_roi_pool_levels(const det_feature_level_t* levels_host, int num_levels, int n, int c, const float* boxes,
+                                const int32_t* batch_index, const int64_t* level, int64_t m, int out_h, int out_w,
+                                void* out, int32_t* argmax, int feat_dtype, void* stream);
+DET_API int det_roi_pool_levels_backward(const det_feature_level_t* grad_levels_host, int num_levels, int n, int c,
+                                         const int32_t* batch_index, const int64_t* level, int64_t m, int out_h,
+                                         int out_w, const int32_t* argmax, const void* grad_out, int grad_dtype,
+                                         void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------
  * (e) the training path's one collective over NVLink peer memory instead of NCCL: SUM of the `width`-float loss/count

@@ -102,6 +102,13 @@ __device__ __forceinline__ float min_nan(float a, float b) {
 // streaming (evict-first) vector accesses for write-once / read-once data
 __device__ __forceinline__ void st_stream(float4* p, float4 v) { __stcs(p, v); }
 __device__ __forceinline__ void st_stream(float* p, float v) { __stcs(p, v); }
+// an fp32 result stored as a 16-bit feature element, rounded to nearest even as torch's CUDA .to() rounds on sm_80+
+__device__ __forceinline__ void st_stream(__nv_bfloat16* p, float v) {
+    __stcs(reinterpret_cast<unsigned short*>(p), __bfloat16_as_ushort(__float2bfloat16_rn(v)));
+}
+__device__ __forceinline__ void st_stream(__half* p, float v) {
+    __stcs(reinterpret_cast<unsigned short*>(p), __half_as_ushort(__float2half_rn(v)));
+}
 __device__ __forceinline__ float4 ld_stream(const float4* p) { return __ldcs(p); }
 __device__ __forceinline__ float ld_stream(const float* p) { return __ldcs(p); }
 

@@ -65,6 +65,11 @@ PROTOTYPES = {
     "det_roi_levels": (c_i, [c_p, c_l, c_i, c_i, c_f, c_i, c_p, c_p]),
     "det_roi_align_levels": (c_i, [c_p, c_i, c_i, c_i, c_p, c_p, c_p, c_l, c_i, c_i, c_i, c_i, c_p, c_p]),
     "det_roi_align_levels_backward": (c_i, [c_p, c_i, c_i, c_i, c_p, c_p, c_p, c_l, c_i, c_i, c_i, c_i, c_p, c_p]),
+    "det_roi_align_levels_typed": (c_i, [c_p, c_i, c_i, c_i, c_p, c_p, c_p, c_l, c_i, c_i, c_i, c_i, c_p, c_i, c_p]),
+    "det_roi_align_levels_backward_typed": (c_i, [c_p, c_i, c_i, c_i, c_p, c_p, c_p, c_l, c_i, c_i, c_i, c_i, c_p, c_i,
+                                                  c_p]),
+    "det_roi_pool_levels": (c_i, [c_p, c_i, c_i, c_i, c_p, c_p, c_p, c_l, c_i, c_i, c_p, c_p, c_i, c_p]),
+    "det_roi_pool_levels_backward": (c_i, [c_p, c_i, c_i, c_i, c_p, c_p, c_l, c_i, c_i, c_p, c_p, c_i, c_p]),
     "det_match_workspace_bytes": (c_l, [c_i, c_l, c_l]),
     "det_match_anchors": (c_i, [c_p, c_p, c_i, c_l, c_p, c_l, c_p, c_p, c_i, c_i, c_p, c_p, c_p, c_p, c_l, c_p]),
     "det_match_grid_workspace_bytes": (c_l, [c_i, c_l, c_p, c_i]),

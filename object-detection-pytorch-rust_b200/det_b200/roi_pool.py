@@ -1,10 +1,16 @@
-"""FPN level assignment + ROIAlign -- drop-in for ``assign_boxes_to_levels``, ``convert_boxes_to_pooler_format``,
-``ROIAlign`` and ``ROIPooler`` of the reference (python/src/models/modules/roi_poolers.py:15-331), forward and
-backward (gradients flow to the feature maps, as through torchvision's roi_align).
+"""FPN level assignment + ROIAlign / ROIPool -- drop-in for ``assign_boxes_to_levels``,
+``convert_boxes_to_pooler_format``, ``ROIAlign`` and ``ROIPooler`` of the reference
+(python/src/models/modules/roi_poolers.py:15-331), forward and backward (gradients flow to the feature maps, as through
+torchvision's roi_align / roi_pool).
 
-The reference loops over the pyramid levels with nonzero / gather / torchvision ``roi_align`` / ``index_put_``; here
-one kernel computes every box's level (det_roi_levels) and one kernel samples all levels (det_roi_align_levels).
-Third-party arithmetic: torchvision.ops.roi_align (un-vendored) -- the parity oracle is the installed CPU kernel."""
+The reference loops over the pyramid levels with nonzero / gather / torchvision ``roi_align`` or ``roi_pool`` /
+``index_put_``; here one kernel computes every box's level (det_roi_levels) and one kernel pools all levels
+(det_roi_align_levels_typed, det_roi_pool_levels).  Third-party arithmetic: torchvision.ops.roi_align / roi_pool
+(un-vendored) -- the parity oracle is the installed CPU kernel.
+
+bf16 / fp16 feature pyramids are read natively: the kernels widen each element to fp32, compute in fp32 and round the
+output once to the feature dtype, bit-identical to the fp32 route on ``f.float()`` followed by ``.to(dtype)``
+(torchvision's autocast rule).  Gradients accumulate in fp32 and are returned in each feature map's dtype."""
 import ctypes
 import math
 from typing import List, Sequence, Tuple, Union
@@ -45,55 +51,125 @@ def _level_table(tensors, scales):
     return lv
 
 
+def _feature_route(features: Sequence[torch.Tensor]) -> Tuple[List[torch.Tensor], int]:
+    """(feature maps for the kernels, DET_DTYPE_* code), for both poolers.  When every level is fp32, bf16 or fp16 alike
+    the maps are read in their dtype (contiguous; the kernels widen each element to fp32 on load); anything else (mixed
+    dtypes, fp64) is converted to fp32.  No detach: the returned tensors keep the autograd graph of the inputs."""
+    dts = {f.dtype for f in features}
+    if len(dts) == 1 and features[0].dtype in N.DTYPE_CODES:
+        return [f.contiguous() for f in features], N.DTYPE_CODES[features[0].dtype]
+    return [f.to(torch.float32).contiguous() for f in features], N.DTYPE_CODES[torch.float32]
+
+
+def _grad_route(grad_out: torch.Tensor) -> Tuple[torch.Tensor, int]:
+    """grad_out read in its own dtype (no fp32 copy) when the kernels take it, else as fp32."""
+    if grad_out.dtype in N.DTYPE_CODES:
+        return grad_out.contiguous(), N.DTYPE_CODES[grad_out.dtype]
+    return grad_out.contiguous().float(), N.DTYPE_CODES[torch.float32]
+
+
 class _RoiAlignLevels(torch.autograd.Function):
-    """forward: det_roi_align_levels; backward: det_roi_align_levels_backward (gradients w.r.t. the feature maps)."""
+    """forward: det_roi_align_levels_typed; backward: det_roi_align_levels_backward_typed (gradients w.r.t. the feature
+    maps, accumulated in fp32 and returned in each map's dtype)."""
 
     @staticmethod
-    def forward(ctx, boxes, batch_index, level, scales, output_size, sampling_ratio, aligned, *feats):
+    def forward(ctx, boxes, batch_index, level, scales, output_size, sampling_ratio, aligned, code, *feats):
         n, c = feats[0].shape[0], feats[0].shape[1]
         m = boxes.shape[0]
-        out = torch.empty((m, c, output_size[0], output_size[1]), dtype=torch.float32, device=boxes.device)
+        out = torch.empty((m, c, output_size[0], output_size[1]), dtype=feats[0].dtype, device=boxes.device)
         if m:
             lv = _level_table(feats, scales)
             with torch.cuda.device(boxes.device):
-                N.call("det_roi_align_levels", ctypes.cast(lv, ctypes.c_void_p), len(feats), n, c, N.ptr(boxes),
+                N.call("det_roi_align_levels_typed", ctypes.cast(lv, ctypes.c_void_p), len(feats), n, c, N.ptr(boxes),
                        N.ptr(batch_index), N.ptr(level), m, int(output_size[0]), int(output_size[1]), int(sampling_ratio),
-                       int(bool(aligned)), N.ptr(out), N.stream())
+                       int(bool(aligned)), N.ptr(out), code, N.stream())
         ctx.save_for_backward(boxes, batch_index, level if level is not None else torch.empty(0, device=boxes.device))
-        ctx.meta = (scales, output_size, sampling_ratio, aligned, [tuple(f.shape) for f in feats], level is not None)
+        ctx.meta = (scales, output_size, sampling_ratio, aligned, [(tuple(f.shape), f.dtype) for f in feats],
+                    level is not None)
         return out
 
     @staticmethod
     def backward(ctx, grad_out):
         boxes, batch_index, level = ctx.saved_tensors
         scales, output_size, sampling_ratio, aligned, shapes, has_level = ctx.meta
-        grads = [torch.zeros(sh, dtype=torch.float32, device=boxes.device) for sh in shapes]
+        grads = [torch.zeros(sh, dtype=torch.float32, device=boxes.device) for sh, _ in shapes]
         m = boxes.shape[0]
         if m:
-            go = grad_out.contiguous().float()
+            go, gcode = _grad_route(grad_out)
             lv = _level_table(grads, scales)
             with torch.cuda.device(boxes.device):
-                N.call("det_roi_align_levels_backward", ctypes.cast(lv, ctypes.c_void_p), len(grads), shapes[0][0],
-                       shapes[0][1], N.ptr(boxes), N.ptr(batch_index), N.ptr(level if has_level else None), m,
-                       int(output_size[0]), int(output_size[1]), int(sampling_ratio), int(bool(aligned)), N.ptr(go),
-                       N.stream())
-        return (None, None, None, None, None, None, None) + tuple(grads)
+                N.call("det_roi_align_levels_backward_typed", ctypes.cast(lv, ctypes.c_void_p), len(grads),
+                       shapes[0][0][0], shapes[0][0][1], N.ptr(boxes), N.ptr(batch_index),
+                       N.ptr(level if has_level else None), m, int(output_size[0]), int(output_size[1]),
+                       int(sampling_ratio), int(bool(aligned)), N.ptr(go), gcode, N.stream())
+        return (None,) * 8 + tuple(g.to(dt) for g, (_, dt) in zip(grads, shapes))
+
+
+class _RoiPoolLevels(torch.autograd.Function):
+    """forward: det_roi_pool_levels; backward: det_roi_pool_levels_backward.  argmax is written and saved only when some
+    feature map requires grad (inference passes NULL and writes no argmax bytes)."""
+
+    @staticmethod
+    def forward(ctx, boxes, batch_index, level, scales, output_size, code, *feats):
+        n, c = feats[0].shape[0], feats[0].shape[1]
+        m = boxes.shape[0]
+        out = torch.empty((m, c, output_size[0], output_size[1]), dtype=feats[0].dtype, device=boxes.device)
+        argmax = None
+        if any(ctx.needs_input_grad[6:]):
+            argmax = torch.empty(out.shape, dtype=torch.int32, device=boxes.device)
+        if m:
+            lv = _level_table(feats, scales)
+            with torch.cuda.device(boxes.device):
+                N.call("det_roi_pool_levels", ctypes.cast(lv, ctypes.c_void_p), len(feats), n, c, N.ptr(boxes),
+                       N.ptr(batch_index), N.ptr(level), m, int(output_size[0]), int(output_size[1]), N.ptr(out),
+                       N.ptr(argmax), code, N.stream())
+        if argmax is not None:
+            ctx.save_for_backward(batch_index, level if level is not None else torch.empty(0, device=boxes.device),
+                                  argmax)
+        ctx.meta = (scales, output_size, [(tuple(f.shape), f.dtype) for f in feats], level is not None)
+        return out
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        batch_index, level, argmax = ctx.saved_tensors
+        scales, output_size, shapes, has_level = ctx.meta
+        grads = [torch.zeros(sh, dtype=torch.float32, device=grad_out.device) for sh, _ in shapes]
+        m = argmax.shape[0]
+        if m:
+            go, gcode = _grad_route(grad_out)
+            lv = _level_table(grads, scales)
+            with torch.cuda.device(grad_out.device):
+                N.call("det_roi_pool_levels_backward", ctypes.cast(lv, ctypes.c_void_p), len(grads), shapes[0][0][0],
+                       shapes[0][0][1], N.ptr(batch_index), N.ptr(level if has_level else None), m,
+                       int(output_size[0]), int(output_size[1]), N.ptr(argmax), N.ptr(go), gcode, N.stream())
+        return (None,) * 6 + tuple(g.to(dt) for g, (_, dt) in zip(grads, shapes))
+
+
+def _pool_inputs(features: List[torch.Tensor], boxes: torch.Tensor, batch_index: torch.Tensor):
+    """the feature route, shape checks and kernel-ready boxes / batch indices shared by both poolers"""
+    N.require_cuda(boxes, *features)
+    feats, code = _feature_route(features)
+    n, c = feats[0].shape[0], feats[0].shape[1]
+    for f in feats:
+        assert f.dim() == 4 and f.shape[0] == n and f.shape[1] == c, "feature maps must share batch and channels"
+    return feats, code, N.f32c(boxes), batch_index.to(torch.int32).contiguous()
 
 
 def _roi_align_levels(features: List[torch.Tensor], scales: Sequence[float], boxes: torch.Tensor,
                       batch_index: torch.Tensor, level, output_size: Tuple[int, int], sampling_ratio: int,
                       aligned: bool) -> torch.Tensor:
-    N.require_cuda(boxes, *features)
-    feats = [f.to(torch.float32).contiguous() for f in features]  # keeps the autograd graph of the feature maps
-    n, c = feats[0].shape[0], feats[0].shape[1]
-    for f in feats:
-        assert f.dim() == 4 and f.shape[0] == n and f.shape[1] == c, "feature maps must share batch and channels"
-    b = N.f32c(boxes)
-    bi = batch_index.to(torch.int32).contiguous()
+    feats, code, b, bi = _pool_inputs(features, boxes, batch_index)
     out = _RoiAlignLevels.apply(b, bi, level, tuple(float(s) for s in scales), tuple(output_size), int(sampling_ratio),
-                                bool(aligned), *feats)
-    # the kernels compute in fp32; the result carries the feature maps' dtype like torchvision.ops.roi_align's does
-    return out if features[0].dtype == torch.float32 else out.to(features[0].dtype)
+                                bool(aligned), code, *feats)
+    # the result carries the feature maps' dtype like torchvision.ops.roi_align's does (fp32 route: cast back)
+    return out if out.dtype == features[0].dtype else out.to(features[0].dtype)
+
+
+def _roi_pool_levels(features: List[torch.Tensor], scales: Sequence[float], boxes: torch.Tensor,
+                     batch_index: torch.Tensor, level, output_size: Tuple[int, int]) -> torch.Tensor:
+    feats, code, b, bi = _pool_inputs(features, boxes, batch_index)
+    out = _RoiPoolLevels.apply(b, bi, level, tuple(float(s) for s in scales), tuple(output_size), code, *feats)
+    return out if out.dtype == features[0].dtype else out.to(features[0].dtype)
 
 
 class ROIAlign:
@@ -132,14 +208,10 @@ class ROIPooler:
             output_size = (output_size, output_size)
         assert len(output_size) == 2 and isinstance(output_size[0], int) and isinstance(output_size[1], int)
         self.output_size = (output_size[0], output_size[1])
-        if type == "ROIAlign":
-            self.aligned = False
-        elif type == "ROIAlignV2":
-            self.aligned = True
-        elif type == "ROIPool":
-            raise NotImplementedError("ROIPool (max pooling) is not part of this build; use ROIAlign / ROIAlignV2")
-        else:
+        if type not in ("ROIAlign", "ROIAlignV2", "ROIPool"):
             raise ValueError("Unknown pooler type: {}".format(type))
+        self.type = type
+        self.aligned = type == "ROIAlignV2"  # ROIAlign: legacy half-pixel-free sampling; ROIPool: not used
         self.scales = [float(s) for s in scales]
         self.sampling_ratio = int(sampling_ratio)
         min_level, max_level = -(math.log2(scales[0])), -(math.log2(scales[-1]))
@@ -173,6 +245,8 @@ class ROIPooler:
         if nl > 1:
             level = assign_boxes_to_levels(ts, self.min_level, self.max_level, self.canonical_box_size,
                                            self.canonical_level)
+        if self.type == "ROIPool":
+            return _roi_pool_levels(x, self.scales, boxes, batch_index, level, self.output_size)
         return _roi_align_levels(x, self.scales, boxes, batch_index, level, self.output_size, self.sampling_ratio,
                                  self.aligned)
 
