@@ -8,7 +8,6 @@
 //   python/src/models/rpn.py:187-244 + components/box_regression.py:128-168   losses (BCE-with-logits + L1/smooth-L1)
 // The (G,R) IoU matrix, the (N,R,4) matched-gt tensor and the (N,R,4) target-delta tensor of the reference are
 // never materialised: IoUs are recomputed from the box tables, targets are encoded on the fly for positives only.
-#include <stdlib.h>
 #include "common.cuh"
 #include "peer.cuh"
 #include "assign.cuh"
@@ -1042,15 +1041,8 @@ int launch_subsample_lazy(const float* gt_boxes, const int32_t* gt_offsets, cons
     return DET_OK;
 }
 
-// CTAs per SM of the dense loss kernel's grid-stride launch (DET_LOSS_GRID overrides it for measurements)
-static int loss_grid_factor() {
-    static const int f = [] {
-        const char* v = getenv("DET_LOSS_GRID");
-        const int x = v ? atoi(v) : 0;
-        return x > 0 ? x : 16;
-    }();
-    return f;
-}
+// CTAs per SM of the dense loss kernel's grid-stride launch
+constexpr int kLossGridFactor = 16;
 
 extern "C" {
 
@@ -1203,7 +1195,7 @@ int det_rpn_loss(const float* logits, const float* deltas, const int8_t* labels,
     const int64_t total = (int64_t)n * r;
     const int64_t nwarps = (total + 127) / 128;
     int64_t blocks = (nwarps + kLossThreads / 32 - 1) / (kLossThreads / 32);
-    const int64_t cap = (int64_t)sm_count() * loss_grid_factor();
+    const int64_t cap = (int64_t)sm_count() * kLossGridFactor;
     if (blocks > cap) blocks = cap;
     auto g4 = reinterpret_cast<const float4*>(gt_boxes);
     auto a4 = reinterpret_cast<const float4*>(anchors);

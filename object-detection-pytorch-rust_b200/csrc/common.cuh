@@ -60,7 +60,6 @@ static inline float float_threshold_below(double thr) {
 // semantics are unchanged as long as a kernel touches global memory only after pdl_wait().  pdl_trigger() (first
 // statement of a kernel) lets the NEXT launch_pdl() kernel in the stream start that early; after a kernel that never
 // triggers (any foreign kernel, a copy) the launch simply behaves like <<<>>>.  The edges survive stream capture.
-bool pdl_enabled();  // core.cu: false when DET_NO_PDL=1 is set in the environment (A/B measurements)
 template <typename... KArgs, typename... Args>
 static inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
                                      Args&&... args) {
@@ -73,7 +72,7 @@ static inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 b
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = pdl_enabled() ? 1 : 0;
+    cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 

@@ -1,5 +1,4 @@
 // Error plumbing and device queries for libdet_b200.so.
-#include <stdlib.h>
 #include "common.cuh"
 #include <stdarg.h>
 #include <stdio.h>
@@ -18,14 +17,6 @@ void set_error(const char* fmt, ...) {
 int cuda_fail(cudaError_t e, const char* what) {
     set_error("CUDA error in %s: %s (%d)", what, cudaGetErrorString(e), (int)e);
     return DET_ERR_CUDA;
-}
-
-bool pdl_enabled() {
-    static const bool on = [] {
-        const char* v = getenv("DET_NO_PDL");
-        return !(v && v[0] == '1');
-    }();
-    return on;
 }
 
 int sm_count() {

@@ -65,14 +65,14 @@ struct FlatArgs {
     int32_t* overflow_flag;  // cleared here (first thread of the grid); the NMS kernel behind this one sets it
 };
 
-template <int MODE, int TH = kFlatThreads, typename T = float>
-__global__ void __launch_bounds__(TH) dense_decode_flat_kernel(const __grid_constant__ FlatArgs g) {
+template <int MODE, typename T>
+__global__ void __launch_bounds__(kFlatThreads) dense_decode_flat_kernel(const __grid_constant__ FlatArgs g) {
     using V = typename Head<T>::vec;  // 4 positions of one plane: 16 bytes (fp32) or 8 bytes (bf16 / fp16)
     if (MODE != kModeDense) {
         pdl_trigger();  // det_dense_detect: the NMS kernel's CTAs may move in as SM slots free up
         if (blockIdx.x == 0 && threadIdx.x == 0 && g.overflow_flag) *g.overflow_flag = 0;
     }
-    long long gt = (long long)blockIdx.x * TH + threadIdx.x;
+    long long gt = (long long)blockIdx.x * kFlatThreads + threadIdx.x;
     bool active = gt < g.thread_begin[g.num_levels];
     if (MODE == kModeDense) {
         if (!active) return;
@@ -372,14 +372,12 @@ static int launch_detect_nms_t(const SelectArgs& sel, int n, float thr_f, int mo
                                float* det_boxes, float* det_scores, int64_t* det_classes, int32_t* det_count,
                                int32_t* overflow_flag, cudaStream_t st) {
     const size_t smem = sizeof(DetectSmem<CAP, T>);
-    static const int use_fast = [] { const char* v = getenv("DET_NO_FAST_NMS"); return (v && v[0] == '1') ? 0 : 1; }();
     cudaError_t e = cudaFuncSetAttribute(dense_detect_nms_kernel<CAP, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(dense_detect_nms_kernel)");
     // programmatic dependent launch: the CTAs take their SM slots while the select kernel drains (see common.cuh)
     e = launch_pdl(dense_detect_nms_kernel<CAP, T>, dim3(n), dim3(T), smem, st, sel.cand_count, sel.cand_box, sel.cand_score,
                    sel.cand_cls, sel.cand_id, sel.cand_cap, thr_f, mode, max_det, det_idx,
-                   reinterpret_cast<float4*>(det_boxes), det_scores, det_classes, det_count, overflow_flag, nullptr, nullptr,
-                   use_fast);
+                   reinterpret_cast<float4*>(det_boxes), det_scores, det_classes, det_count, overflow_flag, nullptr, nullptr);
     if (e != cudaSuccess) return cuda_fail(e, "dense_detect_nms_kernel");
     return DET_OK;
 }
@@ -438,21 +436,12 @@ static int launch_flat(const det_dense_level_t* levels_host, int num_levels, int
     }
     for (int l = num_levels; l <= kMaxLevels; ++l) f.thread_begin[l] = tb;
     if (tb == 0) return DET_OK;
-    static const int th_env = [] { const char* v = getenv("DET_FLAT_THREADS"); return v ? atoi(v) : 0; }();
-    const int th = (th_env == 256 || th_env == 512) ? th_env : kFlatThreads;
-    const long long blocks = (tb + th - 1) / th;
+    const long long blocks = (tb + kFlatThreads - 1) / kFlatThreads;
     DET_CHECK_ARG(blocks < (1ll << 31), "too many positions");
-    if (!sel) {
-        if (th == 256) dense_decode_flat_kernel<kModeDense, 256, T><<<(unsigned)blocks, 256, 0, st>>>(f);
-        else if (th == 512) dense_decode_flat_kernel<kModeDense, 512, T><<<(unsigned)blocks, 512, 0, st>>>(f);
-        else dense_decode_flat_kernel<kModeDense, kFlatThreads, T><<<(unsigned)blocks, kFlatThreads, 0, st>>>(f);
-    } else if (sel->mode == kModeSelectGated) {
-        dense_decode_flat_kernel<kModeSelectGated, kFlatThreads, T><<<(unsigned)blocks, kFlatThreads, 0, st>>>(f);
-    } else {
-        if (th == 256) dense_decode_flat_kernel<kModeSelect, 256, T><<<(unsigned)blocks, 256, 0, st>>>(f);
-        else if (th == 512) dense_decode_flat_kernel<kModeSelect, 512, T><<<(unsigned)blocks, 512, 0, st>>>(f);
-        else dense_decode_flat_kernel<kModeSelect, kFlatThreads, T><<<(unsigned)blocks, kFlatThreads, 0, st>>>(f);
-    }
+    const unsigned grid = (unsigned)blocks;
+    if (!sel) dense_decode_flat_kernel<kModeDense, T><<<grid, kFlatThreads, 0, st>>>(f);
+    else if (sel->mode == kModeSelectGated) dense_decode_flat_kernel<kModeSelectGated, T><<<grid, kFlatThreads, 0, st>>>(f);
+    else dense_decode_flat_kernel<kModeSelect, T><<<grid, kFlatThreads, 0, st>>>(f);
     DET_LAUNCH_OK("dense_decode_flat_kernel");
     return DET_OK;
 }

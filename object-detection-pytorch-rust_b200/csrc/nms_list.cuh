@@ -513,7 +513,7 @@ dense_detect_nms_kernel(int32_t* cand_count, const float4* __restrict__ cand_box
                         int64_t* __restrict__ det_idx, float4* __restrict__ det_boxes, float* __restrict__ det_scores,
                         int64_t* __restrict__ det_classes, int32_t* __restrict__ det_count,
                         int32_t* __restrict__ overflow_flag, const FullStats* __restrict__ ext_full = nullptr,
-                        int32_t* __restrict__ todo = nullptr, int use_fast = 1) {
+                        int32_t* __restrict__ todo = nullptr) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     DetectSmem<CAP, T>& sm = *reinterpret_cast<DetectSmem<CAP, T>*>(smem_raw);
     using KL = KeyLayout<kSmallIdxBits>;
@@ -522,7 +522,7 @@ dense_detect_nms_kernel(int32_t* cand_count, const float4* __restrict__ cand_box
     DET_MARK(0);
     FastFirst first;
     first.b = make_float4(0.f, 0.f, 0.f, 0.f); first.s = 0.f; first.c = 0; first.id = 0;
-    if (!ext_full && use_fast && tid < cand_cap) {  // in flight together with the count
+    if (!ext_full && tid < cand_cap) {  // in flight together with the count
         const int64_t o = (int64_t)img * cand_cap + tid;
         first.b = cand_box[o]; first.s = cand_score[o]; first.c = cand_cls[o]; first.id = cand_id[o];
     }
@@ -545,7 +545,7 @@ dense_detect_nms_kernel(int32_t* cand_count, const float4* __restrict__ cand_box
     const int64_t base = (int64_t)img * cand_cap;
     const int cap_out = (int)min(max_det, (int64_t)CAP);
     const int lane = tid & 31, wid = tid >> 5;
-    if (!ext_full && use_fast) {
+    if (!ext_full) {
         static_assert(sizeof(DetectFastSmem<CAP>) <= sizeof(DetectSmem<CAP, T>), "the fast form lives in the same shared memory");
         const int r = detect_fast<CAP, T>(*reinterpret_cast<DetectFastSmem<CAP>*>(smem_raw), cnt, cand_box + base,
                                           cand_score + base, cand_cls + base, cand_id + base, thr_f, mode, cap_out,

@@ -84,9 +84,8 @@ rpn_select_kernel(const float* __restrict__ logits, int64_t r, int64_t mp, Level
     const float* lg = logits + (int64_t)img * r;
     uint64_t* out = keys + (int64_t)img * mp;
     // grid (images, levels): one CTA per (image, level) -- the levels of an image are independent selections into
-    // disjoint ranges of the compact row; blockIdx.y = 0 (the largest level of a pyramid) is dispatched first.  (With
-    // DET_RPN_SELECT_SPLIT=0 one CTA per image walks the levels: 0.199 / 0.256 / 0.560 ms per 16 / 64 / 256 images
-    // against 0.179 / 0.237 / 0.541 ms.)
+    // disjoint ranges of the compact row; blockIdx.y = 0 (the largest level of a pyramid) is dispatched first.  (One CTA
+    // per image walking the levels took 0.199 / 0.256 / 0.560 ms per 16 / 64 / 256 images against 0.179 / 0.237 / 0.541.)
     if (blockIdx.y == 0) {
         if (tid == 0) {
             LargeImg li;
@@ -97,190 +96,187 @@ rpn_select_kernel(const float* __restrict__ logits, int64_t r, int64_t mp, Level
         }
         for (int64_t j = ct.off[ct.num_levels] + tid; j < len1; j += T) out[j] = kSentinelKey;
     }
-    for (int l = blockIdx.y; l < lt.num_levels; l += gridDim.y) {
-        const int64_t i0 = lt.off[l], size = lt.off[l + 1] - i0;
-        const int take = (int)(ct.off[l + 1] - ct.off[l]);
-        if (take == 0) continue;
-        // cut: keys with score key < cut are in; in tie mode those == cut only while `tie_want` lasts (index order),
-        // otherwise every key <= cut is in
-        uint32_t cut = 0xffffffffu;
-        bool tie_mode = false;
-        int tie_want = 0;
-        const bool staged = take < size && size <= (int64_t)stage_cap;
-        auto count_top_byte = [&](bool valid, uint32_t key) {
-            // (counting lanes that share a bin with one atomic -- match.any -- was measured slower than letting the
-            //  shared-memory atomics serialise: 82 vs 58 us per 64 images with one CTA per image)
-            if (valid) atomicAdd(&hist[key >> 24], 1u);
-        };
-        if (staged) {
-            // one pass over the level: keys into the staging area + the histogram of the first radix pass, eight
-            // loads of a thread in flight together
-            const int sz = (int)size;
-            const float* lgl = lg + i0;
-            for (int b = tid; b < 256; b += T) hist[b] = 0u;
-            __syncthreads();  // (also: the previous level is done with the staging area)
-            for (int base = 0; base < sz; base += 8 * T) {
-                uint32_t kk[8];
+    const int l = blockIdx.y;
+    const int64_t i0 = lt.off[l], size = lt.off[l + 1] - i0;
+    const int take = (int)(ct.off[l + 1] - ct.off[l]);
+    if (take == 0) return;
+    // cut: keys with score key < cut are in; in tie mode those == cut only while `tie_want` lasts (index order),
+    // otherwise every key <= cut is in
+    uint32_t cut = 0xffffffffu;
+    bool tie_mode = false;
+    int tie_want = 0;
+    const bool staged = take < size && size <= (int64_t)stage_cap;
+    auto count_top_byte = [&](bool valid, uint32_t key) {
+        // (counting lanes that share a bin with one atomic -- match.any -- was measured slower than letting the
+        //  shared-memory atomics serialise: 82 vs 58 us per 64 images with one CTA per image)
+        if (valid) atomicAdd(&hist[key >> 24], 1u);
+    };
+    if (staged) {
+        // one pass over the level: keys into the staging area + the histogram of the first radix pass, eight
+        // loads of a thread in flight together
+        const int sz = (int)size;
+        const float* lgl = lg + i0;
+        for (int b = tid; b < 256; b += T) hist[b] = 0u;
+        __syncthreads();
+        for (int base = 0; base < sz; base += 8 * T) {
+            uint32_t kk[8];
 #pragma unroll
-                for (int u = 0; u < 8; ++u) {
-                    const int i = base + u * T + tid;
-                    kk[u] = i < sz ? score_desc_key(lgl[i]) : 0u;
-                }
+            for (int u = 0; u < 8; ++u) {
+                const int i = base + u * T + tid;
+                kk[u] = i < sz ? score_desc_key(lgl[i]) : 0u;
+            }
 #pragma unroll
-                for (int u = 0; u < 8; ++u) {
-                    const int i = base + u * T + tid;
-                    if (i < sz) {
-                        staged_keys[i] = kk[u];
-                        atomicAdd(&hist[kk[u] >> 24], 1u);
-                    }
+            for (int u = 0; u < 8; ++u) {
+                const int i = base + u * T + tid;
+                if (i < sz) {
+                    staged_keys[i] = kk[u];
+                    atomicAdd(&hist[kk[u] >> 24], 1u);
                 }
             }
-            if (tid == 0) {
-                s_prefix = 0u;
-                s_want = take;
-                s_done = 0;
-                s_slot = 0;
+        }
+        if (tid == 0) {
+            s_prefix = 0u;
+            s_want = take;
+            s_done = 0;
+            s_slot = 0;
+        }
+        // the remaining passes and the compaction read the copy four keys at a time
+        const uint4* s4 = reinterpret_cast<const uint4*>(staged_keys);
+        const int n4 = sz >> 2;
+        for (int shift = 24; shift >= 0; shift -= 8) {
+            if (shift != 24) {
+                for (int b = tid; b < 256; b += T) hist[b] = 0u;
+                __syncthreads();
+                if (s_done) break;
+                const uint32_t prefix = s_prefix, himask = 0xffffffffu << (shift + 8);
+                for (int j = tid; j < n4; j += T) {
+                    const uint4 v = s4[j];
+                    if ((v.x & himask) == prefix) atomicAdd(&hist[(v.x >> shift) & 255u], 1u);
+                    if ((v.y & himask) == prefix) atomicAdd(&hist[(v.y >> shift) & 255u], 1u);
+                    if ((v.z & himask) == prefix) atomicAdd(&hist[(v.z >> shift) & 255u], 1u);
+                    if ((v.w & himask) == prefix) atomicAdd(&hist[(v.w >> shift) & 255u], 1u);
+                }
+                if (tid < (sz & 3)) {
+                    const uint32_t key = staged_keys[(n4 << 2) + tid];
+                    if ((key & himask) == prefix) atomicAdd(&hist[(key >> shift) & 255u], 1u);
+                }
             }
-            // the remaining passes and the compaction read the copy four keys at a time
-            const uint4* s4 = reinterpret_cast<const uint4*>(staged_keys);
-            const int n4 = sz >> 2;
-            for (int shift = 24; shift >= 0; shift -= 8) {
-                if (shift != 24) {
-                    for (int b = tid; b < 256; b += T) hist[b] = 0u;
-                    __syncthreads();
-                    if (s_done) break;
-                    const uint32_t prefix = s_prefix, himask = 0xffffffffu << (shift + 8);
-                    for (int j = tid; j < n4; j += T) {
-                        const uint4 v = s4[j];
-                        if ((v.x & himask) == prefix) atomicAdd(&hist[(v.x >> shift) & 255u], 1u);
-                        if ((v.y & himask) == prefix) atomicAdd(&hist[(v.y >> shift) & 255u], 1u);
-                        if ((v.z & himask) == prefix) atomicAdd(&hist[(v.z >> shift) & 255u], 1u);
-                        if ((v.w & himask) == prefix) atomicAdd(&hist[(v.w >> shift) & 255u], 1u);
-                    }
-                    if (tid < (sz & 3)) {
-                        const uint32_t key = staged_keys[(n4 << 2) + tid];
+            __syncthreads();
+            if (wid == 0) radix_decide(hist, lane, shift, &s_prefix, &s_want, &s_done);
+            __syncthreads();
+        }
+        __syncthreads();
+        cut = s_prefix;
+        tie_mode = s_done == 0;
+        tie_want = s_want;
+        if (!tie_mode) {
+            const uint64_t lvl = (uint64_t)l << KLL::kSegShift;
+            uint64_t* o = out + ct.off[l];
+            const uint32_t a0 = (uint32_t)i0;
+            const unsigned lt_mask = (1u << lane) - 1u;
+            for (int j0 = 0; j0 < n4; j0 += T) {
+                const int j = j0 + tid;
+                uint4 v = make_uint4(0xffffffffu, 0xffffffffu, 0xffffffffu, 0xffffffffu);
+                if (j < n4) v = s4[j];
+                const bool i0n = j < n4 && v.x <= cut, i1n = j < n4 && v.y <= cut, i2n = j < n4 && v.z <= cut,
+                           i3n = j < n4 && v.w <= cut;
+                const unsigned b0 = __ballot_sync(0xffffffffu, i0n), b1 = __ballot_sync(0xffffffffu, i1n),
+                               b2 = __ballot_sync(0xffffffffu, i2n), b3 = __ballot_sync(0xffffffffu, i3n);
+                const int c0 = __popc(b0), c1 = __popc(b1), c2 = __popc(b2), c3 = __popc(b3);
+                if (c0 + c1 + c2 + c3 == 0) continue;  // warp-uniform
+                int pos = 0;
+                if (lane == 0) pos = atomicAdd(&s_slot, c0 + c1 + c2 + c3);
+                pos = __shfl_sync(0xffffffffu, pos, 0);
+                const uint32_t a = a0 + (uint32_t)(j << 2);
+                int q = pos + __popc(b0 & lt_mask);
+                if (i0n && q < take) o[q] = lvl | ((uint64_t)v.x << KLL::kScoreShift) | (uint64_t)a;
+                q = pos + c0 + __popc(b1 & lt_mask);
+                if (i1n && q < take) o[q] = lvl | ((uint64_t)v.y << KLL::kScoreShift) | (uint64_t)(a + 1u);
+                q = pos + c0 + c1 + __popc(b2 & lt_mask);
+                if (i2n && q < take) o[q] = lvl | ((uint64_t)v.z << KLL::kScoreShift) | (uint64_t)(a + 2u);
+                q = pos + c0 + c1 + c2 + __popc(b3 & lt_mask);
+                if (i3n && q < take) o[q] = lvl | ((uint64_t)v.w << KLL::kScoreShift) | (uint64_t)(a + 3u);
+            }
+            if (tid < (sz & 3)) {
+                const int i = (n4 << 2) + tid;
+                const uint32_t key = staged_keys[i];
+                if (key <= cut) {
+                    const int q = atomicAdd(&s_slot, 1);
+                    if (q < take) o[q] = lvl | ((uint64_t)key << KLL::kScoreShift) | (uint64_t)(a0 + (uint32_t)i);
+                }
+            }
+            return;
+        }
+        // ties at the cut: the index-ordered walk below (cut / tie_mode / tie_want are set)
+    }
+    auto key_at = [&](int64_t i) -> uint32_t { return staged ? staged_keys[i] : score_desc_key(lg[i0 + i]); };
+    if (take < size && !staged) {
+        // radix select of the take-th best 32-bit descending-logit key, one byte per pass
+        if (tid == 0) {
+            s_prefix = 0u;
+            s_want = take;
+            s_done = 0;
+        }
+        for (int shift = 24; shift >= 0; shift -= 8) {
+            {
+                for (int b = tid; b < 256; b += T) hist[b] = 0u;
+                __syncthreads();
+                if (s_done) break;
+                const uint32_t prefix = s_prefix, himask = (shift == 24) ? 0u : (0xffffffffu << (shift + 8));
+                if (shift == 24) {
+                    for (int64_t base = 0; base < size; base += T)
+                        count_top_byte(base + tid < size, base + tid < size ? key_at(base + tid) : 0u);
+                } else {
+                    for (int64_t i = tid; i < size; i += T) {
+                        const uint32_t key = key_at(i);
                         if ((key & himask) == prefix) atomicAdd(&hist[(key >> shift) & 255u], 1u);
                     }
                 }
                 __syncthreads();
-                if (wid == 0) radix_decide(hist, lane, shift, &s_prefix, &s_want, &s_done);
-                __syncthreads();
             }
+            if (wid == 0) radix_decide(hist, lane, shift, &s_prefix, &s_want, &s_done);
             __syncthreads();
-            cut = s_prefix;
-            tie_mode = s_done == 0;
-            tie_want = s_want;
-            if (!tie_mode) {
-                const uint64_t lvl = (uint64_t)l << KLL::kSegShift;
-                uint64_t* o = out + ct.off[l];
-                const uint32_t a0 = (uint32_t)i0;
-                const unsigned lt_mask = (1u << lane) - 1u;
-                for (int j0 = 0; j0 < n4; j0 += T) {
-                    const int j = j0 + tid;
-                    uint4 v = make_uint4(0xffffffffu, 0xffffffffu, 0xffffffffu, 0xffffffffu);
-                    if (j < n4) v = s4[j];
-                    const bool i0n = j < n4 && v.x <= cut, i1n = j < n4 && v.y <= cut, i2n = j < n4 && v.z <= cut,
-                               i3n = j < n4 && v.w <= cut;
-                    const unsigned b0 = __ballot_sync(0xffffffffu, i0n), b1 = __ballot_sync(0xffffffffu, i1n),
-                                   b2 = __ballot_sync(0xffffffffu, i2n), b3 = __ballot_sync(0xffffffffu, i3n);
-                    const int c0 = __popc(b0), c1 = __popc(b1), c2 = __popc(b2), c3 = __popc(b3);
-                    if (c0 + c1 + c2 + c3 == 0) continue;  // warp-uniform
-                    int pos = 0;
-                    if (lane == 0) pos = atomicAdd(&s_slot, c0 + c1 + c2 + c3);
-                    pos = __shfl_sync(0xffffffffu, pos, 0);
-                    const uint32_t a = a0 + (uint32_t)(j << 2);
-                    int q = pos + __popc(b0 & lt_mask);
-                    if (i0n && q < take) o[q] = lvl | ((uint64_t)v.x << KLL::kScoreShift) | (uint64_t)a;
-                    q = pos + c0 + __popc(b1 & lt_mask);
-                    if (i1n && q < take) o[q] = lvl | ((uint64_t)v.y << KLL::kScoreShift) | (uint64_t)(a + 1u);
-                    q = pos + c0 + c1 + __popc(b2 & lt_mask);
-                    if (i2n && q < take) o[q] = lvl | ((uint64_t)v.z << KLL::kScoreShift) | (uint64_t)(a + 2u);
-                    q = pos + c0 + c1 + c2 + __popc(b3 & lt_mask);
-                    if (i3n && q < take) o[q] = lvl | ((uint64_t)v.w << KLL::kScoreShift) | (uint64_t)(a + 3u);
-                }
-                if (tid < (sz & 3)) {
-                    const int i = (n4 << 2) + tid;
-                    const uint32_t key = staged_keys[i];
-                    if (key <= cut) {
-                        const int q = atomicAdd(&s_slot, 1);
-                        if (q < take) o[q] = lvl | ((uint64_t)key << KLL::kScoreShift) | (uint64_t)(a0 + (uint32_t)i);
-                    }
-                }
-                __syncthreads();
-                continue;
-            }
-            // ties at the cut: the index-ordered walk below (cut / tie_mode / tie_want are set)
-        }
-        auto key_at = [&](int64_t i) -> uint32_t { return staged ? staged_keys[i] : score_desc_key(lg[i0 + i]); };
-        if (take < size && !staged) {
-            // radix select of the take-th best 32-bit descending-logit key, one byte per pass
-            if (tid == 0) {
-                s_prefix = 0u;
-                s_want = take;
-                s_done = 0;
-            }
-            for (int shift = 24; shift >= 0; shift -= 8) {
-                {
-                    for (int b = tid; b < 256; b += T) hist[b] = 0u;
-                    __syncthreads();
-                    if (s_done) break;
-                    const uint32_t prefix = s_prefix, himask = (shift == 24) ? 0u : (0xffffffffu << (shift + 8));
-                    if (shift == 24) {
-                        for (int64_t base = 0; base < size; base += T)
-                            count_top_byte(base + tid < size, base + tid < size ? key_at(base + tid) : 0u);
-                    } else {
-                        for (int64_t i = tid; i < size; i += T) {
-                            const uint32_t key = key_at(i);
-                            if ((key & himask) == prefix) atomicAdd(&hist[(key >> shift) & 255u], 1u);
-                        }
-                    }
-                    __syncthreads();
-                }
-                if (wid == 0) radix_decide(hist, lane, shift, &s_prefix, &s_want, &s_done);
-                __syncthreads();
-            }
-            __syncthreads();
-            cut = s_prefix;
-            // not done after the last byte: several anchors share the cut logit and only s_want of them fit -- the
-            // reference's stable sort keeps the lower indices
-            tie_mode = s_done == 0;
-            tie_want = s_want;
-        }
-        if (tid == 0) s_slot = 0;
-        __syncthreads();
-        const uint64_t lvl = (uint64_t)l << KLL::kSegShift;
-        int tie_seen = 0;  // equal-logit anchors already passed, in index order (block-uniform)
-        for (int64_t base = 0; base < size; base += T) {
-            const int64_t i = base + tid;
-            uint32_t k32 = 0xffffffffu;
-            bool in = false, eq = false;
-            if (i < size) {
-                k32 = key_at(i);
-                in = tie_mode ? (k32 < cut) : (k32 <= cut);
-                eq = tie_mode && k32 == cut;
-            }
-            if (tie_mode) {  // block-uniform branch: rank the equal keys of this step in index order
-                const unsigned be = __ballot_sync(0xffffffffu, eq);
-                if (lane == 0) s_warp[wid] = __popc(be);
-                __syncthreads();
-                int before = tie_seen, total = 0;
-                for (int w = 0; w < T / 32; ++w) {
-                    const int v = s_warp[w];
-                    before += (w < wid) ? v : 0;
-                    total += v;
-                }
-                if (eq && before + __popc(be & ((1u << lane) - 1u)) < tie_want) in = true;
-                tie_seen += total;
-                __syncthreads();
-            }
-            const unsigned bal = __ballot_sync(0xffffffffu, in);
-            int pos = 0;
-            if (lane == 0 && bal) pos = atomicAdd(&s_slot, __popc(bal));
-            pos = __shfl_sync(0xffffffffu, pos, 0) + __popc(bal & ((1u << lane) - 1u));
-            if (in && pos < take)
-                out[ct.off[l] + pos] = lvl | ((uint64_t)k32 << KLL::kScoreShift) | (uint64_t)(uint32_t)(i0 + i);
         }
         __syncthreads();
+        cut = s_prefix;
+        // not done after the last byte: several anchors share the cut logit and only s_want of them fit -- the
+        // reference's stable sort keeps the lower indices
+        tie_mode = s_done == 0;
+        tie_want = s_want;
+    }
+    if (tid == 0) s_slot = 0;
+    __syncthreads();
+    const uint64_t lvl = (uint64_t)l << KLL::kSegShift;
+    int tie_seen = 0;  // equal-logit anchors already passed, in index order (block-uniform)
+    for (int64_t base = 0; base < size; base += T) {
+        const int64_t i = base + tid;
+        uint32_t k32 = 0xffffffffu;
+        bool in = false, eq = false;
+        if (i < size) {
+            k32 = key_at(i);
+            in = tie_mode ? (k32 < cut) : (k32 <= cut);
+            eq = tie_mode && k32 == cut;
+        }
+        if (tie_mode) {  // block-uniform branch: rank the equal keys of this step in index order
+            const unsigned be = __ballot_sync(0xffffffffu, eq);
+            if (lane == 0) s_warp[wid] = __popc(be);
+            __syncthreads();
+            int before = tie_seen, total = 0;
+            for (int w = 0; w < T / 32; ++w) {
+                const int v = s_warp[w];
+                before += (w < wid) ? v : 0;
+                total += v;
+            }
+            if (eq && before + __popc(be & ((1u << lane) - 1u)) < tie_want) in = true;
+            tie_seen += total;
+            __syncthreads();
+        }
+        const unsigned bal = __ballot_sync(0xffffffffu, in);
+        int pos = 0;
+        if (lane == 0 && bal) pos = atomicAdd(&s_slot, __popc(bal));
+        pos = __shfl_sync(0xffffffffu, pos, 0) + __popc(bal & ((1u << lane) - 1u));
+        if (in && pos < take)
+            out[ct.off[l] + pos] = lvl | ((uint64_t)k32 << KLL::kScoreShift) | (uint64_t)(uint32_t)(i0 + i);
     }
 }
 
@@ -723,13 +719,10 @@ int det_rpn_proposals(const float* boxes, const float* logits, int n, int64_t r,
     // measured: 45.8 us instead of 54.8 us for 64 images but 163 us instead of 140 us for 256 (ten cluster barriers per CTA); a
     // second form with two visits per key (keys below the cut's top byte written at once, the rest listed) executed MORE
     // instructions than these seven tight visits (336 k vs 292 k warp-instructions per image) -- both rejected.
-    static const int sel_split = [] { const char* v = getenv("DET_RPN_SELECT_SPLIT"); return v ? atoi(v) : 1; }();
-    const unsigned sel_y = sel_split ? (unsigned)num_levels : 1u;
-    rpn_select_kernel<<<dim3((unsigned)n, sel_y), 1024, (size_t)(stage * 4), st>>>(logits, r, mp, lt, ct, len1, ws.info, ws.keys_a, (int)stage);
+    rpn_select_kernel<<<dim3((unsigned)n, (unsigned)num_levels), 1024, (size_t)(stage * 4), st>>>(logits, r, mp, lt, ct, len1, ws.info, ws.keys_a, (int)stage);
     DET_LAUNCH_OK("rpn_select_kernel");
-    static const bool old_sorts = [] { const char* v = getenv("DET_RPN_OLD_SORTS"); return v && v[0] == '1'; }();
     uint64_t* sorted;
-    if (!old_sorts && std::min(*std::max_element(level_sizes_host, level_sizes_host + num_levels), pre_nms_topk) <= kTile) {
+    if (std::min(*std::max_element(level_sizes_host, level_sizes_host + num_levels), pre_nms_topk) <= kTile) {
         rpn_sort_levels_kernel<<<dim3((unsigned)num_levels, (unsigned)n), kLevelSortThreads, 0, st>>>(ws.keys_a, mp, ct);
         sorted = ws.keys_a;
     } else {
@@ -759,7 +752,7 @@ int det_rpn_proposals(const float* boxes, const float* logits, int n, int64_t r,
     if (status != DET_OK) return status;
     int64_t kept_bound = 0;
     for (int l = 0; l < num_levels; ++l) kept_bound += std::min({level_sizes_host[l], pre_nms_topk, post_nms_topk});
-    if (!old_sorts && kept_bound * 8 <= 200 * 1024) {  // the kept keys of an image fit into shared memory
+    if (kept_bound * 8 <= 200 * 1024) {  // the kept keys of an image fit into shared memory
         const size_t smem = (size_t)kept_bound * 8;
         if (smem > 40 * 1024) {  // (static + dynamic share the 48 KB default)
             cudaError_t ea = cudaFuncSetAttribute(rpn_finish_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

@@ -20,10 +20,8 @@ g = torch.Generator(device="cuda").manual_seed(3)
 hs = [torch.randn(n, 3 * (5 + C), 640 // s, 640 // s, device="cuda", generator=g) for s in strides]
 for h in hs:
     h.view(n, 3, 5 + C, h.shape[2], h.shape[3])[:, :, 4] -= 4.0
-FAST = os.environ.get("DET_NO_FAST_NMS") != "1"
-names = {0: "start", 1: "keys+stats", 2: "counting sort", 3: "gather+file", 6: "suppressors (own category)", 4: "pairs across categories", 5: "rounds", 14: "output"} if FAST else {0: "start", 1: "row-order sort", 4: "0 trick stats", 5: "1 keys", 6: "2 sort", 7: "3 gather+segments", 8: "classify",
-         9: "4a tiny pairs", 10: "4a resolve", 11: "4b/4c mid+long", 12: "5 re-key", 13: "5 sort", 14: "output"}
-order = [0, 1, 2, 3, 6, 4, 5, 14] if FAST else [0, 1, 4, 5, 6, 7, 8, 9, 10, 11, 12, 13, 14]
+names = {0: "start", 1: "keys+stats", 2: "counting sort", 3: "gather+file", 6: "suppressors (own category)", 4: "pairs across categories", 5: "rounds", 14: "output"}
+order = [0, 1, 2, 3, 6, 4, 5, 14]
 for thr, cap in ((0.1, 2048), (0.25, 1024)):
     for _ in range(3):
         r = dh.detect_thresholded(hs, thr, 0.5, max_det=300, cand_cap=cap, check=False)

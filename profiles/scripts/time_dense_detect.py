@@ -1,5 +1,5 @@
 """det_dense_detect (decode + threshold + per-class NMS + top 300) at the bench's settings, graph-replayed: ms per batch and
-the fraction of the HBM copy peak.  DET_NO_FAST_NMS=1 runs the general NMS body for comparison."""
+the fraction of the HBM copy peak."""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "object-detection-pytorch-rust_b200"))

@@ -21,4 +21,4 @@ logits = torch.randn(nb, R, device=dev); deltas = torch.randn(nb, R, 4, device=d
 gl, gd = torch.empty_like(logits), torch.empty_like(deltas)
 ms = time_region(lambda: rpn._run_loss(anchors, logits, deltas, asg, nb, None, gl, gd), 20)
 by = nb * 21 * R + nb * 256 * 4 + nb * 128 * 40
-print(f"DET_LOSS_GRID={os.environ.get('DET_LOSS_GRID','16')}: {ms*1e3:.1f} us  {by/ms/1e6:.0f} GB/s  frac {by/ms/1e6/6537.6:.3f}")
+print(f"{ms*1e3:.1f} us  {by/ms/1e6:.0f} GB/s  frac {by/ms/1e6/6537.6:.3f}")

@@ -224,48 +224,3 @@ def test_find_top_rpn_proposals_stress(det, O, seed):
         assert torch.equal(got[i].objectness_logits.cpu(), ws), i
         assert torch.equal(got[i].proposal_boxes.tensor.cpu(), wb), i
 
-
-_ALT_PATH_SCRIPT = r"""
-import sys, torch
-sys.path.insert(0, sys.argv[1]); sys.path.insert(0, sys.argv[1] + "/object-detection-pytorch-rust_b200")
-import det_b200 as det
-g = torch.Generator().manual_seed(77)
-strides = [4, 8, 16, 32, 64]
-rpn = det.RegionProposalNetwork(strides)
-n = 3
-obj = [torch.randn(n, 3, 256 // s, 256 // s, generator=g).cuda() for s in strides]
-obj[0] = (obj[0] * 4).round() / 4  # ties at the cuts of the finest level
-dlt = [(torch.randn(n, 12, 256 // s, 256 // s, generator=g) * 0.4).cuda() for s in strides]
-sizes = torch.tensor([[256, 256], [250, 240], [256, 200]], dtype=torch.int32, device="cuda")
-logits, boxes, level_sizes = rpn.decode_heads(obj, dlt)
-out = {}
-for pre, post in ((2000, 1000), (300, 50), (12000, 2000)):
-    b, s, c, f = det.rpn_proposals_batched(boxes, logits, level_sizes, sizes, 0.7, pre, post, 0.0)
-    for i in range(n):
-        k = int(c[i])
-        out[(pre, post, i)] = (b[i, :k].cpu(), s[i, :k].cpu())
-torch.save(out, sys.argv[2])
-"""
-
-
-def test_proposal_path_variants_agree_bitwise(tmp_path):
-    """The default proposal path (one select CTA per (image, level), per-level tile sort, finish kernel) against the forms
-    it replaced and still falls back to for large pyramids (DET_RPN_OLD_SORTS=1: tile sort + merge passes, rekey / pad /
-    sort / emit; DET_RPN_SELECT_SPLIT=0: one select CTA per image): same proposals, same logits, same counts, bit for bit.
-    The switches are read once per process, so each variant runs in its own interpreter."""
-    import os, subprocess, sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    script = tmp_path / "alt_path.py"
-    script.write_text(_ALT_PATH_SCRIPT)
-    results = []
-    for extra in ({}, {"DET_RPN_OLD_SORTS": "1"}, {"DET_RPN_SELECT_SPLIT": "0"}):
-        out = tmp_path / ("out_" + "_".join(extra) + ".pt")
-        env = dict(os.environ, **extra)
-        subprocess.run([sys.executable, str(script), root, str(out)], check=True, env=env, timeout=300)
-        results.append(torch.load(out))
-    base = results[0]
-    assert len(base) == 9 and all(v[0].shape[0] > 0 for v in base.values())
-    for other in results[1:]:
-        assert other.keys() == base.keys()
-        for k in base:
-            assert torch.equal(base[k][0], other[k][0]) and torch.equal(base[k][1], other[k][1]), k

@@ -1,6 +1,7 @@
 """GPU parity for the kernel variants that only production-sized inputs select: ROIAlign channel groups and its direct
 (untabulated) path, the YOLO loss's direct kernel and multi-image shared-memory tile, the RPN loss's grid-stride loop,
-and the generic IoU matcher with several images per CTA and more than one chunk of gt boxes in pass 2.
+the generic IoU matcher with several images per CTA and more than one chunk of gt boxes in pass 2, and the RPN
+proposal path's multi-tile sorts and rekey / pad / sort / emit finish.
 
 Every test first restates the launcher's selection arithmetic (a small helper naming the source line) and asserts that
 its inputs reach the variant, so that retuning a constant makes the test fail instead of quietly covering the other
@@ -194,13 +195,13 @@ def test_roi_align_stress_random_shapes(det, seed):
 # ---------------------------------------------------------------------------------------------------------------------
 # YOLO grid loss (csrc/assign_loss.cu, yolo_loss_impl)
 # ---------------------------------------------------------------------------------------------------------------------
-YOLO_LOSS_TILE = 5888  # kYoloLossTile, assign_loss.cu:922: floats of head staged per CTA
+YOLO_LOSS_TILE = 5888  # kYoloLossTile, assign_loss.cu:921: floats of head staged per CTA
 
 
 def yolo_loss_plan(n, S, B, C, sms):
-    """The launch yolo_loss_impl chooses (assign_loss.cu:1266-1278): the direct kernel when one image's head exceeds the
+    """The launch yolo_loss_impl chooses (assign_loss.cu:1258-1270): the direct kernel when one image's head exceeds the
     tile, else the tile kernel with `imgs` images per CTA; the last CTA holds `last` images and stages them with 16-byte
-    loads only if its base and length are multiples of 4 floats (assign_loss.cu:939-944)."""
+    loads only if its base and length are multiples of 4 floats (assign_loss.cu:938-943)."""
     per_img = S * S * (B * 5 + C)
     if per_img > YOLO_LOSS_TILE:
         return {"kernel": "direct", "per_img": per_img}
@@ -282,21 +283,12 @@ def test_yolo_loss_size_variants(det, O, sms, variant):
 # ---------------------------------------------------------------------------------------------------------------------
 # RPN loss grid-stride loop (csrc/assign_loss.cu, det_rpn_loss)
 # ---------------------------------------------------------------------------------------------------------------------
-LOSS_THREADS = 256  # kLossThreads, assign_loss.cu:760
-
-
-def loss_grid_factor():
-    """CTAs per SM of the loss grid (assign_loss.cu:1046-1053): DET_LOSS_GRID when positive, else 16."""
-    v = os.environ.get("DET_LOSS_GRID")
-    try:
-        x = int(v) if v else 0
-    except ValueError:
-        x = 0
-    return x if x > 0 else 16
+LOSS_THREADS = 256  # kLossThreads, assign_loss.cu:759
+LOSS_GRID_FACTOR = 16  # kLossGridFactor, assign_loss.cu:1045: CTAs per SM of the loss grid
 
 
 def rpn_loss_iterations(total, sms, factor):
-    """Grid-stride iterations of the first warp of det_rpn_loss (assign_loss.cu:1203-1207, :794-796): a warp owns 128
+    """Grid-stride iterations of the first warp of det_rpn_loss (assign_loss.cu:1195-1199, :793-795): a warp owns 128
     labels per iteration, the grid is capped at SMs * factor CTAs of 8 warps."""
     nwarps = (total + 127) // 128
     blocks = min((nwarps + LOSS_THREADS // 32 - 1) // (LOSS_THREADS // 32), sms * factor)
@@ -368,7 +360,7 @@ def test_rpn_loss_grid_stride_loop(det, O, sms, rpn_big, loss_type, beta):
     label word while the current one is processed.  Losses, counts and both gradients against the oracle, through
     autograd (upstream 1 and 2) and through the fused forward+backward launch."""
     n, r = rpn_big["labels"].shape
-    assert rpn_loss_iterations(n * r, sms, loss_grid_factor()) >= 2
+    assert rpn_loss_iterations(n * r, sms, LOSS_GRID_FACTOR) >= 2
     want = rpn_big["oracle"][(loss_type, beta)]
     rpn = det.RegionProposalNetwork(STRIDES, SIZES, RATIOS, smooth_l1_beta=beta, box_reg_loss_type=loss_type)
     asg = _rpn_asg(det, rpn_big)
@@ -386,59 +378,47 @@ def test_rpn_loss_grid_stride_loop(det, O, sms, rpn_big, loss_type, beta):
     _check_rpn_grads(res2["grad_logits"].cpu(), res2["grad_deltas"].cpu(), want["grad_one"], loss_type)
 
 
-_LOSS_GRID_SCRIPT = r"""
-import sys, torch
-sys.path.insert(0, sys.argv[1]); sys.path.insert(0, sys.argv[1] + "/object-detection-pytorch-rust_b200")
-import det_b200 as det
-case = torch.load(sys.argv[2])
-asg = det.Assignment(case["labels"].cuda(), case["matched"].cuda(), case["table"].cuda(), case["offsets"].cuda())
-out = {"sms": det._native.fn("det_sm_count")()}
-for lt, beta in case["configs"]:
-    rpn = det.RegionProposalNetwork([4, 8, 16, 32, 64], smooth_l1_beta=beta, box_reg_loss_type=lt)
-    res = rpn.fused_losses(case["anchors"].cuda(), case["logits"].cuda(), case["deltas"].cuda(), asg, with_grads=True)
-    out[(lt, beta)] = {k: res[k].cpu() for k in ("cls_loss", "loc_loss", "num_pos_anchors", "num_neg_anchors",
-                                                 "grad_logits", "grad_deltas")}
-torch.save(out, sys.argv[3])
-"""
-
-
-def test_rpn_loss_many_iterations_per_warp(det, rpn_big, tmp_path):
-    """DET_LOSS_GRID=1 (read once per process, so in its own interpreter): one CTA per SM, so every warp walks tens of
-    label blocks.  Same losses, counts and gradients as the oracle, for smooth-L1 (beta 0 and 0.11) and GIoU."""
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+def test_rpn_loss_many_iterations_per_warp(det, sms, rpn_big):
+    """The 64-image batch tiled 16 times: 1 024 images x 50 127 anchors (the training batch of DESIGN section 4), so
+    every warp of the default grid walks tens of label blocks.  The normaliser batch_size_per_image * N grows with the
+    batch, so the losses are the 64-image ones and 16 x every copy's gradients are the 64-image gradients, for
+    smooth-L1 (beta 0 and 0.11) and GIoU through the fused forward+backward launch.  num_pos is compared exactly at
+    16 x the 64-image count; num_neg (about 50 M) lies beyond fp32's exact integers, and each CTA's atomic add of its
+    exact partial count into the fp32 accumulator (assign_loss.cu:849-852) rounds by at most 2 below 2^26."""
+    copies = 16
     n, r = rpn_big["labels"].shape
-    gts = rpn_big["gts"]
-    case = {k: rpn_big[k] for k in ("anchors", "labels", "matched", "logits", "deltas")}
-    case["table"] = torch.cat(gts, 0)
-    case["offsets"] = torch.tensor([0] + [int(x) for x in torch.tensor([len(b) for b in gts]).cumsum(0)],
-                                   dtype=torch.int32)
-    case["configs"] = RPN_LOSS_CONFIGS
-    torch.save(case, tmp_path / "case.pt")
-    script = tmp_path / "loss_grid.py"
-    script.write_text(_LOSS_GRID_SCRIPT)
-    env = dict(os.environ, DET_LOSS_GRID="1")
-    subprocess.run([sys.executable, str(script), root, str(tmp_path / "case.pt"), str(tmp_path / "out.pt")], check=True,
-                   env=env, timeout=600)
-    out = torch.load(tmp_path / "out.pt")
-    assert rpn_loss_iterations(n * r, out["sms"], 1) >= 16
+    assert rpn_loss_iterations(copies * n * r, sms, LOSS_GRID_FACTOR) >= 16
+    ctas = sms * LOSS_GRID_FACTOR
+    assert copies * n * r > ctas * (LOSS_THREADS // 32) * 128  # the grid is at its cap: the bound below counts its CTAs
+    assert copies * max(w["num_neg"] for w in rpn_big["oracle"].values()) < 2 ** 26
+    asg = _rpn_asg(det, {"gts": rpn_big["gts"] * copies, "labels": rpn_big["labels"].cuda().repeat(copies, 1),
+                         "matched": rpn_big["matched"].cuda().repeat(copies, 1)})
+    anc = rpn_big["anchors"].cuda()
+    logits = rpn_big["logits"].cuda().repeat(copies, 1)
+    deltas = rpn_big["deltas"].cuda().repeat(copies, 1, 1)
     for lt, beta in RPN_LOSS_CONFIGS:
-        got, want = out[(lt, beta)], rpn_big["oracle"][(lt, beta)]
-        _check_rpn_sums(got["cls_loss"], got["loc_loss"], got["num_pos_anchors"], got["num_neg_anchors"], want, lt)
-        _check_rpn_grads(got["grad_logits"], got["grad_deltas"], want["grad_one"], lt)
+        want = rpn_big["oracle"][(lt, beta)]
+        rpn = det.RegionProposalNetwork(STRIDES, SIZES, RATIOS, smooth_l1_beta=beta, box_reg_loss_type=lt)
+        res = rpn.fused_losses(anc, logits, deltas, asg, with_grads=True)
+        got_neg = int(res["num_neg_anchors"])
+        assert abs(got_neg - copies * want["num_neg"]) <= 2 * ctas, (got_neg, copies * want["num_neg"])
+        _check_rpn_sums(res["cls_loss"].cpu(), res["loc_loss"].cpu(), res["num_pos_anchors"], got_neg,
+                        dict(want, num_pos=copies * want["num_pos"], num_neg=got_neg), lt)
+        grad_one = tuple(w.cuda().expand(copies, *w.shape) for w in want["grad_one"])
+        _check_rpn_grads(copies * res["grad_logits"].view(copies, n, r), copies * res["grad_deltas"].view(copies, n, r, 4),
+                         grad_one, lt)
 
 
 # ---------------------------------------------------------------------------------------------------------------------
 # IoU matching (csrc/assign_loss.cu, det_match_anchors)
 # ---------------------------------------------------------------------------------------------------------------------
-MATCH_ANCHORS_PER_CTA = 256 * 4  # kMatchThreads * kMatchPerThread, assign_loss.cu:18-19
-MATCH_IMGS = 8                   # kMatchImgs, assign_loss.cu:35
-GT_CHUNK = 512                   # kGtChunk, assign_loss.cu:20: gt boxes pass 2 considers per round
+MATCH_ANCHORS_PER_CTA = 256 * 4  # kMatchThreads * kMatchPerThread, assign_loss.cu:17-18
+MATCH_IMGS = 8                   # kMatchImgs, assign_loss.cu:34
+GT_CHUNK = 512                   # kGtChunk, assign_loss.cu:19: gt boxes pass 2 considers per round
 
 
 def match_images_per_cta(n, r, sms):
-    """`imgs` of det_match_anchors (assign_loss.cu:1102-1105)."""
+    """`imgs` of det_match_anchors (assign_loss.cu:1094-1097)."""
     bx = (r + MATCH_ANCHORS_PER_CTA - 1) // MATCH_ANCHORS_PER_CTA
     return min(max((bx * n) // (sms * 16), 1), MATCH_IMGS)
 
@@ -493,3 +473,47 @@ def test_match_anchors_several_images_per_cta(det, O, sms, match_big, lq):
         assert "status -2" in str(e), str(e)                # DET_ERR_UNSUPPORTED
     else:
         assert torch.equal(ri, gi) and torch.equal(rl, gl)
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# RPN proposal selection for large pyramids (csrc/proposals.cu, det_rpn_proposals)
+# ---------------------------------------------------------------------------------------------------------------------
+RPN_TILE = 2048               # kTile, nms_large.cuh:16: keys of one shared-memory tile sort
+RPN_FINISH_SMEM = 200 * 1024  # proposals.cu:755: shared memory the one-CTA finish kernel may stage kept keys in
+
+
+def rpn_proposal_plan(level_sizes, pre, post):
+    """The sort and the finish det_rpn_proposals launches.  Sort (proposals.cu:725-730): one tile sort per (image,
+    level) while no level keeps more than kTile keys, else sort_rows (tile sort + merge passes).  Finish
+    (proposals.cu:753-755): the one-CTA finish kernel while an image's kept keys, 8 bytes for each of at most
+    min(size, pre, post) per level, fit 200 KB, else rekey / pad / sort_rows / emit."""
+    kept_bytes = 8 * sum(min(s, pre, post) for s in level_sizes)
+    return {"sort": "levels" if min(max(level_sizes), pre) <= RPN_TILE else "sort_rows",
+            "finish": "kernel" if kept_bytes <= RPN_FINISH_SMEM else "rekey", "kept_bytes": kept_bytes}
+
+
+def test_rpn_proposals_large_pyramid_sort_and_finish(det, O):
+    """pre = post = 14 000 on a 448 x 448 pyramid: the select's keys go through sort_rows and the kept ones through
+    rekey / pad / sort_rows / emit.  Quantised logits on the finest level (ties at its top-k cut), ragged image sizes,
+    three images; kept boxes, logits and counts bit-exact against the oracle's find_top_rpn_proposals."""
+    from tests.test_gpu_rpn import _heads, _oracle_decode
+    n, img, pre, post = 3, 448, 14000, 14000
+    g = gen(77)
+    obj, dlt = _heads(n, img, g, 0.4)
+    obj[0] = (obj[0] * 4).round() / 4
+    anchors, lg, dl, props = _oracle_decode(O, obj, dlt, img)
+    level_sizes = [a.shape[0] for a in anchors]
+    assert level_sizes == [37632, 9408, 2352, 588, 147]
+    plan = rpn_proposal_plan(level_sizes, pre, post)
+    assert plan == {"sort": "sort_rows", "finish": "rekey", "kept_bytes": 211960}
+    ranked = lg[0].sort(1, descending=True).values
+    assert bool((ranked[:, pre - 1] == ranked[:, pre]).all())  # every image's finest-level cut splits equal logits
+    sizes = [(448, 448), (430, 400), (448, 360)]
+    want = O.find_top_rpn_proposals([p.clone() for p in props], lg, sizes, 0.7, pre, post, 0.0, False)
+    got = det.find_top_rpn_proposals([p.cuda() for p in props], [l.cuda() for l in lg], sizes, 0.7, pre, post, 0.0,
+                                     False)
+    for i in range(n):
+        wb, ws = want[i]
+        assert len(got[i]) == wb.shape[0], (i, len(got[i]), wb.shape[0])
+        assert torch.equal(got[i].objectness_logits.cpu(), ws), i
+        assert torch.equal(got[i].proposal_boxes.tensor.cpu(), wb), i
