@@ -193,8 +193,8 @@ DET_API int det_dense_decode_level(const float* head, int n, int a, int c, int h
 
 /* All pyramid levels of a dense anchor head in ONE launch (flat 16-byte streaming kernel, csrc/dense_decode.cu).
  * Every level shares n, a, c; level l: head (n, a*(5+c), h, w) device, anchors_wh (a,2) device, first output row
- * out_offset.  Levels whose h*w is not a multiple of 4 (or an unaligned head) make the call fall back to one
- * det_dense_decode_level launch per level -- same results. */
+ * out_offset.  Levels whose h*w is not a multiple of 4 (or whose head is not 16-byte aligned) ride in the same launch
+ * with scalar loads.  limit: h*w < 2^30 per level. */
 typedef struct det_dense_level {
     const float* head;
     const float* anchors_wh;
@@ -204,8 +204,8 @@ typedef struct det_dense_level {
 DET_API int det_dense_decode(const det_dense_level_t* levels_host, int num_levels, int n, int a, int c, float scale_clamp,
                      float* boxes_out, float* score_out, int64_t* class_out, int64_t out_img_stride, void* stream);
 /* det_dense_decode on a head of element type head_dtype (DET_DTYPE_*): every level's `head` points at elements of that
- * type (the `reserved` field stays unread).  The one-launch path needs every level h*w % 4 == 0 and heads aligned to 4
- * elements; otherwise each level takes its own launch (scalar loads where needed) -- same results.  Unknown
+ * type (the `reserved` field stays unread).  Every pyramid is one launch: a level streams with vector loads when
+ * h*w % 4 == 0 and its head is aligned to 4 elements; other levels ride along with scalar loads.  Unknown
  * head_dtype: DET_ERR_BAD_ARG.  det_dense_decode is this call with DET_DTYPE_F32. */
 DET_API int det_dense_decode_typed(const det_dense_level_t* levels_host, int num_levels, int n, int a, int c,
                            float scale_clamp, float* boxes_out, float* score_out, int64_t* class_out,

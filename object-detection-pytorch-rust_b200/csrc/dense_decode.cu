@@ -10,6 +10,8 @@
 // levels ride along with the big one instead of paying their own launch and tail; 64 registers -> 1024 resident
 // threads per SM keep ~130 KB per SM in flight.  Measured (profiles/README.md): 4.9 TB/s algorithmic at N=32
 // (297 MB, ramp-limited like torch's own reductions), 6.1 TB/s = 93 % of the measured copy peak at N=256.
+// A level whose planes are not whole 4-position vectors (h*w % 4 != 0, e.g. 13x13, or a head not aligned to 4
+// elements) rides in the same launch: its threads read their 4 positions with scalar loads and skip the ones past h*w.
 // A bulk-async-copy (cp.async.bulk + mbarrier, producer warp / consumer warps) pipeline was built and measured
 // first (commit "Dense head decode: one-launch ..."): 4.2 TB/s -- the 1 KB-per-plane slabs need 85 copy
 // instructions each and only two 87 KB stages fit, so it lost to plain loads and was removed.
@@ -23,6 +25,8 @@
 // decides ties), runs the exact greedy NMS and writes the detections.  GATED select reads the objectness plane first
 // and skips the other 84 planes of a thread's 4 positions when sigmoid(obj) <= thresh for all of them -- exact, since
 // score = sigmoid(obj) * sigmoid(best) <= sigmoid(obj) in fp32 (a factor <= 1 cannot round a product upwards).
+#include <type_traits>
+
 #include "nms_core.cuh"
 #include "nms_small.cuh"
 #include "nms_list.cuh"
@@ -37,6 +41,7 @@ struct DenseLevelDev {
     const float2* anchors_wh;
     int w, hw;
     float stride;
+    int vec;  // planes are whole 4-element vectors (hw % 4 == 0, head aligned to 4 elements): one vector load per plane
     int64_t out_offset;
 };
 
@@ -65,35 +70,39 @@ struct FlatArgs {
     int32_t* overflow_flag;  // cleared here (first thread of the grid); the NMS kernel behind this one sets it
 };
 
-template <int MODE, typename T>
-__global__ void __launch_bounds__(kFlatThreads) dense_decode_flat_kernel(const __grid_constant__ FlatArgs g) {
-    using V = typename Head<T>::vec;  // 4 positions of one plane: 16 bytes (fp32) or 8 bytes (bf16 / fp16)
-    if (MODE != kModeDense) {
-        pdl_trigger();  // det_dense_detect: the NMS kernel's CTAs may move in as SM slots free up
-        if (blockIdx.x == 0 && threadIdx.x == 0 && g.overflow_flag) *g.overflow_flag = 0;
-    }
-    long long gt = (long long)blockIdx.x * kFlatThreads + threadIdx.x;
-    bool active = gt < g.thread_begin[g.num_levels];
-    if (MODE == kModeDense) {
-        if (!active) return;
-    } else if (!active) {
-        gt = 0;  // SELECT: every lane reaches the warp-collective append below
-    }
-    int l = 0;
+// Four consecutive positions of one plane as fp32; STREAM: evict-first (read once).  Through a vector pointer: one
+// load.  Through an element pointer (a level that is not vec): scalar loads of the first m positions, and the positions
+// past the plane's end read as 0.
+template <typename T, bool STREAM>
+__device__ __forceinline__ float4 ld_quad(const typename Head<T>::vec* p, int) {
+    return STREAM ? ld4_stream<T>(p) : ld4<T>(p);
+}
+template <typename T, bool STREAM>
+__device__ __forceinline__ float4 ld_quad(const T* p, int m) {
+    float r[4];
 #pragma unroll
-    for (int q = 1; q < kMaxLevels; ++q)
-        if (q < g.num_levels && gt >= g.thread_begin[q]) l = q;
+    for (int v = 0; v < 4; ++v) r[v] = v < m ? (STREAM ? ld1_stream(p + v) : ld1(p + v)) : 0.0f;
+    return make_float4(r[0], r[1], r[2], r[3]);
+}
+
+// Flat thread gt of level l (tid = threadIdx.x): 4 consecutive positions of one anchor.  VEC == L.vec.  A non-vec level
+// has ceil(hw / 4) position groups; the positions of its last group that lie past hw are never written.
+template <int MODE, typename T, bool VEC>
+__device__ __forceinline__ void decode_quad(const FlatArgs& g, int l, long long gt, bool active, unsigned tid) {
     const DenseLevelDev& L = g.lv[l];
-    const int groups = L.hw >> 2, A = g.a, C = g.c, nch = 5 + C;
+    // one step along a plane: 4 positions (16 bytes for fp32, 8 for bf16 / fp16) or, on a non-vec level, one
+    using P = typename std::conditional<VEC, typename Head<T>::vec, T>::type;
+    const int groups = VEC ? L.hw >> 2 : (L.hw + 3) >> 2, A = g.a, C = g.c, nch = 5 + C;
     const long long local = gt - g.thread_begin[l];
     const int grp = (int)(local % groups);
     const int ia = (int)(local / groups);  // image * A + anchor
     const int img = ia / A, ai = ia - img * A;
-    const int plane4 = groups;  // stride between planes, in 4-element vectors
-    const V* pl = reinterpret_cast<const V*>(static_cast<const T*>(L.head) + (int64_t)ia * nch * L.hw) + grp;
-    const V* pk = pl + (int64_t)5 * plane4;
+    const int plane = VEC ? groups : L.hw;  // stride between planes, in steps P
+    const int m = L.hw - grp * 4;           // positions of the group inside the plane: < 4 only at a non-vec plane's end
+    const P* pl = reinterpret_cast<const P*>(static_cast<const T*>(L.head) + (int64_t)ia * nch * L.hw) + (VEC ? grp : grp * 4);
+    const P* pk = pl + (int64_t)5 * plane;
     if (MODE == kModeSelectGated && active) {
-        const float4 q = ld4_stream<T>(pl + (int64_t)4 * plane4);
+        const float4 q = ld_quad<T, true>(pl + (int64_t)4 * plane, m);
         const float thr = g.score_thresh;
         // `!(x > thr)` also holds for NaN: a NaN objectness gives a NaN score, which is no candidate either
         if (!(sigmoidf_dd(q.x) > thr) && !(sigmoidf_dd(q.y) > thr) && !(sigmoidf_dd(q.z) > thr) &&
@@ -105,13 +114,15 @@ __global__ void __launch_bounds__(kFlatThreads) dense_decode_flat_kernel(const _
     int bidx[4] = {0, 0, 0, 0};
     if (active) {
         float best[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
+        // class planes in flight: 8 vector loads, or 4 x 4 scalar loads, which keeps the decode kernel at 64 registers
+        constexpr int U = VEC ? 8 : 4;
         int k = 0;
-        for (; k + 8 <= C; k += 8) {
-            float4 q[8];
+        for (; k + U <= C; k += U) {
+            float4 q[U];
 #pragma unroll
-            for (int i = 0; i < 8; ++i) q[i] = ld4_stream<T>(pk + (int64_t)(k + i) * plane4);
+            for (int i = 0; i < U; ++i) q[i] = ld_quad<T, true>(pk + (int64_t)(k + i) * plane, m);
 #pragma unroll
-            for (int i = 0; i < 8; ++i) {
+            for (int i = 0; i < U; ++i) {
                 bidx[0] = (q[i].x > best[0]) ? k + i : bidx[0]; best[0] = max_nan(best[0], q[i].x);
                 bidx[1] = (q[i].y > best[1]) ? k + i : bidx[1]; best[1] = max_nan(best[1], q[i].y);
                 bidx[2] = (q[i].z > best[2]) ? k + i : bidx[2]; best[2] = max_nan(best[2], q[i].z);
@@ -119,7 +130,7 @@ __global__ void __launch_bounds__(kFlatThreads) dense_decode_flat_kernel(const _
             }
         }
         for (; k < C; ++k) {
-            const float4 q = ld4_stream<T>(pk + (int64_t)k * plane4);
+            const float4 q = ld_quad<T, true>(pk + (int64_t)k * plane, m);
             bidx[0] = (q.x > best[0]) ? k : bidx[0]; best[0] = max_nan(best[0], q.x);
             bidx[1] = (q.y > best[1]) ? k : bidx[1]; best[1] = max_nan(best[1], q.y);
             bidx[2] = (q.z > best[2]) ? k : bidx[2]; best[2] = max_nan(best[2], q.z);
@@ -130,7 +141,7 @@ __global__ void __launch_bounds__(kFlatThreads) dense_decode_flat_kernel(const _
         if (best[0] != best[0] || best[1] != best[1] || best[2] != best[2] || best[3] != best[3]) {
             bool found[4] = {false, false, false, false};
             for (int j = 0; j < C; ++j) {
-                const float4 q4 = ld4<T>(pk + (int64_t)j * plane4);
+                const float4 q4 = ld_quad<T, false>(pk + (int64_t)j * plane, m);
                 const float q[4] = {q4.x, q4.y, q4.z, q4.w};
 #pragma unroll
                 for (int v = 0; v < 4; ++v)
@@ -143,7 +154,7 @@ __global__ void __launch_bounds__(kFlatThreads) dense_decode_flat_kernel(const _
         float t[5][4];  // box logits last: they would only occupy registers during the class loop
 #pragma unroll
         for (int j = 0; j < 5; ++j) {
-            const float4 q = ld4_stream<T>(pl + (int64_t)j * plane4);
+            const float4 q = ld_quad<T, true>(pl + (int64_t)j * plane, m);
             t[j][0] = q.x; t[j][1] = q.y; t[j][2] = q.z; t[j][3] = q.w;
         }
         const float2 awh = L.anchors_wh[ai];
@@ -164,6 +175,7 @@ __global__ void __launch_bounds__(kFlatThreads) dense_decode_flat_kernel(const _
         const int64_t obase = (int64_t)img * g.out_img_stride + L.out_offset;
 #pragma unroll
         for (int v = 0; v < 4; ++v) {
+            if (!VEC && v >= m) break;
             const int64_t o = obase + (int64_t)(grp * 4 + v) * A + ai;
             st_stream(g.boxes_out + o, box[v]);
             st_stream(g.score_out + o, score[v]);
@@ -179,7 +191,7 @@ __global__ void __launch_bounds__(kFlatThreads) dense_decode_flat_kernel(const _
             for (int v = 0; v < 4; ++v) pass |= (score[v] > g.score_thresh) ? (1u << v) : 0u;
         }
         const int my = __popc(pass);
-        const int lane = threadIdx.x & 31;
+        const int lane = tid & 31;
         const int img0 = __shfl_sync(0xffffffffu, img, 0);
         int slot = 0;
         if (__all_sync(0xffffffffu, img == img0)) {
@@ -213,80 +225,29 @@ __global__ void __launch_bounds__(kFlatThreads) dense_decode_flat_kernel(const _
     }
 }
 
-// ---- fallback for levels whose h*w is not a multiple of 4 (or an unaligned head): one thread per position, scalar loads
-template <int V, typename T = float>
-__global__ void __launch_bounds__(256)
-dense_decode_level_kernel(const T* __restrict__ head, int a, int c, int h, int w, float stride,
-                          const float2* __restrict__ anchors_wh, float scale_clamp, float4* __restrict__ boxes_out,
-                          float* __restrict__ score_out, int64_t* __restrict__ class_out, int64_t out_img_stride,
-                          int64_t out_offset) {
-    const int64_t hw = (int64_t)h * w;
-    const int64_t groups = (hw + V - 1) / V;
-    const int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const int img = blockIdx.y;
-    if (g >= groups) return;
-    const int64_t p0 = g * V;
-    const int nch = 5 + c;
-    float colf[V], rowf[V];
-#pragma unroll
-    for (int v = 0; v < V; ++v) {
-        colf[v] = (float)((p0 + v) % w);
-        rowf[v] = (float)((p0 + v) / w);
+template <int MODE, typename T>
+__global__ void __launch_bounds__(kFlatThreads) dense_decode_flat_kernel(const __grid_constant__ FlatArgs g) {
+    if (MODE != kModeDense) {
+        pdl_trigger();  // det_dense_detect: the NMS kernel's CTAs may move in as SM slots free up
+        if (blockIdx.x == 0 && threadIdx.x == 0 && g.overflow_flag) *g.overflow_flag = 0;
     }
-    const int64_t obase = (int64_t)img * out_img_stride + out_offset;
-    for (int ai = 0; ai < a; ++ai) {
-        const T* pl = head + ((int64_t)(img * a + ai) * nch) * hw + p0;
-        float t[5][V];
-#pragma unroll
-        for (int k = 0; k < 5; ++k) {
-            if (V == 4) {
-                const float4 q = ld4_stream<T>(reinterpret_cast<const typename Head<T>::vec*>(pl + k * hw));
-                t[k][0] = q.x; t[k][1] = q.y; t[k][2] = q.z; t[k][3] = q.w;
-            } else {
-                t[k][0] = ld1_stream(pl + k * hw);
-            }
-        }
-        float best[V];
-        int bidx[V];
-#pragma unroll
-        for (int v = 0; v < V; ++v) {
-            best[v] = -INFINITY;
-            bidx[v] = 0;
-        }
-        // running arg-max over the class planes; first maximum wins, a NaN wins over everything (torch.max)
-#pragma unroll 4
-        for (int k = 0; k < c; ++k) {
-            float q[V];
-            if (V == 4) {
-                const float4 q4 = ld4_stream<T>(reinterpret_cast<const typename Head<T>::vec*>(pl + (int64_t)(5 + k) * hw));
-                q[0] = q4.x; q[1] = q4.y; q[2] = q4.z; q[3] = q4.w;
-            } else {
-                q[0] = ld1_stream(pl + (int64_t)(5 + k) * hw);
-            }
-#pragma unroll
-            for (int v = 0; v < V; ++v) {
-                const bool take = (k == 0) || (q[v] > best[v]) || (q[v] != q[v] && best[v] == best[v]);
-                best[v] = take ? q[v] : best[v];
-                bidx[v] = take ? k : bidx[v];
-            }
-        }
-        const float2 awh = anchors_wh[ai];
-#pragma unroll
-        for (int v = 0; v < V; ++v) {
-            const float cx = (sigmoidf_dd(t[0][v]) + colf[v]) * stride;
-            const float cy = (sigmoidf_dd(t[1][v]) + rowf[v]) * stride;
-            float tw = t[2][v], th = t[3][v];
-            tw = (tw > scale_clamp) ? scale_clamp : tw;
-            th = (th > scale_clamp) ? scale_clamp : th;
-            const float bw = expf(tw) * awh.x, bh = expf(th) * awh.y;
-            const int64_t o = obase + (p0 + v) * a + ai;
-            boxes_out[o] = make_float4(cx - 0.5f * bw, cy - 0.5f * bh, cx + 0.5f * bw, cy + 0.5f * bh);
-            score_out[o] = sigmoidf_dd(t[4][v]) * (c > 0 ? sigmoidf_dd(best[v]) : 1.0f);
-            class_out[o] = (int64_t)bidx[v];
-        }
+    long long gt = (long long)blockIdx.x * kFlatThreads + threadIdx.x;
+    bool active = gt < g.thread_begin[g.num_levels];
+    if (MODE == kModeDense) {
+        if (!active) return;
+    } else if (!active) {
+        gt = 0;  // SELECT: every lane reaches the warp-collective append below
     }
+    int l = 0;
+#pragma unroll
+    for (int q = 1; q < kMaxLevels; ++q)
+        if (q < g.num_levels && gt >= g.thread_begin[q]) l = q;
+    // Non-vec levels are compiled into the decode only: det_dense_detect admits vec levels alone, so the lanes of a
+    // SELECT warp never split between the two forms around the warp-collective append.  threadIdx.x is read here and
+    // handed down: only in the kernel itself does the compiler bound it by kFlatThreads, and the SELECT code uses that.
+    if (MODE != kModeDense || g.lv[l].vec) decode_quad<MODE, T, true>(g, l, gt, active, threadIdx.x);
+    else decode_quad<MODE, T, false>(g, l, gt, active, threadIdx.x);
 }
-
 
 // ---- candidate compaction / final gather for the unfused detector path (any candidate count: the overflow route of
 // det_dense_detect and pyramids outside its limits).  One CTA per image walks the image's rows in order; a block-wide
@@ -407,6 +368,13 @@ __attribute__((visibility("default"))) int det_debug_read_phase_blocks_dense(lon
 // The entry points below have C linkage through their declarations in det_b200.h; the per-type implementations
 // between them are C++ templates.
 
+// a vec level streams its planes with one vector load per 4 positions: whole vectors per plane, head aligned to 4
+// elements.  det_dense_detect admits vec levels only.
+template <typename T>
+static bool level_is_flat(const void* head, int64_t hw) {
+    return hw % 4 == 0 && aligned_to(head, 4 * sizeof(T)) && hw < (1ll << 30);
+}
+
 template <typename T>
 static int launch_flat(const det_dense_level_t* levels_host, int num_levels, int n, int a, int c, float scale_clamp,
                        float* boxes_out, float* score_out, int64_t* class_out, int64_t out_img_stride, cudaStream_t st,
@@ -424,13 +392,15 @@ static int launch_flat(const det_dense_level_t* levels_host, int num_levels, int
         f.thread_begin[l] = tb;
         if (l < num_levels) {
             const det_dense_level_t& L = levels_host[l];
+            const int64_t hw = (int64_t)L.h * L.w;
+            DET_CHECK_ARG(hw < (1ll << 30), "level too large (h*w >= 2^30)");
+            DET_CHECK_ARG(out_img_stride >= L.out_offset + hw * a, "output slot out of range");
             D.head = L.head; D.anchors_wh = reinterpret_cast<const float2*>(L.anchors_wh);
-            D.w = L.w > 0 ? L.w : 1; D.hw = L.h * L.w;
+            D.w = L.w > 0 ? L.w : 1; D.hw = (int)hw; D.vec = level_is_flat<T>(L.head, hw) ? 1 : 0;
             D.stride = (float)L.stride; D.out_offset = L.out_offset;
-            DET_CHECK_ARG(out_img_stride >= L.out_offset + (int64_t)D.hw * a, "output slot out of range");
-            tb += (long long)n * a * (D.hw / 4);
+            tb += (long long)n * a * ((D.hw + 3) / 4);
         } else {
-            D.head = nullptr; D.anchors_wh = nullptr; D.w = 1; D.hw = 4;
+            D.head = nullptr; D.anchors_wh = nullptr; D.w = 1; D.hw = 4; D.vec = 1;
             D.stride = 0.f; D.out_offset = 0;
         }
     }
@@ -446,49 +416,6 @@ static int launch_flat(const det_dense_level_t* levels_host, int num_levels, int
     return DET_OK;
 }
 
-
-// the one-launch kernel reads 4 positions of a plane per vector load: whole vectors per plane, head aligned to 4 elements
-template <typename T>
-static bool level_is_flat(const void* head, int64_t hw) {
-    return hw % 4 == 0 && aligned_to(head, 4 * sizeof(T)) && hw < (1ll << 30);
-}
-
-template <typename T>
-static int dense_decode_level_t(const T* head, int n, int a, int c, int h, int w, int stride, const float* anchors_wh,
-                                float scale_clamp, float* boxes_out, float* score_out, int64_t* class_out,
-                                int64_t out_img_stride, int64_t out_offset, void* stream) {
-    DET_CHECK_ARG(n >= 0 && a >= 1 && c >= 0 && h >= 0 && w >= 0, "bad size");
-    const int64_t hw = (int64_t)h * w;
-    if (n == 0 || hw == 0) return DET_OK;
-    DET_CHECK_ARG(head && anchors_wh && boxes_out && score_out && class_out, "null pointer");
-    DET_CHECK_ARG(out_offset >= 0 && out_img_stride >= hw * a + out_offset, "output slot out of range");
-    DET_CHECK_ARG(n <= 65535, "n > 65535");
-    if (!aligned16(boxes_out)) {
-        set_error("boxes_out must be 16-byte aligned");
-        return DET_ERR_ALIGN;
-    }
-    cudaStream_t st = as_stream(stream);
-    if (level_is_flat<T>(head, hw)) {
-        det_dense_level_t L;
-        L.head = reinterpret_cast<const float*>(head); L.anchors_wh = anchors_wh; L.h = h; L.w = w; L.stride = stride; L.reserved = 0; L.out_offset = out_offset;
-        return launch_flat<T>(&L, 1, n, a, c, scale_clamp, boxes_out, score_out, class_out, out_img_stride, st);
-    }
-    dim3 grid((unsigned)((hw + 255) / 256), (unsigned)n);
-    dense_decode_level_kernel<1, T><<<grid, 256, 0, st>>>(head, a, c, h, w, (float)stride,
-                                                       reinterpret_cast<const float2*>(anchors_wh), scale_clamp,
-                                                       reinterpret_cast<float4*>(boxes_out), score_out, class_out,
-                                                       out_img_stride, out_offset);
-    DET_LAUNCH_OK("dense_decode_level_kernel");
-    return DET_OK;
-}
-
-int det_dense_decode_level(const float* head, int n, int a, int c, int h, int w, int stride, const float* anchors_wh,
-                           float scale_clamp, float* boxes_out, float* score_out, int64_t* class_out,
-                           int64_t out_img_stride, int64_t out_offset, void* stream) {
-    return dense_decode_level_t<float>(head, n, a, c, h, w, stride, anchors_wh, scale_clamp, boxes_out, score_out,
-                                       class_out, out_img_stride, out_offset, stream);
-}
-
 template <typename T>
 static int dense_decode_t(const det_dense_level_t* levels_host, int num_levels, int n, int a, int c, float scale_clamp,
                           float* boxes_out, float* score_out, int64_t* class_out, int64_t out_img_stride, void* stream) {
@@ -496,23 +423,28 @@ static int dense_decode_t(const det_dense_level_t* levels_host, int num_levels, 
     if (num_levels == 0 || n == 0) return DET_OK;
     DET_CHECK_ARG(levels_host && boxes_out && score_out && class_out, "null pointer");
     DET_CHECK_ARG(num_levels <= kMaxLevels, "too many levels");
-    bool flat_ok = aligned16(boxes_out);
     for (int l = 0; l < num_levels; ++l) {
         const det_dense_level_t& L = levels_host[l];
         DET_CHECK_ARG(L.head && L.anchors_wh && L.h >= 0 && L.w >= 0 && L.out_offset >= 0, "bad level");
-        flat_ok = flat_ok && level_is_flat<T>(L.head, (int64_t)L.h * L.w);
     }
-    if (flat_ok)  // every level streams with vector loads: one launch for the whole pyramid
-        return launch_flat<T>(levels_host, num_levels, n, a, c, scale_clamp, boxes_out, score_out, class_out, out_img_stride,
-                           as_stream(stream));
-    for (int l = 0; l < num_levels; ++l) {
-        const det_dense_level_t& L = levels_host[l];
-        const int rc = dense_decode_level_t<T>(reinterpret_cast<const T*>(L.head), n, a, c, L.h, L.w, L.stride,
-                                               L.anchors_wh, scale_clamp, boxes_out, score_out, class_out, out_img_stride,
-                                               L.out_offset, stream);
-        if (rc != DET_OK) return rc;
+    if (!aligned16(boxes_out)) {
+        set_error("boxes_out must be 16-byte aligned");
+        return DET_ERR_ALIGN;
     }
-    return DET_OK;
+    return launch_flat<T>(levels_host, num_levels, n, a, c, scale_clamp, boxes_out, score_out, class_out, out_img_stride,
+                          as_stream(stream));
+}
+
+int det_dense_decode_level(const float* head, int n, int a, int c, int h, int w, int stride, const float* anchors_wh,
+                           float scale_clamp, float* boxes_out, float* score_out, int64_t* class_out,
+                           int64_t out_img_stride, int64_t out_offset, void* stream) {
+    DET_CHECK_ARG(n >= 0 && a >= 1 && c >= 0 && h >= 0 && w >= 0, "bad size");
+    const int64_t hw = (int64_t)h * w;
+    if (n == 0 || hw == 0) return DET_OK;
+    DET_CHECK_ARG(head && anchors_wh && boxes_out && score_out && class_out, "null pointer");
+    DET_CHECK_ARG(out_offset >= 0 && out_img_stride >= hw * a + out_offset, "output slot out of range");
+    const det_dense_level_t L = {head, anchors_wh, h, w, stride, 0, out_offset};
+    return dense_decode_t<float>(&L, 1, n, a, c, scale_clamp, boxes_out, score_out, class_out, out_img_stride, stream);
 }
 
 int det_dense_decode(const det_dense_level_t* levels_host, int num_levels, int n, int a, int c, float scale_clamp,

@@ -168,14 +168,9 @@ class RegionProposalNetwork:
             for oc, dc, cell, stride, sz in zip(ocs, dcs, cells, self.anchor_generator.strides, sizes):
                 a, h, wd = oc.shape[1], oc.shape[2], oc.shape[3]
                 assert dc.shape[1] == a * 4 and a == cell.shape[0]
-                if code == 0:
-                    N.call("det_rpn_decode_level", N.ptr(oc), N.ptr(dc), n, a, h, wd, int(stride),
-                           float(self.anchor_generator.offset), N.ptr(cell), *w, self.box2box_transform.scale_clamp,
-                           N.ptr(logits), N.ptr(boxes), R, off, N.stream())
-                else:  # a 16-bit level: the typed entry point with this one level
-                    lv = N.RpnLevel(oc.data_ptr(), dc.data_ptr(), cell.data_ptr(), h, wd, int(stride), 0, off)
-                    N.call("det_rpn_decode_typed", ctypes.byref(lv), 1, n, a, float(self.anchor_generator.offset), *w,
-                           self.box2box_transform.scale_clamp, N.ptr(logits), N.ptr(boxes), R, code, N.stream())
+                lv = N.RpnLevel(oc.data_ptr(), dc.data_ptr(), cell.data_ptr(), h, wd, int(stride), 0, off)
+                N.call("det_rpn_decode_typed", ctypes.byref(lv), 1, n, a, float(self.anchor_generator.offset), *w,
+                       self.box2box_transform.scale_clamp, N.ptr(logits), N.ptr(boxes), R, code, N.stream())
                 off += sz
         return logits, boxes, sizes
 

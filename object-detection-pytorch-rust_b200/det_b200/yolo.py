@@ -2,7 +2,8 @@
 
 The reference has no such head (SURVEY.md section 8 row a15); the specification is this repository's own
 (oracle/ref_torch.py: yolo_decode, yolo_select_nms, dense_decode) -- parity is pinned by that oracle only.
-Arithmetic: det_yolo_decode_nms / det_dense_decode_level (csrc/yolo.cu) + det_nms_batched.
+Arithmetic: det_yolo_decode_nms (csrc/yolo.cu), det_dense_decode / det_dense_detect (csrc/dense_decode.cu) +
+det_nms_batched.
 """
 import ctypes
 import math
@@ -342,13 +343,9 @@ class DenseAnchorHead:
         with torch.cuda.device(dev):
             for hc, a, s, sz in zip(hcs, anchors, self.strides, sizes):
                 assert hc.shape[1] == a.shape[0] * (5 + self.C), hc.shape
-                if code == 0:
-                    N.call("det_dense_decode_level", N.ptr(hc), n, a.shape[0], self.C, hc.shape[2], hc.shape[3], s,
-                           N.ptr(a), self.scale_clamp, N.ptr(boxes), N.ptr(scores), N.ptr(classes), R, off, N.stream())
-                else:  # a 16-bit level: the typed entry point with this one level
-                    lv = N.DenseLevel(hc.data_ptr(), a.data_ptr(), hc.shape[2], hc.shape[3], s, 0, off)
-                    N.call("det_dense_decode_typed", ctypes.byref(lv), 1, n, a.shape[0], self.C, self.scale_clamp,
-                           N.ptr(boxes), N.ptr(scores), N.ptr(classes), R, code, N.stream())
+                lv = N.DenseLevel(hc.data_ptr(), a.data_ptr(), hc.shape[2], hc.shape[3], s, 0, off)
+                N.call("det_dense_decode_typed", ctypes.byref(lv), 1, n, a.shape[0], self.C, self.scale_clamp,
+                       N.ptr(boxes), N.ptr(scores), N.ptr(classes), R, code, N.stream())
                 off += sz
         return boxes, scores, classes
 
@@ -363,17 +360,16 @@ class DenseAnchorHead:
             off += hc.shape[2] * hc.shape[3] * na
         return lv
 
-    def _levels(self, heads: List[torch.Tensor], typed: bool = False):
-        """(det_dense_level_t array, contiguous heads, n, A, R) for heads that share the anchor count; the heads are fp32
-        (f32c).  typed=True: bf16 / fp16 heads are kept as they are (N.heads_c) and the DET_DTYPE_* code is appended."""
+    def _levels(self, heads: List[torch.Tensor]):
+        """(det_dense_level_t array, contiguous heads, n, A, R) for heads that share the anchor count; bf16 / fp16 heads
+        are kept as they are (N.heads_c): the DET_DTYPE_* code is N.DTYPE_CODES[hcs[0].dtype]."""
         dev = heads[0].device
         anchors = self._anchors_on(dev)
-        hcs, code = N.heads_c(heads) if typed else ([N.f32c(h) for h in heads], 0)
+        hcs, _ = N.heads_c(heads)
         na = anchors[0].shape[0]
         assert all(a.shape[0] == na for a in anchors), "levels must share the anchor count"
         lv = self._level_array(hcs, anchors, na)
-        res = (lv, hcs, heads[0].shape[0], na, sum(h.shape[2] * h.shape[3] * na for h in hcs))
-        return res + (code,) if typed else res
+        return lv, hcs, heads[0].shape[0], na, sum(h.shape[2] * h.shape[3] * na for h in hcs)
 
     def fused_ok(self, heads: List[torch.Tensor]) -> bool:
         """det_dense_detect's documented limits: equal anchor counts, every level h*w % 4 == 0."""
@@ -407,7 +403,8 @@ class DenseAnchorHead:
                    "overflow": torch.empty((1,), dtype=torch.int32, device=dev)}
         if n == 0:
             return out
-        lv, hcs, _, na, _, code = self._levels(heads, typed=True)
+        lv, hcs, _, na, _ = self._levels(heads)
+        code = N.DTYPE_CODES[hcs[0].dtype]
         wsb = N.fn("det_dense_detect_workspace_bytes")(n, int(cand_cap))
         flags = 1 if gate else 0
         if isinstance(workspace, DenseDetectWorkspace):

@@ -83,7 +83,7 @@ def test_dense_decode_flat_pyramid(det, dt):
 @gpu
 @pytest.mark.parametrize("dt", DTYPES, ids=DT_IDS)
 def test_dense_decode_levels_not_multiple_of_four(det, dt):
-    """13x13 and 7x9 levels (h*w % 4 != 0): per-level scalar kernel"""
+    """13x13 and 7x9 levels (h*w % 4 != 0): scalar loads inside the one flat launch"""
     C = 20
     dh = det.DenseAnchorHead([32, 64], WH[1:], C)
     g = gen(17)
@@ -107,7 +107,7 @@ def test_dense_decode_unequal_anchor_counts(det, dt):
 @pytest.mark.parametrize("dt", DTYPES, ids=DT_IDS)
 def test_dense_decode_unaligned_view(det, dt):
     """a head that starts one element into its buffer: the wrapper copies it to an aligned buffer, and the C entry point
-    handed the unaligned pointer itself takes the scalar kernel -- both equal to the fp32 path"""
+    handed the unaligned pointer itself reads it with scalar loads -- both equal to the fp32 path"""
     C, n, hh = 20, 2, 16
     dh = det.DenseAnchorHead([32], [WH[2]], C)
     src = torch.randn(n, 3 * (5 + C), hh, hh, generator=gen(29)).to(dt)

@@ -24,8 +24,10 @@ def O():
 
 
 def _heads(n, img, g, scale=1.0, a=3):
-    obj = [torch.randn(n, a, img // s, img // s, generator=g) for s in STRIDES]
-    dlt = [torch.randn(n, 4 * a, img // s, img // s, generator=g) * scale for s in STRIDES]
+    """a: anchors per position, one count for every level or a sequence with one count per level"""
+    per_level = [a] * len(STRIDES) if isinstance(a, int) else a
+    obj = [torch.randn(n, k, img // s, img // s, generator=g) for s, k in zip(STRIDES, per_level)]
+    dlt = [torch.randn(n, 4 * k, img // s, img // s, generator=g) * scale for s, k in zip(STRIDES, per_level)]
     return obj, dlt
 
 
@@ -55,6 +57,7 @@ _ANCHOR_SETS = {  # anchors per position: (sizes per level, ratios)
     2: (SIZES, [[0.5, 2.0]]),
     4: ([[s[0], s[0] * 1.5] for s in SIZES], [[0.5, 2.0]]),
     9: ([[s[0], s[0] * 1.26, s[0] * 1.59] for s in SIZES], RATIOS),
+    (3, 6, 3, 3, 3): ([[32], [64, 90], [128], [256], [512]], RATIOS),
 }
 
 
@@ -65,18 +68,27 @@ _ANCHOR_SETS = {  # anchors per position: (sizes per level, ratios)
     pytest.param(224, 2, (10.0, 10.0, 5.0, 5.0), id="224-a2"),
     pytest.param(448, 4, (10.0, 10.0, 5.0, 5.0), id="448-a4"),
     pytest.param(448, 9, (10.0, 10.0, 5.0, 5.0), id="448-a9"),
+    pytest.param(448, (3, 6, 3, 3, 3), (10.0, 10.0, 5.0, 5.0), id="448-a3-6-3-3-3"),
 ])
 def test_decode_heads_matches_oracle(det, O, img, a, weights):
     """a = 3 (the reference's anchors) and other anchor sets: a <= 4 decodes the pyramid in one flat launch, a = 9
-    (three sizes x three ratios) falls back to one launch per level (vec and scalar forms).  With box weights
-    (10, 10, 5, 5) some width / height deltas exceed scale_clamp."""
+    (three sizes x three ratios) falls back to one launch per level (vec and scalar forms).  Unequal anchor counts per
+    level (a = 3, 6, 3, 3, 3): decode_heads calls det_rpn_decode_typed once per level.  With box weights (10, 10, 5, 5)
+    some width / height deltas exceed scale_clamp."""
     sizes, ratios = _ANCHOR_SETS[a] if a != 3 else (SIZES, RATIOS)
-    launches = rpn_decode_launches(a, [(img // s, img // s) for s in STRIDES])
-    if a <= RPN_FLAT_MAX_A:
-        assert launches == ["flat"]
+    level_hw = [(img // s, img // s) for s in STRIDES]
+    if isinstance(a, int):
+        per_level = [a] * len(STRIDES)
+        launches = rpn_decode_launches(a, level_hw)
+        if a <= RPN_FLAT_MAX_A:
+            assert launches == ["flat"]
+        else:
+            assert {"vec", "scalar"} <= set(launches)
     else:
-        assert {"vec", "scalar"} <= set(launches)
-    g = gen(img + (0 if a == 3 else 100 * a))
+        per_level = list(a)
+        launches = [x for k, hw in zip(per_level, level_hw) for x in rpn_decode_launches(k, [hw])]
+        assert launches == ["flat", "vec", "flat", "flat", "flat"]
+    g = gen(img + (0 if a == 3 else 100 * sum(per_level) // len(per_level)))
     obj, dlt = _heads(3, img, g, 0.5 if weights[2] == 1.0 else 4.0, a)
     rpn = det.RegionProposalNetwork(STRIDES, sizes, ratios, box2box_weights=weights)
     if weights[2] != 1.0:
@@ -88,7 +100,7 @@ def test_decode_heads_matches_oracle(det, O, img, a, weights):
     logits, boxes, lsz = rpn.decode_heads([o.cuda() for o in obj], [d.cuda() for d in dlt])
     anchors, lg, dl, props = _oracle_decode(O, obj, dlt, img, weights, sizes, ratios)
     assert lsz == [x.shape[0] for x in anchors]
-    assert sum(lsz) == a * sum((img // s) ** 2 for s in STRIDES)
+    assert sum(lsz) == sum(k * (img // s) ** 2 for k, s in zip(per_level, STRIDES))
     if img == 448 and a == 3:
         assert sum(lsz) == 50127
     assert torch.equal(logits.cpu(), torch.cat(lg, 1))          # pure layout change: bit-exact

@@ -248,10 +248,13 @@ def test_yolo_host_pipeline_matches_detect(det, O, use_graph, index_dtype):
     (2, 80, [(80, 80), (40, 40), (20, 20)]),   # BASELINE configs[3] geometry (640 px)
     (5, 7, [(16, 12), (2, 2)]),                # few classes, tiny levels, odd class count
     (2, 1, [(8, 8)]),                          # single class
-    (1, 80, [(20, 20), (10, 10), (5, 5)]),     # 25 positions: per-level fallback inside det_dense_decode
+    (2, 80, [(20, 20), (10, 10), (5, 5)]),     # 25 positions: the last level reads scalar; a stray write hits image 1
+    (2, 80, [(7, 9), (13, 13), (20, 20)]),     # scalar levels first: arg-max corner cases and the partial last group
 ])
 def test_dense_decode_all_levels_one_launch(det, O, n, C, sizes):
-    """det_dense_decode (one persistent launch, csrc/dense_decode.cu) vs the oracle, level by level."""
+    """det_dense_decode (one persistent launch, csrc/dense_decode.cu) vs the oracle, level by level.  Levels whose h*w
+    is not a multiple of 4 ride in the same launch with scalar loads; the rows after each such level (the next level's,
+    or the next image's) show a write past its last position."""
     A = 3
     strides = [8, 16, 32][:len(sizes)]
     wh = [[[10, 13], [16, 30], [33, 23]], [[30, 61], [62, 45], [59, 119]], [[116, 90], [156, 198], [373, 326]]][:len(sizes)]
