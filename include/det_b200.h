@@ -459,6 +459,56 @@ DET_API int det_roi_pool_levels_backward(const det_feature_level_t* grad_levels_
                                          void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------
+ * Second-stage (Fast R-CNN box predictor) inference -- what detectron2's FastRCNNOutputLayers.inference /
+ *      fast_rcnn_inference_single_image do with the box head's outputs, for the whole batch in two launches and no
+ *      host synchronisation.  The reference never wrote the ROI predictor (SURVEY.md section 0); the specification is
+ *      tests/fast_rcnn_oracle.py fast_rcnn_inference_single_image ("parity unpinned by reference").  Per image, P its rows and
+ *      K = num_classes:
+ *        probs = softmax(logits) with the row sum taken in column order (e[0] + e[1] + ... + e[K]);
+ *        boxes = apply_deltas(deltas, proposals) with k = K, or k = 1 (class_agnostic, deltas (m,4));
+ *        a row is valid iff all its boxes and all its K+1 probabilities are finite -- invalid rows are dropped;
+ *        boxes clipped to (h, w) as Boxes.clip;  candidates (i, c), c < K, with probs[i, c] > score_thresh in
+ *        row-major order;  keep = batched_nms(box, score, c, iou_threshold)[:max_det] (`mode` as in det_nms_batched).
+ *      Deviation from detectron2: i is the proposal's row among the image's ORIGINAL rows (detectron2 counts the rows
+ *      left after the validity filter).
+ *
+ *   Inputs: class_logits (m, K+1) and box_deltas (m, K*4) or (m, 4), both of element type head_dtype (DET_DTYPE_*;
+ *   16-bit rows are widened on load, so results are bit-identical to the fp32 call on the widened values); rows read
+ *   with 16-byte loads where the row pitch and base allow, scalar loads otherwise.  proposals (m, 4) fp32, 16-byte
+ *   aligned.  row_offsets (n+1) int32: image b owns rows [row_offsets[b], row_offsets[b+1]) (row_offsets[0] = 0,
+ *   non-decreasing, row_offsets[n] = m).  image_sizes (n, 2) int32 (h, w).  weights (wx, wy, ww, wh) and scale_clamp of
+ *   Box2BoxTransform (ROI heads: 10, 10, 5, 5 and log(1000/16)).
+ *   det_roi_detect_typed outputs: det_idx (n, max_det) int64 = i*K + c, det_boxes (n, max_det, 4), det_scores (n, max_det),
+ *   det_classes (n, max_det) int64, det_count (n) int32; by descending score, ties by lower flat id; entries past the
+ *   count are undefined.  Workspace, gate bit 1, cand_cap and the overflow report are det_dense_detect's: an image with
+ *   more than cand_cap candidates gets det_count = -1 and sets *overflow_flag (may be NULL; written by the call); gate
+ *   bit 0 is ignored.  m == 0: det_count = 0 for every image, no input pointer is read.
+ *   det_roi_decode_dense_typed: the dense form for the exact route taken by overflowing images -- scores_out
+ *   (n, p_max, K) and boxes_out (n, p_max, K, 4, 16-byte aligned), row i of image b at [b, i]; the probability and clipped
+ *   box of every (row, class), NaN for every class of an invalid row and of the rows i >= the image's count.  Rows past
+ *   p_max are not decoded (p_max >= every image's count).  det_threshold_compact over the (n, p_max*K) view (classes =
+ *   flat % K) -> det_nms_batched -> det_gather_detections then gives det_roi_detect's result.  decoded != 0: the rows
+ *   are probabilities (m, K+1) and boxes (m, K*4) / (m, 4) already (detectron2's fast_rcnn_inference inputs); they are
+ *   taken as they are -- validity rule, clip and padding only -- and proposals / weights are not read.
+ *   limits: num_classes <= 4096 and m * num_classes < 2^31 (every flat id fits int32), cand_cap in [1, 4096]: otherwise
+ *   DET_ERR_UNSUPPORTED.  Unknown head_dtype, unknown mode, max_det < 1, null pointers: DET_ERR_BAD_ARG.
+ * ---------------------------------------------------------------------------------------------------------- */
+DET_API int64_t det_roi_detect_workspace_bytes(int n, int64_t cand_cap);
+DET_API int64_t det_roi_detect_counter_bytes(int n); /* size of the counter block at the head of the workspace */
+DET_API int det_roi_detect_typed(const void* class_logits, const void* box_deltas, int head_dtype, const float* proposals,
+                                 const int32_t* row_offsets, int n, int64_t m, int num_classes, int class_agnostic,
+                                 const int32_t* image_sizes, float wx, float wy, float ww, float wh, float scale_clamp,
+                                 float score_thresh, double iou_threshold, int mode, int gate, int64_t cand_cap,
+                                 int64_t max_det, int64_t* det_idx, float* det_boxes, float* det_scores,
+                                 int64_t* det_classes, int32_t* det_count, int32_t* overflow_flag, void* workspace,
+                                 int64_t workspace_bytes, void* stream);
+DET_API int det_roi_decode_dense_typed(const void* class_logits, const void* box_deltas, int head_dtype,
+                                       const float* proposals, const int32_t* row_offsets, int n, int64_t m,
+                                       int num_classes, int class_agnostic, const int32_t* image_sizes, float wx,
+                                       float wy, float ww, float wh, float scale_clamp, int decoded, int p_max,
+                                       float* scores_out, float* boxes_out, void* stream);
+
+/* ------------------------------------------------------------------------------------------------------------
  * (e) the training path's one collective over NVLink peer memory instead of NCCL: SUM of the `width`-float loss/count
  *     vector (the sums the reference logs per step, python/src/models/rpn.py:216-220, 238-241) over `world` ranks.
  *     Every rank owns a buffer of slots * world * 16 floats that is mapped into every peer (symmetric memory);

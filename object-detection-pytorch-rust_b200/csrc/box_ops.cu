@@ -102,23 +102,7 @@ __global__ void matched_iou_kernel(const float4* __restrict__ b1, const float4* 
 // ------------------------------------------------------------------------------------------------
 // box codec
 // ------------------------------------------------------------------------------------------------
-struct CodecWeights {
-    float wx, wy, ww, wh;
-};
-
-// reference apply_deltas on one (anchor, delta) pair; operation order of box_regression.py:90-114
-__device__ __forceinline__ float4 decode_delta(const float4 box, const float4 d, const CodecWeights wt,
-                                               float scale_clamp) {
-    const float w = box.z - box.x, h = box.w - box.y;
-    const float cx = box.x + 0.5f * w, cy = box.y + 0.5f * h;
-    const float dx = d.x / wt.wx, dy = d.y / wt.wy;
-    float dw = d.z / wt.ww, dh = d.w / wt.wh;
-    dw = (dw > scale_clamp) ? scale_clamp : dw;  // torch.clamp(max=): NaN stays NaN
-    dh = (dh > scale_clamp) ? scale_clamp : dh;
-    const float pcx = dx * w + cx, pcy = dy * h + cy;
-    const float pw = expf(dw) * w, ph = expf(dh) * h;
-    return make_float4(pcx - 0.5f * pw, pcy - 0.5f * ph, pcx + 0.5f * pw, pcy + 0.5f * ph);
-}
+// CodecWeights, decode_delta: common.cuh (shared with roi_detect.cu)
 
 __global__ void apply_deltas_kernel(const float4* __restrict__ deltas, const float4* __restrict__ boxes,
                                     int64_t total, int k, CodecWeights wt, float scale_clamp,

@@ -154,6 +154,25 @@ __device__ __forceinline__ float ld1(const T* p) { return Head<T>::f32(*p); }
 
 __device__ __forceinline__ float box_area(const float4 b) { return (b.z - b.x) * (b.w - b.y); }
 
+// ---- box codec (Box2BoxTransform) ----------------------------------------------------------------
+struct CodecWeights {
+    float wx, wy, ww, wh;
+};
+
+// reference apply_deltas on one (anchor, delta) pair; operation order of box_regression.py:90-114
+__device__ __forceinline__ float4 decode_delta(const float4 box, const float4 d, const CodecWeights wt,
+                                               float scale_clamp) {
+    const float w = box.z - box.x, h = box.w - box.y;
+    const float cx = box.x + 0.5f * w, cy = box.y + 0.5f * h;
+    const float dx = d.x / wt.wx, dy = d.y / wt.wy;
+    float dw = d.z / wt.ww, dh = d.w / wt.wh;
+    dw = (dw > scale_clamp) ? scale_clamp : dw;  // torch.clamp(max=): NaN stays NaN
+    dh = (dh > scale_clamp) ? scale_clamp : dh;
+    const float pcx = dx * w + cx, pcy = dy * h + cy;
+    const float pw = expf(dw) * w, ph = expf(dh) * h;
+    return make_float4(pcx - 0.5f * pw, pcy - 0.5f * ph, pcx + 0.5f * pw, pcy + 0.5f * ph);
+}
+
 // 32-bit key that sorts ASCENDING into torch's descending-score order:
 // NaN first (all NaNs tie), then +inf ... -inf, -0 == +0 tie.
 __device__ __forceinline__ uint32_t score_desc_key(float s) {

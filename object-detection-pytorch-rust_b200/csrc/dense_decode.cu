@@ -316,18 +316,6 @@ __global__ void gather_detections_kernel(const int64_t* __restrict__ keep, const
 
 using namespace det;
 
-struct SelectArgs {
-    int mode;  // kModeSelect / kModeSelectGated
-    float score_thresh;
-    int cand_cap;
-    int32_t* cand_count;
-    float4* cand_box;
-    float* cand_score;
-    int32_t* cand_cls;
-    int32_t* cand_id;
-    int32_t* overflow_flag;
-};
-
 template <int CAP, int T>
 static int launch_detect_nms_t(const SelectArgs& sel, int n, float thr_f, int mode, int64_t max_det, int64_t* det_idx,
                                float* det_boxes, float* det_scores, int64_t* det_classes, int32_t* det_count,
@@ -352,6 +340,19 @@ static int launch_detect_nms(const SelectArgs& sel, int n, float thr_f, int mode
                                              det_count, overflow_flag, st);
     return launch_detect_nms_t<CAP, 256>(sel, n, thr_f, mode, max_det, det_idx, det_boxes, det_scores, det_classes,
                                          det_count, overflow_flag, st);
+}
+
+int det::launch_list_nms(const SelectArgs& sel, int n, float thr_f, int mode, int64_t max_det, int64_t* det_idx,
+                         float* det_boxes, float* det_scores, int64_t* det_classes, int32_t* det_count,
+                         int32_t* overflow_flag, cudaStream_t st) {
+    if (sel.cand_cap <= 1024)
+        return launch_detect_nms<1024>(sel, n, thr_f, mode, max_det, det_idx, det_boxes, det_scores, det_classes,
+                                       det_count, overflow_flag, st);
+    if (sel.cand_cap <= 2048)
+        return launch_detect_nms<2048>(sel, n, thr_f, mode, max_det, det_idx, det_boxes, det_scores, det_classes,
+                                       det_count, overflow_flag, st);
+    return launch_detect_nms<4096>(sel, n, thr_f, mode, max_det, det_idx, det_boxes, det_scores, det_classes, det_count,
+                                   overflow_flag, st);
 }
 
 #ifdef DET_DEBUG_PHASES
@@ -531,15 +532,8 @@ static int dense_detect_t(const det_dense_level_t* levels_host, int num_levels, 
     }
     int rc = launch_flat<T>(levels_host, num_levels, n, a, c, scale_clamp, nullptr, nullptr, nullptr, rows, st, &sel);
     if (rc != DET_OK) return rc;
-    const float thr_f = float_threshold_below(iou_threshold);
-    if (cand_cap <= 1024)
-        return launch_detect_nms<1024>(sel, n, thr_f, mode, max_det, det_idx, det_boxes, det_scores, det_classes,
-                                       det_count, overflow_flag, st);
-    if (cand_cap <= 2048)
-        return launch_detect_nms<2048>(sel, n, thr_f, mode, max_det, det_idx, det_boxes, det_scores, det_classes,
-                                       det_count, overflow_flag, st);
-    return launch_detect_nms<4096>(sel, n, thr_f, mode, max_det, det_idx, det_boxes, det_scores, det_classes, det_count,
-                                   overflow_flag, st);
+    return launch_list_nms(sel, n, float_threshold_below(iou_threshold), mode, max_det, det_idx, det_boxes, det_scores,
+                           det_classes, det_count, overflow_flag, st);
 }
 
 int det_dense_detect(const det_dense_level_t* levels_host, int num_levels, int n, int a, int c, float scale_clamp,

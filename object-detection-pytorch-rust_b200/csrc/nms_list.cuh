@@ -721,4 +721,25 @@ dense_detect_nms_kernel(int32_t* cand_count, const float4* __restrict__ cand_box
     DET_MARK(14);
 }
 
+// The per-image candidate lists of a det_dense_detect / det_roi_detect workspace, and what the select kernel that fills
+// them is told (mode and score_thresh: det_dense_detect's select kernel only).
+struct SelectArgs {
+    int mode;  // kModeSelect / kModeSelectGated
+    float score_thresh;
+    int cand_cap;
+    int32_t* cand_count;  // one counter every kCountStride words
+    float4* cand_box;
+    float* cand_score;
+    int32_t* cand_cls;
+    int32_t* cand_id;
+    int32_t* overflow_flag;
+};
+
+// dense_detect_nms_kernel over the n lists of `sel` (cand_cap <= 4096), launched with programmatic dependent launch
+// behind the select kernel that filled them: the second launch of det_dense_detect and det_roi_detect.  The tie order
+// is ascending cand_id.  Defined in dense_decode.cu.
+int launch_list_nms(const SelectArgs& sel, int n, float thr_f, int mode, int64_t max_det, int64_t* det_idx,
+                    float* det_boxes, float* det_scores, int64_t* det_classes, int32_t* det_count, int32_t* overflow_flag,
+                    cudaStream_t st);
+
 }  // namespace det

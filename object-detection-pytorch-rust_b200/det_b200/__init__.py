@@ -16,6 +16,7 @@ from .proposals import find_top_rpn_proposals, rpn_proposals_batched, add_ground
 from .rpn import RegionProposalNetwork, Assignment, _dense_box_regression_loss
 from .roi import ROIHeads, subsample_labels
 from .roi_pool import ROIAlign, ROIPooler, assign_boxes_to_levels, convert_boxes_to_pooler_format
+from .fast_rcnn import FastRCNNOutputs, fast_rcnn_inference
 from . import dist
 
 __all__ = [
@@ -24,5 +25,5 @@ __all__ = [
     "YoloGridHead", "DenseAnchorHead", "YoloGridTrainer", "YoloHostPipeline", "DenseDetectWorkspace", "Matcher", "subsample_labels_", "find_top_rpn_proposals",
     "rpn_proposals_batched", "add_ground_truth_to_proposals", "RegionProposalNetwork", "Assignment",
     "_dense_box_regression_loss", "ROIHeads", "subsample_labels", "ROIAlign", "ROIPooler", "assign_boxes_to_levels",
-    "convert_boxes_to_pooler_format", "dist",
+    "convert_boxes_to_pooler_format", "FastRCNNOutputs", "fast_rcnn_inference", "dist",
 ]

@@ -70,6 +70,12 @@ PROTOTYPES = {
                                                   c_p]),
     "det_roi_pool_levels": (c_i, [c_p, c_i, c_i, c_i, c_p, c_p, c_p, c_l, c_i, c_i, c_p, c_p, c_i, c_p]),
     "det_roi_pool_levels_backward": (c_i, [c_p, c_i, c_i, c_i, c_p, c_p, c_l, c_i, c_i, c_p, c_p, c_i, c_p]),
+    "det_roi_detect_workspace_bytes": (c_l, [c_i, c_l]),
+    "det_roi_detect_counter_bytes": (c_l, [c_i]),
+    "det_roi_detect_typed": (c_i, [c_p, c_p, c_i, c_p, c_p, c_i, c_l, c_i, c_i, c_p, c_f, c_f, c_f, c_f, c_f, c_f, c_d,
+                                   c_i, c_i, c_l, c_l, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_l, c_p]),
+    "det_roi_decode_dense_typed": (c_i, [c_p, c_p, c_i, c_p, c_p, c_i, c_l, c_i, c_i, c_p, c_f, c_f, c_f, c_f, c_f, c_i,
+                                         c_i, c_p, c_p, c_p]),
     "det_match_workspace_bytes": (c_l, [c_i, c_l, c_l]),
     "det_match_anchors": (c_i, [c_p, c_p, c_i, c_l, c_p, c_l, c_p, c_p, c_i, c_i, c_p, c_p, c_p, c_p, c_l, c_p]),
     "det_match_grid_workspace_bytes": (c_l, [c_i, c_l, c_p, c_i]),
