@@ -509,6 +509,38 @@ DET_API int det_roi_decode_dense_typed(const void* class_logits, const void* box
                                        float* scores_out, float* boxes_out, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------
+ * Second-stage (Fast R-CNN box predictor) training losses, forward and backward in one launch -- what detectron2's
+ *      FastRCNNOutputLayers.losses (softmax cross-entropy + box_reg_loss) and _log_classification_stats compute, and
+ *      autograd's backward of both.  Own specification ("parity unpinned by reference"): tests/fast_rcnn_loss_oracle.py.
+ *      Over the m rows the box head saw (packed over the batch), K = num_classes, fg = 0 <= gt < K:
+ *        loss_cls = scale_cls * sum_i (logsumexp(x_i) - x_i[gt_i])
+ *        loss_box_reg = scale_loc * sum_{fg i} L(d_i, proposal_i, gt_box_i), d_i = the 4 deltas of class gt_i (the row's
+ *        only 4 when class_agnostic); L = smooth-L1(beta) on get_deltas(proposal, gt_box) (beta < 1e-5: L1), loss_type 0,
+ *        or GIoU on apply_deltas(d, proposal) with scale_clamp, loss_type 1; weights (wx, wy, ww, wh) as Box2BoxTransform.
+ *      With scale_x = loss_weight_x / m these are detectron2's losses (F.cross_entropy mean, box loss / m).
+ *
+ *   Inputs: class_logits (m, K+1) with background last and box_deltas (m, K*4) or (m, 4), both of element type
+ *   head_dtype (DET_DTYPE_*; 16-bit rows are widened on load, so sums are the fp32 call's on the widened values).
+ *   proposals, gt_boxes (m, 4) fp32, 16-byte aligned (a row without gt carries any box: it is read only for fg rows).
+ *   gt_classes (m) int64.  A label outside [0, K] contributes to neither sum, gets zero gradient rows and is counted.
+ *   accumulators: 16 floats of device scratch, zero before the first call; the last CTA re-arms them (one per stream).
+ *   sums_out (8) fp32, written by that last CTA: [loss_cls, loss_box_reg, num_fg, num_accurate, fg_num_accurate,
+ *   num_false_negative, num_bad_labels, 0] -- counts exact; pred = argmax of the row (first maximum, NaN the largest,
+ *   first NaN wins).  grad_logits / grad_deltas: shaped and typed like the inputs, both or neither (forward only);
+ *   written in full: (softmax - onehot(gt)) * s_cls and, for fg rows, d L / d d_i * s_loc in the 4 columns of class gt,
+ *   0 everywhere else; s_x = scale_x * upstream[x] with upstream device float[2] or NULL (= 1), so a backward launch
+ *   needs no host synchronisation.  16-bit gradients are the fp32 values rounded once (torch's .to(dtype)).
+ *   m == 0: sums_out = 0 and no input pointer is read.  Limits: num_classes <= 4096, m < 2^24: DET_ERR_UNSUPPORTED.
+ *   Null pointers, unknown head_dtype or loss_type: DET_ERR_BAD_ARG, before any CUDA call.
+ * ---------------------------------------------------------------------------------------------------------- */
+DET_API int det_fast_rcnn_loss_typed(const void* class_logits, const void* box_deltas, int head_dtype,
+                                     const float* proposals, const int64_t* gt_classes, const float* gt_boxes,
+                                     int64_t m, int num_classes, int class_agnostic, float wx, float wy, float ww,
+                                     float wh, float scale_clamp, int loss_type, float smooth_l1_beta, float scale_cls,
+                                     float scale_loc, const float* upstream, float* accumulators, float* sums_out,
+                                     void* grad_logits, void* grad_deltas, void* stream);
+
+/* ------------------------------------------------------------------------------------------------------------
  * (e) the training path's one collective over NVLink peer memory instead of NCCL: SUM of the `width`-float loss/count
  *     vector (the sums the reference logs per step, python/src/models/rpn.py:216-220, 238-241) over `world` ranks.
  *     Every rank owns a buffer of slots * world * 16 floats that is mapped into every peer (symmetric memory);

@@ -119,6 +119,7 @@ template <> struct Head<float> {
     using vec = float4;
     static __device__ __forceinline__ float4 f32(const float4 v) { return v; }
     static __device__ __forceinline__ float f32(const float x) { return x; }
+    static __device__ __forceinline__ float4 pack(const float4 v) { return v; }
 };
 template <> struct Head<__nv_bfloat16> {
     using vec = uint2;
@@ -127,6 +128,11 @@ template <> struct Head<__nv_bfloat16> {
     static __device__ __forceinline__ float4 f32(const uint2 v) {
         return make_float4(f32((unsigned short)(v.x & 0xffffu)), f32((unsigned short)(v.x >> 16)),
                            f32((unsigned short)(v.y & 0xffffu)), f32((unsigned short)(v.y >> 16)));
+    }
+    // 4 fp32 values rounded to nearest even, the lower-address element in the low half of each word
+    static __device__ __forceinline__ uint2 pack(const float4 v) {
+        auto b = [](float x) { return (unsigned)__bfloat16_as_ushort(__float2bfloat16_rn(x)); };
+        return make_uint2(b(v.x) | (b(v.y) << 16), b(v.z) | (b(v.w) << 16));
     }
 };
 template <> struct Head<__half> {
@@ -137,12 +143,19 @@ template <> struct Head<__half> {
         return make_float4(f32((unsigned short)(v.x & 0xffffu)), f32((unsigned short)(v.x >> 16)),
                            f32((unsigned short)(v.y & 0xffffu)), f32((unsigned short)(v.y >> 16)));
     }
+    static __device__ __forceinline__ uint2 pack(const float4 v) {
+        auto h = [](float x) { return (unsigned)__half_as_ushort(__float2half_rn(x)); };
+        return make_uint2(h(v.x) | (h(v.y) << 16), h(v.z) | (h(v.w) << 16));
+    }
 };
 // 4 consecutive head elements as fp32: streaming (read-once) and plain (re-read) forms
 template <typename T>
 __device__ __forceinline__ float4 ld4_stream(const typename Head<T>::vec* p) { return Head<T>::f32(__ldcs(p)); }
 template <typename T>
 __device__ __forceinline__ float4 ld4(const typename Head<T>::vec* p) { return Head<T>::f32(*p); }
+// 4 fp32 results stored as 4 consecutive head elements (streaming), each rounded once as st_stream rounds one
+template <typename T>
+__device__ __forceinline__ void st4_stream(typename Head<T>::vec* p, const float4 v) { __stcs(p, Head<T>::pack(v)); }
 // one head element as fp32
 __device__ __forceinline__ float ld1_stream(const float* p) { return __ldcs(p); }
 template <typename T>

@@ -76,6 +76,8 @@ PROTOTYPES = {
                                    c_i, c_i, c_l, c_l, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_l, c_p]),
     "det_roi_decode_dense_typed": (c_i, [c_p, c_p, c_i, c_p, c_p, c_i, c_l, c_i, c_i, c_p, c_f, c_f, c_f, c_f, c_f, c_i,
                                          c_i, c_p, c_p, c_p]),
+    "det_fast_rcnn_loss_typed": (c_i, [c_p, c_p, c_i, c_p, c_p, c_p, c_l, c_i, c_i, c_f, c_f, c_f, c_f, c_f, c_i, c_f,
+                                       c_f, c_f, c_p, c_p, c_p, c_p, c_p, c_p]),
     "det_match_workspace_bytes": (c_l, [c_i, c_l, c_l]),
     "det_match_anchors": (c_i, [c_p, c_p, c_i, c_l, c_p, c_l, c_p, c_p, c_i, c_i, c_p, c_p, c_p, c_p, c_l, c_p]),
     "det_match_grid_workspace_bytes": (c_l, [c_i, c_l, c_p, c_i]),

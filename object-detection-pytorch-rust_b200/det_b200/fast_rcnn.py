@@ -5,8 +5,12 @@ class-specific decode, clip, score threshold, per-class NMS and top-k, for the w
 
 Specification: tests/fast_rcnn_oracle.py fast_rcnn_inference_single_image (detectron2's fast_rcnn_inference_single_image).
 One deviation: the kept proposal index of a detection counts the image's ORIGINAL rows; detectron2 counts the rows
-left after dropping those with a non-finite box or score, which differs only when such a row exists."""
-from typing import List, Optional, Sequence, Tuple
+left after dropping those with a non-finite box or score, which differs only when such a row exists.
+
+Training: ``FastRCNNOutputs.losses`` is detectron2's ``FastRCNNOutputLayers.losses`` (softmax cross-entropy and
+smooth-L1 / GIoU box regression on the gt class's deltas, plus ``_log_classification_stats``), forward and backward in
+one kernel (det_fast_rcnn_loss_typed, csrc/fast_rcnn_loss.cu); specification tests/fast_rcnn_loss_oracle.py."""
+from typing import Dict, List, Optional, Sequence, Tuple, Union
 
 import torch
 
@@ -85,16 +89,43 @@ def _instances(out, image_shapes, K):
     return results, kept
 
 
+class _FastRCNNLoss(torch.autograd.Function):
+    """det_fast_rcnn_loss_typed behind autograd.  Forward: one launch that reduces the sums (no gradient stores).
+    Backward: the same kernel with the upstream gradients read on the device, writing grad_logits / grad_deltas in the
+    inputs' dtype.  Everything the backward launch reads goes through save_for_backward, so an in-place change of the
+    labels or boxes between forward and backward trips autograd's version check."""
+
+    @staticmethod
+    def forward(ctx, owner, class_logits, deltas, proposal_boxes, gt_classes, gt_boxes):
+        (lg, dl), code = N.heads_c([class_logits, deltas])
+        sums = owner._run_loss(lg, dl, code, proposal_boxes, gt_classes, gt_boxes, None, None, None)
+        ctx.owner, ctx.code = owner, code
+        ctx.save_for_backward(lg, dl, proposal_boxes, gt_classes, gt_boxes)
+        return sums
+
+    @staticmethod
+    def backward(ctx, grad_sums):
+        lg, dl, props, gtc, gtb = ctx.saved_tensors
+        up = grad_sums[:2].contiguous().float()
+        gl, gd = torch.empty_like(lg), torch.empty_like(dl)
+        ctx.owner._run_loss(lg, dl, ctx.code, props, gtc, gtb, up, gl, gd)
+        return None, gl, gd, None, None, None
+
+
 class FastRCNNOutputs:
-    """The inference half of detectron2's FastRCNNOutputLayers on the box head's outputs.
+    """detectron2's FastRCNNOutputLayers on the box head's outputs: inference, and the training losses.
 
     num_classes K foreground classes (the logits carry K+1 columns, background last); box2box_transform defaults to the
     ROI heads' weights (10, 10, 5, 5); topk_per_image < 0 keeps every detection.  cand_cap (<= 4096) bounds the
-    per-image candidate list of the fused path; mode is det_nms_batched's NMS branch rule."""
+    per-image candidate list of the fused path; mode is det_nms_batched's NMS branch rule.  box_reg_loss_type
+    ("smooth_l1" or "giou"), smooth_l1_beta and loss_weight (a float for both losses, or a dict keyed "loss_cls" /
+    "loss_box_reg", 1.0 for a missing key) configure the losses as in detectron2."""
 
     def __init__(self, num_classes: int, box2box_transform: Optional[Box2BoxTransform] = None,
                  score_thresh: float = 0.05, nms_thresh: float = 0.5, topk_per_image: int = 100,
-                 class_agnostic: bool = False, cand_cap: int = 4096, mode: int = MODE_AUTO):
+                 class_agnostic: bool = False, cand_cap: int = 4096, mode: int = MODE_AUTO, *,
+                 box_reg_loss_type: str = "smooth_l1", smooth_l1_beta: float = 0.0,
+                 loss_weight: Union[float, Dict[str, float]] = 1.0):
         self.num_classes = int(num_classes)
         self.box2box_transform = box2box_transform if box2box_transform is not None else Box2BoxTransform(ROI_HEAD_WEIGHTS)
         self.score_thresh, self.nms_thresh = float(score_thresh), float(nms_thresh)
@@ -104,8 +135,14 @@ class FastRCNNOutputs:
         self.mode = int(mode)
         if not 1 <= self.cand_cap <= 4096:
             raise ValueError("cand_cap must lie in [1, 4096]")
+        self.box_reg_loss_type = box_reg_loss_type
+        self.smooth_l1_beta = float(smooth_l1_beta)
+        if not isinstance(loss_weight, dict):
+            loss_weight = {"loss_cls": loss_weight, "loss_box_reg": loss_weight}
+        self.loss_weight = loss_weight
+        self.last_sums = None
 
-    def _prepare(self, class_logits, deltas, proposal_boxes):
+    def _check_rows(self, class_logits, deltas, proposal_boxes):
         K = self.num_classes
         M = class_logits.shape[0]
         if class_logits.shape != (M, K + 1):
@@ -114,6 +151,9 @@ class FastRCNNOutputs:
         if deltas.shape != want or proposal_boxes.shape != (M, 4):
             raise ValueError(f"deltas must be {want} and proposals (M, 4), got {tuple(deltas.shape)}, "
                              f"{tuple(proposal_boxes.shape)}")
+
+    def _prepare(self, class_logits, deltas, proposal_boxes):
+        self._check_rows(class_logits, deltas, proposal_boxes)
         (lg, dl), code = N.heads_c([class_logits, deltas])
         return lg, dl, code, N.f32c(proposal_boxes)
 
@@ -181,6 +221,80 @@ class FastRCNNOutputs:
         out = self.inference_batched(class_logits, deltas, pb, _packed_offsets([len(b) for b in boxes], dev),
                                      _sizes_tensor(shapes, dev), check=True)
         return _instances(out, shapes, self.num_classes)
+
+    # ------------------------------------------------------------------ training losses
+    def _loss_scales(self, m):
+        """(loss_type, w_cls / max(m, 1), w_loc / max(m, 1)): detectron2 averages both losses over all m rows."""
+        if self.box_reg_loss_type not in ("smooth_l1", "giou"):
+            raise ValueError(f"Invalid bbox reg loss type '{self.box_reg_loss_type}'")
+        norm = float(max(m, 1))
+        return (0 if self.box_reg_loss_type == "smooth_l1" else 1), \
+            float(self.loss_weight.get("loss_cls", 1.0)) / norm, float(self.loss_weight.get("loss_box_reg", 1.0)) / norm
+
+    def _run_loss(self, lg, dl, code, props, gt_classes, gt_boxes, upstream, grad_logits, grad_deltas):
+        """One det_fast_rcnn_loss_typed launch: returns sums (8) = [loss_cls, loss_box_reg, num_fg, num_accurate,
+        fg_num_accurate, num_false_negative, num_bad_labels, 0], the losses already weighted and normalised."""
+        m = lg.shape[0]
+        loss_type, s_cls, s_loc = self._loss_scales(m)
+        w = self.box2box_transform
+        dev = lg.device
+        with torch.cuda.device(dev):
+            sums = torch.empty((8,), dtype=torch.float32, device=dev)
+            N.call("det_fast_rcnn_loss_typed", N.ptr(lg), N.ptr(dl), code, N.ptr(props), N.ptr(gt_classes),
+                   N.ptr(gt_boxes), m, self.num_classes, int(self.class_agnostic), *w.weights, w.scale_clamp,
+                   loss_type, self.smooth_l1_beta, s_cls, s_loc, N.ptr(upstream), N.ptr(N.accumulators(dev)),
+                   N.ptr(sums), N.ptr(grad_logits), N.ptr(grad_deltas), N.stream())
+        return sums
+
+    def losses_batched(self, class_logits: torch.Tensor, deltas: torch.Tensor, proposal_boxes: torch.Tensor,
+                       gt_classes: torch.Tensor, gt_boxes: torch.Tensor, with_grads: bool = False) -> dict:
+        """detectron2's FastRCNNOutputLayers.losses on the M rows the box head saw, packed over the batch:
+        class_logits (M, K+1), deltas (M, K*4) or (M, 4) (fp32, or bf16 / fp16 read as they are), proposal_boxes and
+        gt_boxes (M, 4) (a row without gt carries its proposal box), gt_classes (M,) int64 in [0, K], K = background.
+
+        Returns {"loss_cls", "loss_box_reg", "sums"}: device scalars autograd-connected to class_logits and deltas
+        (backward is one more launch, gradients in the inputs' dtype), and the 8-float sums vector of
+        det_fast_rcnn_loss_typed with detectron2's classification statistics in [2:6].  with_grads=True: one fused
+        forward + backward launch that adds grad_logits / grad_deltas (d(loss_cls + loss_box_reg)/d(input), detached).
+        No host synchronisation either way, so the call can be captured in a CUDA graph."""
+        N.require_cuda(class_logits, deltas, proposal_boxes, gt_classes, gt_boxes)
+        self._check_rows(class_logits, deltas, proposal_boxes)
+        m = class_logits.shape[0]
+        if gt_classes.shape != (m,) or gt_boxes.shape != (m, 4):
+            raise ValueError(f"gt_classes must be ({m},) and gt_boxes ({m}, 4), got {tuple(gt_classes.shape)}, "
+                             f"{tuple(gt_boxes.shape)}")
+        self._loss_scales(m)  # an unknown loss type raises before anything is launched
+        props, gtb = N.f32c(proposal_boxes), N.f32c(gt_boxes)
+        gtc = gt_classes.detach().to(torch.int64).contiguous()
+        if with_grads:
+            (lg, dl), code = N.heads_c([class_logits, deltas])
+            gl, gd = torch.empty_like(lg), torch.empty_like(dl)
+            sums = self._run_loss(lg, dl, code, props, gtc, gtb, None, gl, gd)
+        else:
+            sums = _FastRCNNLoss.apply(self, class_logits, deltas, props, gtc, gtb)
+        out = {"loss_cls": sums[0], "loss_box_reg": sums[1], "sums": sums}
+        if with_grads:
+            out["grad_logits"], out["grad_deltas"] = gl, gd
+        return out
+
+    def losses(self, predictions: Tuple[torch.Tensor, torch.Tensor], proposals: List[Instances]) -> Dict[str, torch.Tensor]:
+        """detectron2's FastRCNNOutputLayers.losses: predictions = (class_logits, proposal_deltas) over the sampled
+        proposals of the images, proposals = per-image Instances with proposal_boxes, gt_classes and, where the image
+        has gt, gt_boxes.  Returns {"loss_cls", "loss_box_reg"}; the device sums vector (classification statistics
+        included) stays in self.last_sums for logging, read back only when the caller wants it."""
+        class_logits, deltas = predictions
+        dev = class_logits.device
+        box = lambda b: b.tensor if isinstance(b, Boxes) else b
+        if len(proposals):
+            pb = torch.cat([box(p.proposal_boxes) for p in proposals], 0)
+            gtc = torch.cat([p.gt_classes for p in proposals], 0)
+            gtb = torch.cat([box(p.gt_boxes if p.has("gt_boxes") else p.proposal_boxes) for p in proposals], 0)
+        else:
+            pb = gtb = torch.empty((0, 4), dtype=torch.float32, device=dev)
+            gtc = torch.empty((0,), dtype=torch.int64, device=dev)
+        res = self.losses_batched(class_logits, deltas, pb, gtc, gtb)
+        self.last_sums = res["sums"].detach()
+        return {"loss_cls": res["loss_cls"], "loss_box_reg": res["loss_box_reg"]}
 
 
 def fast_rcnn_inference(boxes: List[torch.Tensor], scores: List[torch.Tensor], image_shapes: List[Tuple[int, int]],
