@@ -541,6 +541,46 @@ DET_API int det_fast_rcnn_loss_typed(const void* class_logits, const void* box_d
                                      void* grad_logits, void* grad_deltas, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------
+ * Batched ROI-head proposal sampling -- replaces label_and_sample_proposals + _sample_proposals,
+ *      python/src/models/roi.py:68-193, add_ground_truth_to_proposals, models/utils.py:111-155, and
+ *      subsample_labels, utils.py:34-76, for the whole batch in two launches, no host synchronisation, no allocation
+ *      and no memset (CUDA-graph capturable).
+ *   Inputs: proposals (n, p_stride, 4) fp32, image b's P_b = proposal_counts[b] (device int32) rows first -- rows past
+ *   P_b are never read (rpn_proposals_batched's padded output).  gt_boxes (sum_g, 4) fp32 with gt_offsets (n+1) int32
+ *   (Matcher.pack_gt), gt_classes (sum_g) int64, num_classes K.  The Matcher rule as det_match_anchors'.
+ *   seed: device uint64 read by the kernel, so a replayed graph that advances it draws new samples.
+ *   Per image, candidates j = 0 .. P_b-1 are the proposals, then (append_gt) P_b .. P_b+G_b-1 the gt boxes:
+ *     label: pair_iou(gt, candidate) -> column max (first maximum) -> threshold buckets -> low-quality promotion
+ *       (IoU == a gt's row maximum; a row maximum of 0 promotes every candidate) -> class gt_classes[matched], K for
+ *       matcher label 0, -1 for label -1; every candidate of an image without gt is background (K).
+ *     counts: fg = class neither -1 nor K; want_fg = min(#fg, int(S*f)) with S*f in double, want_bg = min(#bg,
+ *       S - want_fg).  S = batch_size_per_image.
+ *     selection: candidate j's key is sample_key(image_seed(*seed, b), j) (csrc/assign.cuh), a bijection of j; each class
+ *       keeps its want smallest keys (a uniformly random subset; the stream differs from torch.randperm's).
+ *   Outputs, padded (n, S): foreground rows first, then background, each in ascending j.  out_boxes (n,S,4) = the
+ *   candidate's box; out_gt_classes (n,S) int64; out_gt_boxes (n,S,4) = gt[matched] for every row of an image with gt,
+ *   the row's own box for an image without; out_matched (n,S) int32 = index into the image's gt (-1 without gt);
+ *   out_src (n,S) int32 = j.  out_count (n) int32 = want_fg + want_bg, out_num_fg (n) int32 = want_fg.  Rows past the
+ *   count: src = -1, gt_classes = -1, matched = -1, zero boxes.  *underfull_flag (device int32, written by the call) = 1
+ *   iff some image has count < S.
+ *   workspace: det_roi_sample_workspace_bytes(n, p_stride, sum_g) bytes, 16-byte aligned, ALL ZERO BEFORE THE FIRST
+ *   CALL; every call leaves it zero again (so a larger one fits every smaller call).  One workspace per stream.
+ *   Limits: n <= 65535, p_stride < 2^24, sum_g < 2^24, S < 2^24, n * p_stride + sum_g < 2^31: DET_ERR_UNSUPPORTED.
+ *   Null pointers (proposals may be NULL when p_stride == 0, gt_boxes / gt_classes when sum_g == 0), S < 1, f outside
+ *   [0, 1], num_classes < 1, a bad rule: DET_ERR_BAD_ARG, before any CUDA call.  n == 0: DET_OK, nothing is read.
+ * ---------------------------------------------------------------------------------------------------------- */
+DET_API int64_t det_roi_sample_workspace_bytes(int n, int64_t p_stride, int64_t sum_g);
+DET_API int det_roi_sample_proposals(const float* proposals, const int32_t* proposal_counts, int n, int64_t p_stride,
+                                     const float* gt_boxes, const int32_t* gt_offsets, const int64_t* gt_classes,
+                                     int64_t sum_g, int num_classes, const float* thresholds_host,
+                                     const int32_t* labels_host, int num_thresholds, int allow_low_quality,
+                                     int batch_size_per_image, double positive_fraction, int append_gt,
+                                     const uint64_t* seed, float* out_boxes, int64_t* out_gt_classes,
+                                     float* out_gt_boxes, int32_t* out_matched, int32_t* out_src, int32_t* out_count,
+                                     int32_t* out_num_fg, int32_t* underfull_flag, void* workspace,
+                                     int64_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------------------------
  * (e) the training path's one collective over NVLink peer memory instead of NCCL: SUM of the `width`-float loss/count
  *     vector (the sums the reference logs per step, python/src/models/rpn.py:216-220, 238-241) over `world` ranks.
  *     Every rank owns a buffer of slots * world * 16 floats that is mapped into every peer (symmetric memory);

@@ -39,6 +39,10 @@ __device__ __forceinline__ uint32_t mix32(uint32_t h) {
     return h;
 }
 __device__ __forceinline__ uint32_t sample_key(uint32_t img_seed, uint32_t j) { return mix32(j * 0x9E3779B1u + img_seed); }
+// per-image seed of the 64-bit call seed: the keys of image `img` are sample_key(image_seed(seed, img), j)
+__device__ __forceinline__ uint32_t image_seed(uint64_t seed, int img) {
+    return mix32((uint32_t)seed ^ mix32((uint32_t)(seed >> 32) + 0x632BE5ABu * (uint32_t)(img + 1)));
+}
 
 // b-bit bijection (odd multiplies and right xor-shifts are invertible mod 2^b): k -> a pseudo-random permutation of
 // [0, 2^b).  Walking k = 0, 1, 2, ... and keeping the first `want` indices that fall inside the row and carry the class

@@ -324,10 +324,6 @@ struct SampleSmem {
     int cidx[2][kCandCap];  // anchor index of the candidate | its original label in the top byte
 };
 
-__device__ __forceinline__ uint32_t image_seed(uint64_t seed, int img) {
-    return mix32((uint32_t)seed ^ mix32((uint32_t)(seed >> 32) + 0x632BE5ABu * (uint32_t)(img + 1)));
-}
-
 // class c of one image sampled by walking a pseudo-random permutation of the row (block-wide, all threads call it):
 // the first `want` hits, in walk order, land in sm.cidx[c][0..want) with key 0
 __device__ __forceinline__ void walk_class(SampleSmem& sm, const RowView& rv, int c, int want, uint32_t img_seed, int pbits) {

@@ -78,6 +78,9 @@ PROTOTYPES = {
                                          c_i, c_p, c_p, c_p]),
     "det_fast_rcnn_loss_typed": (c_i, [c_p, c_p, c_i, c_p, c_p, c_p, c_l, c_i, c_i, c_f, c_f, c_f, c_f, c_f, c_i, c_f,
                                        c_f, c_f, c_p, c_p, c_p, c_p, c_p, c_p]),
+    "det_roi_sample_workspace_bytes": (c_l, [c_i, c_l, c_l]),
+    "det_roi_sample_proposals": (c_i, [c_p, c_p, c_i, c_l, c_p, c_p, c_p, c_l, c_i, c_p, c_p, c_i, c_i, c_i, c_d, c_i,
+                                       c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_l, c_p]),
     "det_match_workspace_bytes": (c_l, [c_i, c_l, c_l]),
     "det_match_anchors": (c_i, [c_p, c_p, c_i, c_l, c_p, c_l, c_p, c_p, c_i, c_i, c_p, c_p, c_p, c_p, c_l, c_p]),
     "det_match_grid_workspace_bytes": (c_l, [c_i, c_l, c_p, c_i]),
