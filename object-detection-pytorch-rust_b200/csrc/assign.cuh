@@ -98,20 +98,6 @@ __device__ __forceinline__ int label_class(int8_t l) { return l == 0 ? 1 : (l ==
 // per-byte masks (0xff where true) of a word of 4 labels
 __device__ __forceinline__ uint32_t bytes_eq(uint32_t w, uint32_t pattern) { return __vcmpeq4(w, pattern); }
 
-struct CodecW {
-    float wx, wy, ww, wh;
-};
-
-__device__ __forceinline__ float4 encode_target(const float4 s, const float4 t, const CodecW wt) {
-    // Box2BoxTransform.get_deltas, box_regression.py:53-69
-    const float sw = s.z - s.x, sh = s.w - s.y;
-    const float scx = s.x + 0.5f * sw, scy = s.y + 0.5f * sh;
-    const float tw = t.z - t.x, th = t.w - t.y;
-    const float tcx = t.x + 0.5f * tw, tcy = t.y + 0.5f * th;
-    return make_float4(wt.wx * (tcx - scx) / sw, wt.wy * (tcy - scy) / sh, wt.ww * logf(tw / sw),
-                       wt.wh * logf(th / sh));
-}
-
 // smooth-L1 value and derivative wrt the prediction (fvcore semantics: beta < 1e-5 -> pure L1)
 __device__ __forceinline__ void smooth_l1(float pred, float tgt, float beta, float& val, float& grad) {
     const float d = pred - tgt, n = fabsf(d);
@@ -133,7 +119,7 @@ __device__ __forceinline__ void smooth_l1(float pred, float tgt, float beta, flo
 //   iou = I / (U + eps), loss = 1 - iou + (H - U) / (H + eps), I = 0 unless the boxes strictly overlap, eps = 1e-7.
 // Gradient: what autograd produces for that expression composed with Box2BoxTransform.apply_deltas
 // (box_regression.py:87-115): ties of max / min split the gradient in half, clamp(max=) passes it up to equality.
-__device__ __forceinline__ float giou_fwd_bwd(const float4 p, const float4 a, const float4 g, const CodecW wt,
+__device__ __forceinline__ float giou_fwd_bwd(const float4 p, const float4 a, const float4 g, const CodecWeights wt,
                                               float scale_clamp, float4& grad) {
     const float eps = 1e-7f;
     const float w = a.z - a.x, h = a.w - a.y;

@@ -618,7 +618,7 @@ rpn_loss_sampled_kernel(HeadLayoutDev hl, const int32_t* __restrict__ samples, c
                         int sample_cap, const int32_t* __restrict__ clear_samples,
                         const int32_t* __restrict__ clear_count, const int64_t* __restrict__ matched,
                         const int32_t* __restrict__ sample_gt, const float4* __restrict__ gt, const int32_t* __restrict__ gt_off,
-                        const float4* __restrict__ anchors, int64_t r, CodecW wt, float scale_clamp, float beta,
+                        const float4* __restrict__ anchors, int64_t r, CodecWeights wt, float scale_clamp, float beta,
                         float scale_cls, float scale_loc, const float* __restrict__ upstream, float* __restrict__ acc,
                         int32_t* __restrict__ ticket, float* __restrict__ sums_out, int write_grads) {
     __shared__ float s_part[4][kSampledThreads / 32];
@@ -680,7 +680,7 @@ rpn_loss_sampled_kernel(HeadLayoutDev hl, const int32_t* __restrict__ samples, c
                 acc_loc += giou_fwd_bwd(p, anchors[j], g, wt, scale_clamp, dd);
                 gd = make_float4(dd.x * gs_loc, dd.y * gs_loc, dd.z * gs_loc, dd.w * gs_loc);
             } else {
-                const float4 tgt = encode_target(anchors[j], g, wt);
+                const float4 tgt = encode_delta(anchors[j], g, wt);
                 float v, d;
                 smooth_l1(p.x, tgt.x, beta, v, d); acc_loc += v; gd.x = d * gs_loc;
                 smooth_l1(p.y, tgt.y, beta, v, d); acc_loc += v; gd.y = d * gs_loc;
@@ -968,7 +968,7 @@ int det_rpn_loss_sampled(const det_head_level_t* levels_host, int num_levels, in
         DET_CHECK_ARG(with == 0 || with == num_levels, "gradients for all levels or none");
         write_grads = with != 0;
     }
-    const CodecW wt{wx, wy, ww, wh};
+    const CodecWeights wt{wx, wy, ww, wh};
     auto g4 = reinterpret_cast<const float4*>(gt_boxes);
     auto a4 = reinterpret_cast<const float4*>(anchors);
     int32_t* ticket = reinterpret_cast<int32_t*>(accumulators + 8);

@@ -758,7 +758,7 @@ template <bool GIOU>
 __global__ void __launch_bounds__(kLossThreads)
 rpn_loss_kernel(const float* __restrict__ logits, const float4* __restrict__ deltas, const int8_t* __restrict__ labels,
                 const int64_t* __restrict__ matched, const float4* __restrict__ gt, const int32_t* __restrict__ gt_off,
-                const float4* __restrict__ anchors, int64_t total, int64_t r, CodecW wt, float scale_clamp,
+                const float4* __restrict__ anchors, int64_t total, int64_t r, CodecWeights wt, float scale_clamp,
                 float beta, float gs_cls,
                 float gs_loc, const float* __restrict__ upstream, float* __restrict__ acc, float* __restrict__ sums_out,
                 float* __restrict__ grad_logits, float4* __restrict__ grad_deltas) {
@@ -819,7 +819,7 @@ rpn_loss_kernel(const float* __restrict__ logits, const float4* __restrict__ del
                     acc_loc += giou_fwd_bwd(p, anchors[j], g, wt, scale_clamp, dd);
                     gd = make_float4(dd.x * gs_loc, dd.y * gs_loc, dd.z * gs_loc, dd.w * gs_loc);
                 } else {
-                    const float4 tgt = encode_target(anchors[j], g, wt);
+                    const float4 tgt = encode_delta(anchors[j], g, wt);
                     float v, d;
                     smooth_l1(p.x, tgt.x, beta, v, d); acc_loc += v; gd.x = d * gs_loc;
                     smooth_l1(p.y, tgt.y, beta, v, d); acc_loc += v; gd.y = d * gs_loc;
@@ -1197,7 +1197,7 @@ int det_rpn_loss(const float* logits, const float* deltas, const int8_t* labels,
     auto a4 = reinterpret_cast<const float4*>(anchors);
     auto d4 = reinterpret_cast<const float4*>(deltas);
     auto gd4 = reinterpret_cast<float4*>(grad_deltas);
-    const CodecW wt{wx, wy, ww, wh};
+    const CodecWeights wt{wx, wy, ww, wh};
     if (loss_type == 1)
         rpn_loss_kernel<true><<<(unsigned)blocks, kLossThreads, 0, as_stream(stream)>>>(
             logits, d4, labels, matched_idx, g4, gt_offsets, a4, total, r, wt, scale_clamp, smooth_l1_beta, grad_scale_cls,

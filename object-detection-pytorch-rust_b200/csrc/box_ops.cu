@@ -102,7 +102,7 @@ __global__ void matched_iou_kernel(const float4* __restrict__ b1, const float4* 
 // ------------------------------------------------------------------------------------------------
 // box codec
 // ------------------------------------------------------------------------------------------------
-// CodecWeights, decode_delta: common.cuh (shared with roi_detect.cu)
+// CodecWeights, decode_delta, encode_delta: common.cuh (shared with roi_detect.cu and the loss kernels)
 
 __global__ void apply_deltas_kernel(const float4* __restrict__ deltas, const float4* __restrict__ boxes,
                                     int64_t total, int k, CodecWeights wt, float scale_clamp,
@@ -143,16 +143,6 @@ __global__ void apply_deltas_backward_kernel(const float4* __restrict__ deltas, 
         gb.w += gcy * (0.5f + dy) + gph * eh;
     }
     if (grad_boxes) grad_boxes[i] = gb;
-}
-
-// reference get_deltas on one (src, tgt) pair; operation order of box_regression.py:53-69
-__device__ __forceinline__ float4 encode_delta(const float4 s, const float4 t, const CodecWeights wt) {
-    const float sw = s.z - s.x, sh = s.w - s.y;
-    const float scx = s.x + 0.5f * sw, scy = s.y + 0.5f * sh;
-    const float tw = t.z - t.x, th = t.w - t.y;
-    const float tcx = t.x + 0.5f * tw, tcy = t.y + 0.5f * th;
-    return make_float4(wt.wx * (tcx - scx) / sw, wt.wy * (tcy - scy) / sh, wt.ww * logf(tw / sw),
-                       wt.wh * logf(th / sh));
 }
 
 __global__ void get_deltas_kernel(const float4* __restrict__ src, const float4* __restrict__ tgt, int64_t m,

@@ -164,6 +164,17 @@ __device__ __forceinline__ float ld1_stream(const T* p) {
 }
 template <typename T>
 __device__ __forceinline__ float ld1(const T* p) { return Head<T>::f32(*p); }
+// 4-element group q of a (rows, groups * 4) delta tensor as fp32: one vector load when the base is aligned to 4
+// elements (vec), four scalar loads otherwise
+template <typename T>
+__device__ __forceinline__ float4 ld_group(const void* base, int vec, int64_t q) {
+    if (vec) return ld4<T>(static_cast<const typename Head<T>::vec*>(base) + q);
+    const T* p = static_cast<const T*>(base) + q * 4;
+    return make_float4(ld1(p), ld1(p + 1), ld1(p + 2), ld1(p + 3));
+}
+
+// 1 / (1 + e^-x): __frcp_rn is the correctly rounded reciprocal, i.e. bit-identical to the IEEE quotient 1.0f / d
+__device__ __forceinline__ float sigmoidf_rn(float x) { return __frcp_rn(1.0f + expf(-x)); }
 
 __device__ __forceinline__ float box_area(const float4 b) { return (b.z - b.x) * (b.w - b.y); }
 
@@ -184,6 +195,16 @@ __device__ __forceinline__ float4 decode_delta(const float4 box, const float4 d,
     const float pcx = dx * w + cx, pcy = dy * h + cy;
     const float pw = expf(dw) * w, ph = expf(dh) * h;
     return make_float4(pcx - 0.5f * pw, pcy - 0.5f * ph, pcx + 0.5f * pw, pcy + 0.5f * ph);
+}
+
+// reference get_deltas on one (src, tgt) pair; operation order of box_regression.py:53-69
+__device__ __forceinline__ float4 encode_delta(const float4 s, const float4 t, const CodecWeights wt) {
+    const float sw = s.z - s.x, sh = s.w - s.y;
+    const float scx = s.x + 0.5f * sw, scy = s.y + 0.5f * sh;
+    const float tw = t.z - t.x, th = t.w - t.y;
+    const float tcx = t.x + 0.5f * tw, tcy = t.y + 0.5f * th;
+    return make_float4(wt.wx * (tcx - scx) / sw, wt.wy * (tcy - scy) / sh, wt.ww * logf(tw / sw),
+                       wt.wh * logf(th / sh));
 }
 
 // 32-bit key that sorts ASCENDING into torch's descending-score order:

@@ -45,9 +45,6 @@ struct DenseLevelDev {
     int64_t out_offset;
 };
 
-// 1 / (1 + e^-x): __frcp_rn is the correctly rounded reciprocal, i.e. bit-identical to the IEEE quotient 1.0f / d
-__device__ __forceinline__ float sigmoidf_dd(float x) { return __frcp_rn(1.0f + expf(-x)); }
-
 constexpr int kFlatThreads = 128;  // 8 CTAs per SM: at one or two waves (N=32) the finer grain trims the tail, 62.0 -> 61.2 us
 
 struct FlatArgs {
@@ -105,8 +102,8 @@ __device__ __forceinline__ void decode_quad(const FlatArgs& g, int l, long long 
         const float4 q = ld_quad<T, true>(pl + (int64_t)4 * plane, m);
         const float thr = g.score_thresh;
         // `!(x > thr)` also holds for NaN: a NaN objectness gives a NaN score, which is no candidate either
-        if (!(sigmoidf_dd(q.x) > thr) && !(sigmoidf_dd(q.y) > thr) && !(sigmoidf_dd(q.z) > thr) &&
-            !(sigmoidf_dd(q.w) > thr))
+        if (!(sigmoidf_rn(q.x) > thr) && !(sigmoidf_rn(q.y) > thr) && !(sigmoidf_rn(q.z) > thr) &&
+            !(sigmoidf_rn(q.w) > thr))
             active = false;
     }
     float4 box[4];
@@ -162,13 +159,13 @@ __device__ __forceinline__ void decode_quad(const FlatArgs& g, int l, long long 
         for (int v = 0; v < 4; ++v) {
             const int pos = grp * 4 + v;
             const int row = pos / L.w, colx = pos - row * L.w;
-            const float cx = (sigmoidf_dd(t[0][v]) + (float)colx) * L.stride;
-            const float cy = (sigmoidf_dd(t[1][v]) + (float)row) * L.stride;
+            const float cx = (sigmoidf_rn(t[0][v]) + (float)colx) * L.stride;
+            const float cy = (sigmoidf_rn(t[1][v]) + (float)row) * L.stride;
             const float tw = (t[2][v] > g.scale_clamp) ? g.scale_clamp : t[2][v];  // torch.clamp(max=): NaN stays NaN
             const float th = (t[3][v] > g.scale_clamp) ? g.scale_clamp : t[3][v];
             const float bw = expf(tw) * awh.x, bh = expf(th) * awh.y;
             box[v] = make_float4(cx - 0.5f * bw, cy - 0.5f * bh, cx + 0.5f * bw, cy + 0.5f * bh);
-            score[v] = sigmoidf_dd(t[4][v]) * (C > 0 ? sigmoidf_dd(best[v]) : 1.0f);
+            score[v] = sigmoidf_rn(t[4][v]) * (C > 0 ? sigmoidf_rn(best[v]) : 1.0f);
         }
     }
     if (MODE == kModeDense) {
@@ -468,6 +465,38 @@ int64_t det_dense_detect_workspace_bytes(int n, int64_t cand_cap) {
 
 int64_t det_dense_detect_counter_bytes(int n) { return n <= 0 ? 0 : (int64_t)n * kCountStride * 4; }
 
+int det::bind_select_workspace(SelectArgs& sel, int n, int64_t cand_cap, void* workspace, int64_t workspace_bytes,
+                               bool counters_zero, cudaStream_t st) {
+    const int64_t need = det_dense_detect_workspace_bytes(n, cand_cap);
+    if (!workspace || workspace_bytes < need) {
+        set_error("workspace too small: need %lld bytes", (long long)need);
+        return DET_ERR_WORKSPACE;
+    }
+    if (!aligned16(workspace)) {
+        set_error("workspace must be 16-byte aligned");
+        return DET_ERR_ALIGN;
+    }
+    unsigned char* w = static_cast<unsigned char*>(workspace);
+    sel.cand_cap = (int)cand_cap;
+    sel.cand_count = reinterpret_cast<int32_t*>(w);
+    w += (int64_t)n * kCountStride * 4;
+    sel.cand_box = reinterpret_cast<float4*>(w);
+    w += (int64_t)n * cand_cap * 16;
+    sel.cand_score = reinterpret_cast<float*>(w);
+    w += (int64_t)n * cand_cap * 4;
+    sel.cand_cls = reinterpret_cast<int32_t*>(w);
+    w += (int64_t)n * cand_cap * 4;
+    sel.cand_id = reinterpret_cast<int32_t*>(w);
+    // The NMS CTA of an image puts the image's counter back to zero once it has read it and the select kernel clears
+    // the overflow word itself, so a call on a workspace whose counters are known to be zero (gate bit 1: zeroed once by
+    // the caller, then only ever used by this call) is exactly two launches; otherwise the counters are cleared here.
+    if (!counters_zero) {
+        cudaError_t e = cudaMemsetAsync(sel.cand_count, 0, sizeof(int32_t) * (size_t)n * kCountStride, st);
+        if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync");
+    }
+    return DET_OK;
+}
+
 template <typename T>
 static int dense_detect_t(const det_dense_level_t* levels_host, int num_levels, int n, int a, int c, float scale_clamp,
                           float score_thresh, double iou_threshold, int mode, int gate, int64_t cand_cap, int64_t max_det,
@@ -499,38 +528,13 @@ static int dense_detect_t(const det_dense_level_t* levels_host, int num_levels, 
         rows = L.out_offset + (int64_t)L.h * L.w * a > rows ? L.out_offset + (int64_t)L.h * L.w * a : rows;
     }
     DET_CHECK_ARG(rows < (1ll << 31), "too many rows per image");
-    const int64_t need = det_dense_detect_workspace_bytes(n, cand_cap);
-    if (!workspace || workspace_bytes < need) {
-        set_error("workspace too small: need %lld bytes", (long long)need);
-        return DET_ERR_WORKSPACE;
-    }
-    if (!aligned16(workspace)) {
-        set_error("workspace must be 16-byte aligned");
-        return DET_ERR_ALIGN;
-    }
-    unsigned char* w = static_cast<unsigned char*>(workspace);
     SelectArgs sel;
+    int rc = bind_select_workspace(sel, n, cand_cap, workspace, workspace_bytes, gate & 2, st);
+    if (rc != DET_OK) return rc;
     sel.mode = (gate & 1) ? kModeSelectGated : kModeSelect;
     sel.overflow_flag = overflow_flag;
     sel.score_thresh = score_thresh;
-    sel.cand_cap = (int)cand_cap;
-    sel.cand_count = reinterpret_cast<int32_t*>(w);
-    w += (int64_t)n * kCountStride * 4;
-    sel.cand_box = reinterpret_cast<float4*>(w);
-    w += (int64_t)n * cand_cap * 16;
-    sel.cand_score = reinterpret_cast<float*>(w);
-    w += (int64_t)n * cand_cap * 4;
-    sel.cand_cls = reinterpret_cast<int32_t*>(w);
-    w += (int64_t)n * cand_cap * 4;
-    sel.cand_id = reinterpret_cast<int32_t*>(w);
-    // The NMS CTA of an image puts the image's counter back to zero once it has read it and the select kernel clears
-    // the overflow word itself, so a call on a workspace whose counters are known to be zero (gate bit 1: zeroed once by
-    // the caller, then only ever used by this call) is exactly two launches; otherwise the counters are cleared here.
-    if (!(gate & 2)) {
-        cudaError_t e = cudaMemsetAsync(sel.cand_count, 0, sizeof(int32_t) * (size_t)n * kCountStride, st);
-        if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync");
-    }
-    int rc = launch_flat<T>(levels_host, num_levels, n, a, c, scale_clamp, nullptr, nullptr, nullptr, rows, st, &sel);
+    rc = launch_flat<T>(levels_host, num_levels, n, a, c, scale_clamp, nullptr, nullptr, nullptr, rows, st, &sel);
     if (rc != DET_OK) return rc;
     return launch_list_nms(sel, n, float_threshold_below(iou_threshold), mode, max_det, det_idx, det_boxes, det_scores,
                            det_classes, det_count, overflow_flag, st);

@@ -12,7 +12,7 @@
 //   lane).  NC = 0, larger K: the columns are walked three times (max / argmax, exp-sum, gradient); the re-reads hit L1.
 //   Reductions are xor butterflies, so every lane holds the same max, sum and argmax bit for bit.
 //   The lane that owns column gt adds the row's cross-entropy logsumexp - x[gt]; the lane that owns delta group gt (group
-//   0 when class-agnostic) computes the box term with assign.cuh's smooth_l1 / encode_target / giou_fwd_bwd -- the RPN
+//   0 when class-agnostic) computes the box term with smooth_l1 / encode_delta / giou_fwd_bwd -- the RPN
 //   losses' arithmetic.  Gradients: (softmax - onehot) * s_cls for every column, and for every delta group zero except
 //   group gt of a foreground row; all stores streaming, a warp's stores covering consecutive sectors.
 //   Every CTA adds its partial sums to the accumulators with one atomic per sum, and the last CTA writes the 8 weighted
@@ -37,7 +37,7 @@ struct LossArgs {
     const float4* gt_boxes;
     int64_t m;
     int k, agnostic, giou, deltas_vec;
-    CodecW wt;
+    CodecWeights wt;
     float scale_clamp, beta, scale_cls, scale_loc;
     const float* upstream;
     float* acc;
@@ -73,13 +73,6 @@ __device__ __forceinline__ void warp_argmax(float& v, int& i) {
 }
 
 template <typename T>
-__device__ __forceinline__ float4 load_group(const LossArgs& g, int64_t q) {
-    if (g.deltas_vec) return ld4<T>(static_cast<const typename Head<T>::vec*>(g.deltas) + q);
-    const T* p = static_cast<const T*>(g.deltas) + q * 4;
-    return make_float4(ld1(p), ld1(p + 1), ld1(p + 2), ld1(p + 3));
-}
-
-template <typename T>
 __device__ __forceinline__ void store_group(const LossArgs& g, int64_t q, const float4 v) {
     if (g.deltas_vec) {
         st4_stream<T>(static_cast<typename Head<T>::vec*>(g.grad_deltas) + q, v);
@@ -92,13 +85,13 @@ __device__ __forceinline__ void store_group(const LossArgs& g, int64_t q, const 
 // the box term of a foreground row (one lane): adds the loss to part.loc and returns d(loss)/d(deltas) * gs_loc
 template <typename T>
 __device__ __forceinline__ float4 box_term(const LossArgs& g, int64_t row, int64_t q, float gs_loc, LossPart& part) {
-    const float4 d = load_group<T>(g, q);
+    const float4 d = ld_group<T>(g.deltas, g.deltas_vec, q);
     const float4 pr = g.proposals[row], gb = g.gt_boxes[row];
     float4 gd;
     if (g.giou) {
         part.loc += giou_fwd_bwd(d, pr, gb, g.wt, g.scale_clamp, gd);
     } else {
-        const float4 t = encode_target(pr, gb, g.wt);
+        const float4 t = encode_delta(pr, gb, g.wt);
         float v;
         smooth_l1(d.x, t.x, g.beta, v, gd.x); part.loc += v;
         smooth_l1(d.y, t.y, g.beta, v, gd.y); part.loc += v;
@@ -291,7 +284,7 @@ static int fast_rcnn_loss_t(const void* class_logits, const void* box_deltas, co
     g.gt_boxes = reinterpret_cast<const float4*>(gt_boxes);
     g.m = m; g.k = num_classes; g.agnostic = class_agnostic ? 1 : 0; g.giou = loss_type;
     g.deltas_vec = aligned_to(box_deltas, 4 * sizeof(T)) && (!grad_deltas || aligned_to(grad_deltas, 4 * sizeof(T)));
-    g.wt = CodecW{wx, wy, ww, wh};
+    g.wt = CodecWeights{wx, wy, ww, wh};
     g.scale_clamp = scale_clamp; g.beta = smooth_l1_beta; g.scale_cls = scale_cls; g.scale_loc = scale_loc;
     g.upstream = upstream;
     g.acc = accumulators; g.sums_out = sums_out;

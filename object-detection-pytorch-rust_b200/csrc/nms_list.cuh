@@ -735,6 +735,13 @@ struct SelectArgs {
     int32_t* overflow_flag;
 };
 
+// Points the lists of `sel` (and its cand_cap) into `workspace`: counters (one per 128-byte line), boxes, scores,
+// classes, ids -- det_dense_detect_workspace_bytes(n, cand_cap) bytes, 16-byte aligned, else DET_ERR_WORKSPACE /
+// DET_ERR_ALIGN.  The counters are cleared on `st` unless `counters_zero` (gate bit 1: the NMS CTAs leave them zero).
+// Defined in dense_decode.cu.
+int bind_select_workspace(SelectArgs& sel, int n, int64_t cand_cap, void* workspace, int64_t workspace_bytes,
+                          bool counters_zero, cudaStream_t st);
+
 // dense_detect_nms_kernel over the n lists of `sel` (cand_cap <= 4096), launched with programmatic dependent launch
 // behind the select kernel that filled them: the second launch of det_dense_detect and det_roi_detect.  The tie order
 // is ascending cand_id.  Defined in dense_decode.cu.

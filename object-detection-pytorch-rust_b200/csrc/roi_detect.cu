@@ -65,13 +65,9 @@ __device__ __forceinline__ bool finite4(const float4 b) {
     return isfinite(b.x) && isfinite(b.y) && isfinite(b.z) && isfinite(b.w);
 }
 
-template <typename T>
-__device__ __forceinline__ float4 load_delta(const RoiArgs& g, int64_t row, int c) {
-    const int per_row = g.agnostic ? 1 : g.k;
-    const int64_t q = row * per_row + (g.agnostic ? 0 : c);  // 4-element group
-    if (g.deltas_vec) return ld4<T>(static_cast<const typename Head<T>::vec*>(g.deltas) + q);
-    const T* p = static_cast<const T*>(g.deltas) + q * 4;
-    return make_float4(ld1(p), ld1(p + 1), ld1(p + 2), ld1(p + 3));
+// the delta group of (row, class c): group row * K + c, or group row when class-agnostic
+__device__ __forceinline__ int64_t delta_group(const RoiArgs& g, int64_t row, int c) {
+    return row * (g.agnostic ? 1 : g.k) + (g.agnostic ? 0 : c);
 }
 
 // General path (any K up to kRoiMaxClasses): the logits live in the warp's shared-memory slice, the deltas are read
@@ -83,7 +79,7 @@ __device__ __forceinline__ void row_general(const RoiArgs& g, float* xs, int img
     // the box of class c, before clipping
     const float4 prop = g.decoded ? make_float4(0.f, 0.f, 0.f, 0.f) : g.proposals[row];
     auto box_of = [&](int c) {
-        const float4 d = load_delta<T>(g, row, c);
+        const float4 d = ld_group<T>(g.deltas, g.deltas_vec, delta_group(g, row, c));
         return g.decoded ? d : decode_delta(prop, d, g.wt, g.scale_clamp);
     };
     // ---- softmax over the K+1 logits
@@ -188,7 +184,8 @@ __device__ __forceinline__ void row_registers(const RoiArgs& g, float* xs, int i
 #pragma unroll
     for (int j = 0; j < NC; ++j) {
         const int c = lane + 32 * j;
-        bx[j] = c < K ? load_delta<T>(g, row, c) : make_float4(0.f, 0.f, 0.f, 0.f);
+        bx[j] = c < K ? ld_group<T>(g.deltas, g.deltas_vec, delta_group(g, row, c))
+                      : make_float4(0.f, 0.f, 0.f, 0.f);
     }
     float mx = -INFINITY;
 #pragma unroll
@@ -388,38 +385,13 @@ static int roi_detect_t(const void* class_logits, const void* box_deltas, const 
         set_error("proposals and det_boxes must be 16-byte aligned");
         return DET_ERR_ALIGN;
     }
-    const int64_t need = det_roi_detect_workspace_bytes(n, cand_cap);
-    if (!workspace || workspace_bytes < need) {
-        set_error("workspace too small: need %lld bytes", (long long)need);
-        return DET_ERR_WORKSPACE;
-    }
-    if (!aligned16(workspace)) {
-        set_error("workspace must be 16-byte aligned");
-        return DET_ERR_ALIGN;
-    }
-    // the layout of a det_dense_detect workspace: counters (one per 128-byte line), boxes, scores, classes, flat ids
-    unsigned char* w = static_cast<unsigned char*>(workspace);
-    SelectArgs& sel = g.sel;
-    sel.mode = 0;
-    sel.overflow_flag = overflow_flag;
-    sel.score_thresh = score_thresh;
-    sel.cand_cap = (int)cand_cap;
-    sel.cand_count = reinterpret_cast<int32_t*>(w);
-    w += (int64_t)n * kCountStride * 4;
-    sel.cand_box = reinterpret_cast<float4*>(w);
-    w += (int64_t)n * cand_cap * 16;
-    sel.cand_score = reinterpret_cast<float*>(w);
-    w += (int64_t)n * cand_cap * 4;
-    sel.cand_cls = reinterpret_cast<int32_t*>(w);
-    w += (int64_t)n * cand_cap * 4;
-    sel.cand_id = reinterpret_cast<int32_t*>(w);
-    if (!(gate & 2)) {  // gate bit 1: the counters are known to be zero (the NMS CTAs leave them so)
-        cudaError_t e = cudaMemsetAsync(sel.cand_count, 0, sizeof(int32_t) * (size_t)n * kCountStride, st);
-        if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync");
-    }
+    rc = bind_select_workspace(g.sel, n, cand_cap, workspace, workspace_bytes, gate & 2, st);
+    if (rc != DET_OK) return rc;
+    g.sel.overflow_flag = overflow_flag;
+    g.sel.score_thresh = score_thresh;
     rc = launch_roi<true, T>(g, m, st);
     if (rc != DET_OK) return rc;
-    return launch_list_nms(sel, n, float_threshold_below(iou_threshold), mode, max_det, det_idx, det_boxes, det_scores,
+    return launch_list_nms(g.sel, n, float_threshold_below(iou_threshold), mode, max_det, det_idx, det_boxes, det_scores,
                            det_classes, det_count, overflow_flag, st);
 }
 

@@ -76,10 +76,10 @@ yolo_decode_nms_kernel(const HT* __restrict__ head, const float2* __restrict__ p
                 const float cl = (x > prm.scale_clamp) ? prm.scale_clamp : x;  // torch.clamp(max=): NaN stays NaN
                 y = expf(cl);
             } else {
-                y = sigmoidf_ref(x);
+                y = sigmoidf_rn(x);
             }
         } else {
-            y = sigmoidf_ref(x);
+            y = sigmoidf_rn(x);
         }
         hs[i] = y;
     }

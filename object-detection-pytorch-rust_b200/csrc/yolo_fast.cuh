@@ -43,9 +43,6 @@ struct YoloParams {
     int flat32;  // det_flat points to int32 (serving wire format: 4 bytes less per detection over PCIe) instead of int64
 };
 
-// 1 / (1 + e^-x): __frcp_rn is the correctly rounded reciprocal, i.e. bit-identical to the IEEE quotient 1.0f / d
-__device__ __forceinline__ float sigmoidf_ref(float x) { return __frcp_rn(1.0f + expf(-x)); }
-
 struct FastLayout {
     int hs_floats, pp, cls_stride, pcp;
     size_t bytes;
@@ -123,11 +120,11 @@ yolo_fast_kernel(const HT* __restrict__ head, const float2* __restrict__ priors,
         if (k < B * 5) {
             const int bi = k / 5, comp = k - bi * 5;
             if (comp == 2 || comp == 3) return expf((x > prm.scale_clamp) ? prm.scale_clamp : x);  // clamp(max=): NaN stays
-            const float y = sigmoidf_ref(x);
+            const float y = sigmoidf_rn(x);
             if (comp == 4 && dense_conf) dense_conf[(int64_t)img * P + cell * B + bi] = y;
             return y;
         }
-        return sigmoidf_ref(x);
+        return sigmoidf_rn(x);
     };
     for (int64_t v = (g0 >> 2) + tid; v < ((g1 + 3) >> 2); v += T) {
         const int64_t base = v << 2;

@@ -9,8 +9,8 @@ from .structures import (Boxes, Instances, pairwise_iou, pairwise_ioa, pairwise_
                          matched_boxlist_iou)
 from .box_regression import Box2BoxTransform
 from .anchors import AnchorGenerator, generate_cell_anchors
-from .nms import batched_nms, nms, nms_images
-from .yolo import YoloGridHead, DenseAnchorHead, YoloGridTrainer, YoloHostPipeline, DenseDetectWorkspace
+from .nms import batched_nms, nms, nms_images, DenseDetectWorkspace
+from .yolo import YoloGridHead, DenseAnchorHead, YoloGridTrainer, YoloHostPipeline
 from .matcher import Matcher, subsample_labels_
 from .proposals import find_top_rpn_proposals, rpn_proposals_batched, add_ground_truth_to_proposals
 from .rpn import RegionProposalNetwork, Assignment, _dense_box_regression_loss

@@ -16,9 +16,8 @@ import torch
 
 from . import _native as N
 from .box_regression import Box2BoxTransform
-from .nms import MODE_AUTO, nms_images
+from .nms import MODE_AUTO, detect_unfused, detect_workspace, detection_buffers
 from .structures import Boxes, Instances
-from .yolo import DenseDetectWorkspace
 
 ROI_HEAD_WEIGHTS = (10.0, 10.0, 5.0, 5.0)  # detectron2's ROI_BOX_HEAD.BBOX_REG_WEIGHTS default
 
@@ -36,42 +35,21 @@ def _sizes_tensor(image_shapes: Sequence[Tuple[int, int]], device) -> torch.Tens
 
 def _select_dense(rows, cols, code, proposals, offsets, sizes, n, p_max, K, agnostic, decoded, weights, scale_clamp,
                   score_thresh, nms_thresh, max_det, mode):
-    """The exact route for any candidate count: det_roi_decode_dense_typed -> det_threshold_compact (row-major
-    candidates, classes = flat % K) -> det_nms_batched -> det_gather_detections.  Library kernels only, no host sync.
-    max_det < 0: every kept detection (max_det = p_max * K)."""
+    """The exact route for any candidate count: det_roi_decode_dense_typed -> nms.detect_unfused on the (n, p_max * K)
+    rows with classes = flat % K.  Library kernels only, no host sync.  max_det < 0: every kept detection
+    (max_det = p_max * K)."""
     dev = rows.device
     R = p_max * K
     max_det = max(R, 1) if max_det < 0 else max_det
-    out = {"idx": torch.empty((n, max_det), dtype=torch.int64, device=dev),
-           "boxes": torch.empty((n, max_det, 4), dtype=torch.float32, device=dev),
-           "scores": torch.empty((n, max_det), dtype=torch.float32, device=dev),
-           "classes": torch.empty((n, max_det), dtype=torch.int64, device=dev),
-           "overflow": torch.zeros((1,), dtype=torch.int32, device=dev)}
-    if n == 0 or R == 0:
-        out["count"] = torch.zeros((n,), dtype=torch.int32, device=dev)
-        return out
     scores = torch.empty((n, R), dtype=torch.float32, device=dev)
     boxes = torch.empty((n, R, 4), dtype=torch.float32, device=dev)
-    with torch.cuda.device(dev):
-        N.call("det_roi_decode_dense_typed", N.ptr(rows), N.ptr(cols), code, N.ptr(proposals), N.ptr(offsets), n,
-               rows.shape[0], K, int(agnostic), N.ptr(sizes), *weights, scale_clamp, int(decoded), p_max, N.ptr(scores),
-               N.ptr(boxes), N.stream())
+    if n and R:
+        with torch.cuda.device(dev):
+            N.call("det_roi_decode_dense_typed", N.ptr(rows), N.ptr(cols), code, N.ptr(proposals), N.ptr(offsets), n,
+                   rows.shape[0], K, int(agnostic), N.ptr(sizes), *weights, scale_clamp, int(decoded), p_max,
+                   N.ptr(scores), N.ptr(boxes), N.stream())
     classes = torch.arange(K, dtype=torch.int64, device=dev).repeat(n * p_max).view(n, R)
-    cand_rows = torch.empty((n, R), dtype=torch.int64, device=dev)
-    cb = torch.empty((n, R, 4), dtype=torch.float32, device=dev)
-    cs = torch.empty((n, R), dtype=torch.float32, device=dev)
-    cc = torch.empty((n, R), dtype=torch.int64, device=dev)
-    counts = torch.empty((n,), dtype=torch.int32, device=dev)
-    with torch.cuda.device(dev):
-        N.call("det_threshold_compact", N.ptr(boxes), N.ptr(scores), N.ptr(classes), n, R, float(score_thresh), R,
-               N.ptr(cand_rows), N.ptr(cb), N.ptr(cs), N.ptr(cc), N.ptr(counts), N.stream())
-    keep, cnt = nms_images(cb, cs, cc, counts, nms_thresh, max_det, mode)
-    with torch.cuda.device(dev):
-        N.call("det_gather_detections", N.ptr(keep), N.ptr(cnt), n, max_det, N.ptr(cand_rows), N.ptr(cb), N.ptr(cs),
-               N.ptr(cc), R, N.ptr(out["idx"]), N.ptr(out["boxes"]), N.ptr(out["scores"]), N.ptr(out["classes"]),
-               N.stream())
-    out["count"] = cnt
-    return out
+    return detect_unfused(boxes, scores, classes, score_thresh, nms_thresh, max_det, mode)
 
 
 def _instances(out, image_shapes, K):
@@ -180,21 +158,10 @@ class FastRCNNOutputs:
         sizes = image_sizes.detach().to(torch.int32).contiguous()
         max_det = self.topk_per_image if self.topk_per_image >= 0 else self.cand_cap
         if out is None:
-            out = {"idx": torch.empty((n, max_det), dtype=torch.int64, device=dev),
-                   "boxes": torch.empty((n, max_det, 4), dtype=torch.float32, device=dev),
-                   "scores": torch.empty((n, max_det), dtype=torch.float32, device=dev),
-                   "classes": torch.empty((n, max_det), dtype=torch.int64, device=dev),
-                   "count": torch.empty((n,), dtype=torch.int32, device=dev),
-                   "overflow": torch.empty((1,), dtype=torch.int32, device=dev)}
+            out = detection_buffers(n, max_det, dev)
         if n == 0:
             return out
-        wsb = N.fn("det_roi_detect_workspace_bytes")(n, self.cand_cap)
-        gate = 0
-        if isinstance(workspace, DenseDetectWorkspace):
-            workspace = workspace.claim(n, self.cand_cap, dev)
-            gate = 2  # counters zeroed once at construction and left zero by every call: no memset node
-        elif workspace is None or workspace.numel() < wsb:
-            workspace = torch.empty((wsb,), dtype=torch.uint8, device=dev)
+        workspace, wsb, gate = detect_workspace(workspace, n, self.cand_cap, dev)
         w = self.box2box_transform
         with torch.cuda.device(dev):
             N.call("det_roi_detect_typed", N.ptr(lg), N.ptr(dl), code, N.ptr(props), N.ptr(offsets), n, lg.shape[0], K,

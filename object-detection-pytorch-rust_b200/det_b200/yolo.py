@@ -13,7 +13,7 @@ import torch
 
 from . import _native as N
 from .matcher import Matcher
-from .nms import nms_images, MODE_AUTO
+from .nms import nms_images, MODE_AUTO, detect_unfused, detect_workspace, detection_buffers
 
 _DEFAULT_SCALE_CLAMP = math.log(1000.0 / 16)
 
@@ -166,28 +166,6 @@ class YoloHostPipeline:
         self.h_in[0].copy_(host_head)
         self.launch(0)
         return self.wait(0)
-
-
-class DenseDetectWorkspace:
-    """Scratch memory of det_dense_detect that is used for nothing else: the per-image candidate counters at its head are
-    zeroed once here and every call leaves them zero, so ``detect_thresholded(..., workspace=this)`` is exactly two
-    launches (no memset node).  One object per stream of calls in flight."""
-
-    def __init__(self, n: int, cand_cap: int, device):
-        self.n, self.cand_cap, self.device = int(n), int(cand_cap), self._norm(device)
-        nbytes = N.fn("det_dense_detect_workspace_bytes")(self.n, self.cand_cap)
-        self.buf = torch.empty((nbytes,), dtype=torch.uint8, device=self.device)
-        self.buf[:N.fn("det_dense_detect_counter_bytes")(self.n)].zero_()
-
-    @staticmethod
-    def _norm(device) -> torch.device:
-        d = torch.device(device)
-        return torch.device("cuda", torch.cuda.current_device()) if d.type == "cuda" and d.index is None else d
-
-    def claim(self, n: int, cand_cap: int, device) -> torch.Tensor:
-        if (n, cand_cap) != (self.n, self.cand_cap) or self._norm(device) != self.device:
-            raise ValueError(f"DenseDetectWorkspace was built for n={self.n}, cand_cap={self.cand_cap} on {self.device}")
-        return self.buf
 
 
 class _FusedYoloLoss(torch.autograd.Function):
@@ -395,23 +373,13 @@ class DenseAnchorHead:
         if not self.fused_ok(heads) or cand_cap > 4096:
             return self._detect_thresholded_unfused(heads, score_thresh, iou_thresh, max_det, mode)
         if out is None:
-            out = {"idx": torch.empty((n, max_det), dtype=torch.int64, device=dev),
-                   "boxes": torch.empty((n, max_det, 4), dtype=torch.float32, device=dev),
-                   "scores": torch.empty((n, max_det), dtype=torch.float32, device=dev),
-                   "classes": torch.empty((n, max_det), dtype=torch.int64, device=dev),
-                   "count": torch.empty((n,), dtype=torch.int32, device=dev),
-                   "overflow": torch.empty((1,), dtype=torch.int32, device=dev)}
+            out = detection_buffers(n, max_det, dev)
         if n == 0:
             return out
         lv, hcs, _, na, _ = self._levels(heads)
         code = N.DTYPE_CODES[hcs[0].dtype]
-        wsb = N.fn("det_dense_detect_workspace_bytes")(n, int(cand_cap))
-        flags = 1 if gate else 0
-        if isinstance(workspace, DenseDetectWorkspace):
-            workspace = workspace.claim(n, int(cand_cap), dev)
-            flags |= 2  # counters zeroed once at construction and left zero by every call: no memset node
-        elif workspace is None or workspace.numel() < wsb:
-            workspace = torch.empty((wsb,), dtype=torch.uint8, device=dev)
+        workspace, wsb, zeroed = detect_workspace(workspace, n, int(cand_cap), dev)
+        flags = (1 if gate else 0) | zeroed
         with torch.cuda.device(dev):
             N.call("det_dense_detect_typed", ctypes.cast(lv, ctypes.c_void_p), len(hcs), n, na, self.C,
                    self.scale_clamp, float(score_thresh), float(iou_thresh), int(mode), flags, int(cand_cap), max_det,
@@ -422,35 +390,10 @@ class DenseAnchorHead:
         return out
 
     def _detect_thresholded_unfused(self, heads, score_thresh, iou_thresh, max_det, mode):
-        """Same contract through det_dense_decode -> det_threshold_compact (row-ordered candidates) -> det_nms_batched ->
-        det_gather_detections: any candidate count up to 131071 per image, library kernels only, no host sync."""
+        """Same contract through det_dense_decode -> nms.detect_unfused: any candidate count up to 131071 per image,
+        library kernels only, no host sync."""
         boxes, scores, classes = self.decode(heads)
-        n, R = scores.shape
-        dev = scores.device
-        cap = max(int(R), 1)
-        rows = torch.empty((n, cap), dtype=torch.int64, device=dev)
-        cb = torch.empty((n, cap, 4), dtype=torch.float32, device=dev)
-        cs = torch.empty((n, cap), dtype=torch.float32, device=dev)
-        cc = torch.empty((n, cap), dtype=torch.int64, device=dev)
-        counts = torch.empty((n,), dtype=torch.int32, device=dev)
-        out = {"idx": torch.empty((n, max_det), dtype=torch.int64, device=dev),
-               "boxes": torch.empty((n, max_det, 4), dtype=torch.float32, device=dev),
-               "scores": torch.empty((n, max_det), dtype=torch.float32, device=dev),
-               "classes": torch.empty((n, max_det), dtype=torch.int64, device=dev),
-               "overflow": torch.zeros((1,), dtype=torch.int32, device=dev)}
-        if n == 0 or R == 0:
-            out["count"] = torch.zeros((n,), dtype=torch.int32, device=dev)
-            return out
-        with torch.cuda.device(dev):
-            N.call("det_threshold_compact", N.ptr(boxes), N.ptr(scores), N.ptr(classes), n, R, float(score_thresh), cap,
-                   N.ptr(rows), N.ptr(cb), N.ptr(cs), N.ptr(cc), N.ptr(counts), N.stream())
-        keep, cnt = nms_images(cb, cs, cc, counts, iou_thresh, max_det, mode)
-        with torch.cuda.device(dev):
-            N.call("det_gather_detections", N.ptr(keep), N.ptr(cnt), n, max_det, N.ptr(rows), N.ptr(cb), N.ptr(cs),
-                   N.ptr(cc), cap, N.ptr(out["idx"]), N.ptr(out["boxes"]), N.ptr(out["scores"]), N.ptr(out["classes"]),
-                   N.stream())
-        out["count"] = cnt
-        return out
+        return detect_unfused(boxes, scores, classes, score_thresh, iou_thresh, max_det, mode)
 
     def detect(self, heads: List[torch.Tensor], iou_thresh: float = 0.5, max_det: Optional[int] = None,
                mode: int = MODE_AUTO):
