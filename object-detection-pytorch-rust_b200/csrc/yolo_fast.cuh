@@ -9,12 +9,12 @@
 //   T  tier cut: only the first max_det kept detections (global score order) are output and a box can only be
 //      suppressed by higher-scored ones, so the NMS first runs on the candidates above a histogram cut holding about
 //      4/3 max_det of them; if that yields max_det kept boxes the rest cannot matter, else everything is redone
-//   C  order-preserving ballot compaction of the class's candidates
-//   D  rank-by-counting sort (score descending, predictor ascending) -> boxes (+ coordinate offset when the
-//      image takes torchvision's offset-trick branch), areas and scores in sorted order
-//   E  every unordered pair of the class tested exactly once, load-balanced over the 32 lanes; a hit sets one bit
-//      of the earlier box's suppression row (shared-memory atomicOr) and flags the row as non-empty
-//   F  greedy resolution on the bit rows alone, visiting only non-empty rows
+//   E  pair filter, once per image: every unordered pair of PREDICTORS is tested once, by all warps, with a conservative
+//      bound that holds in every class's shifted frame (see pair_may_suppress); a pass sets a bit of the symmetric
+//      predictor matrix `edge`.  Every class uses the same boxes, and nearly all pairs are far below the threshold.
+//   R  per class, on `edge`: a tier candidate with no edge to another candidate of its class is kept; the others are
+//      resolved greedily in (score descending, predictor ascending) order, each in-class edge decided by the exact
+//      nms_suppresses on the class's (shifted) boxes -- the same decision as a sweep over all pairs of the class
 //   M  the kept detections of all classes are put in output order by a counting sort on a 256-bin score histogram
 //      (suffix scan -> bin-grouped placement -> rank inside the bin by direct comparison): no second sort
 // Images whose offset-trick branch cannot be swept per class (non-finite or <= -1 coordinates: only possible with
@@ -43,21 +43,17 @@ struct YoloParams {
     int flat32;  // det_flat points to int32 (serving wire format: 4 bytes less per detection over PCIe) instead of int64
 };
 
+// dynamic shared memory: staged head float[hs_floats] | boxes float4[pp] | merge: two u64 key buffers + one state byte
+// per (predictor, class)
 struct FastLayout {
-    int hs_floats, pp, cls_stride, pcp;
+    int hs_floats, pp, pcp;
     size_t bytes;
     __host__ __device__ constexpr FastLayout(int s2, int ch, int p, int c)
         : hs_floats((s2 * ch + 3) & ~3),
           pp((p + 3) & ~3),
-          // per class: sbox float4[pp] | rows uint4[pp] | sarea float[pp] | skey u32[pp] | spred u8[pad16(pp)]
-          cls_stride(((p + 3) & ~3) * 40 + ((((p + 3) & ~3) + 15) & ~15)),
           pcp((p * c + 3) & ~3),
-          bytes(0) {
-        size_t cls_bytes = (size_t)cls_stride * c;
-        const size_t merge_bytes = (size_t)pcp * 17 + 16;  // two u64 key buffers + one state byte per (p, c)
-        if (cls_bytes < merge_bytes) cls_bytes = merge_bytes;
-        bytes = (size_t)hs_floats * 4 + (size_t)pp * 16 + ((cls_bytes + 15) & ~(size_t)15);
-    }
+          bytes((size_t)((s2 * ch + 3) & ~3) * 4 + (size_t)((p + 3) & ~3) * 16 +
+                ((((size_t)((p * c + 3) & ~3) * 17 + 16) + 15) & ~(size_t)15)) {}
 };
 
 // histogram bin of a score: bits in [base, 0x3F800000], `shift` chosen so that the range spans <= 256 bins
@@ -66,6 +62,41 @@ __device__ __forceinline__ int score_bin(unsigned bits, unsigned base, int shift
 }
 __device__ __forceinline__ int score_shift(unsigned base) {
     return 0x3F800000u > base ? max(0, 32 - __clz(0x3F800000u - base) - 8) : 0;
+}
+
+// Pair filter: may box a suppress box b (or b suppress a) in SOME class frame?  Must be true whenever
+// nms_suppresses(a + off, area, b + off, area, thr_f) is, for every shift off = fl(c * span) the image uses (off = 0
+// in the per-category branch); the exact test then decides the pairs it lets through.
+//   Inputs: thr_f >= 2^-60; r = max(1, largest |coordinate| of the image's candidate boxes) + the largest shift, r < 2^60
+//   (the caller makes every pair an edge otherwise: a non-finite candidate coordinate makes r non-finite); dl = r * 2^-20;
+//   al = lower_area(a, dl).  Only pairs of candidate boxes matter.  Let R be r before rounding and u = 2^-24.
+//   1. Every shifted coordinate fl(v + off) is within u R of v + off, and |v + off| <= R.  A difference of two of them
+//      (the same axis) is within 2uR of the unshifted real difference, and rounding it adds at most u * 2R(1+u): the
+//      class frame's w' = fl(min(z') - max(x')) (min/max commute with the monotone shift) and a box's own side are
+//      within 4.0001 uR of the real unshifted value.
+//   2. dl >= 15.99 uR.  fl(min(z) - max(x)) is within 2uR of the real value, so wu = fl(fl(min(z) - max(x)) + dl) >= w'
+//      (the margin left, > 7 uR, covers the rounding of the sum), and max(0, wu) >= max(0, w').  Likewise
+//      max(0, fl(fl(x2 - x1) - dl)) <= the class frame's side of a box whenever that side is >= 0.
+//   3. The exact test suppresses only if inter' > 0 (threshold >= 0), i.e. w', h' > 0: both boxes then have positive
+//      sides in the class frame and inter' <= area_a', area_b', so denom' >= inter' > 0 (no overflow: r < 2^60).
+//      Rounding is monotone and every operand below is >= 0, so iu = fl(wu * hu) >= inter', al <= area_a',
+//      bl <= area_b', and den = fl(fl(al + bl) - iu) <= denom'.
+//   4. Suppression needs fl(inter' / denom') > thr_f, so the real quotient exceeds thr_f and iu > thr_f * den.  With
+//      den >= 2^-60 the product thr_lo * den is normal, and thr_lo = fl(thr_f * (1 - 2^-20)) gives fl(thr_lo * den) <
+//      thr_f * den (an overflow to inf would need thr_f * den > 2^127 > iu): the test below then passes.  den < 2^-60
+//      passes as well.
+// The bound is symmetric in a and b, so one test covers both orders.  The margin only adds pairs: dl is about 0.01 px at
+// the largest shifted coordinate of a 448 x 448, 20-class image.
+__device__ __forceinline__ float lower_area(const float4 a, float dl) {
+    return fmaxf(0.0f, (a.z - a.x) - dl) * fmaxf(0.0f, (a.w - a.y) - dl);
+}
+__device__ __forceinline__ bool pair_may_suppress(const float4 a, float al, const float4 b, float dl, float thr_lo) {
+    const float wu = fmaxf(0.0f, (fminf(a.z, b.z) - fmaxf(a.x, b.x)) + dl);
+    const float hu = fmaxf(0.0f, (fminf(a.w, b.w) - fmaxf(a.y, b.y)) + dl);
+    const float iu = wu * hu;
+    if (iu == 0.0f) return false;
+    const float den = (al + lower_area(b, dl)) - iu;
+    return !(den >= 0x1p-60f && iu <= thr_lo * den);
 }
 
 template <int MAXT, int MINB, int CS, int CB, int CC, typename HT = float>
@@ -81,12 +112,12 @@ yolo_fast_kernel(const HT* __restrict__ head, const float2* __restrict__ priors,
     const int Pp = lay.pp;
     float* hs = reinterpret_cast<float*>(smem_raw);
     float4* pbox = reinterpret_cast<float4*>(hs + lay.hs_floats);
-    unsigned char* cls_region = reinterpret_cast<unsigned char*>(pbox + Pp);
+    uint64_t* buf_a = reinterpret_cast<uint64_t*>(pbox + Pp);  // merge key buffers (and the slow path's state bytes)
+    uint64_t* buf_b = buf_a + lay.pcp;
     __shared__ int s_m[kFastMaxC];
     __shared__ float s_mx[4], s_mn[4];
     __shared__ int s_fl[4];
-    __shared__ unsigned s_nz[kFastMaxC][4];
-    __shared__ __align__(16) int4 s_work[kFastMaxC];  // per class: candidates, 32-item chunks of pair tests, 2^32/half
+    __shared__ __align__(16) uint4 s_edge[kFastMaxP];  // symmetric pair-filter matrix: bit q of row p = pair (p, q)
     __shared__ int s_total;
     __shared__ struct {
         int cnt, gcat;
@@ -98,7 +129,6 @@ yolo_fast_kernel(const HT* __restrict__ head, const float2* __restrict__ priors,
     __shared__ int s_base[kFastBins];
     const unsigned FULL = 0xffffffffu;
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5, T = blockDim.x;
-    const unsigned lt_mask = (1u << lane) - 1u;
     const int img = blockIdx.x;
     const int K = (int)min(prm.max_det, (int64_t)PC);
 
@@ -107,6 +137,7 @@ yolo_fast_kernel(const HT* __restrict__ head, const float2* __restrict__ priors,
         s_hist[i] = 0;
         s_hist2[i] = 0;
     }
+    for (int i = tid; i < P; i += T) s_edge[i] = make_uint4(0u, 0u, 0u, 0u);
     if (tid == 0) s_total = 0;
     pdl_wait();     // everything earlier in the stream is complete and visible from here on
     DET_MARK(0);
@@ -290,12 +321,46 @@ yolo_fast_kernel(const HT* __restrict__ head, const float2* __restrict__ priors,
     const unsigned tier_cut[3] = {s_img.cut[0], s_img.cut[1], 0u};
     DET_MARK(2);
 
-    uint64_t* buf_a = reinterpret_cast<uint64_t*>(cls_region);
-    uint64_t* buf_b = buf_a + lay.pcp;
     const uint64_t* fin_keys = buf_a;
     int nout = 0;
 
     if (by_cat) {
+        // ---- E: pair filter over all predictor pairs, once per image (pair_may_suppress).  Row i meets the partners
+        // (i + d) mod P, d = 1 .. P/2 (every unordered pair once); the T / P threads of a row split its partners, so box
+        // i and its area bound are loaded once per thread.
+        if (cnt > 0) {
+            const float max_off = trick ? (float)gcat * span : 0.0f;  // the largest shift of a class with candidates
+            const float r = max_nan(max_nan(fabsf(gmx), fabsf(gmn)), 1.0f) + max_off;
+            const bool every = !(thr_f >= 0x1p-60f) || !(r < 0x1p60f);
+            const float dl = r * 0x1p-20f;
+            const float thr_lo = thr_f * (1.0f - 0x1p-20f);
+            const int half = P >> 1, per_row = T / P, chunk = (half + per_row - 1) / per_row;
+            const int i = tid % P, g = tid / P;
+            if (g < per_row && half > 0) {
+                const float4 a = pbox[i];
+                const float al = lower_area(a, dl);
+                const int d0 = g * chunk + 1, d1 = min(half, d0 + chunk - 1);
+                int j = i + d0 >= P ? i + d0 - P : i + d0;
+                for (int d = d0; d <= d1; ++d) {
+                    // distance-P/2 pairs (P even) are met from both ends: taken from the lower half only
+                    if (!((P & 1) == 0 && d == half && i >= half) && (every || pair_may_suppress(a, al, pbox[j], dl, thr_lo))) {
+                        atomicOr(reinterpret_cast<unsigned*>(&s_edge[i]) + (j >> 5), 1u << (j & 31));
+                        atomicOr(reinterpret_cast<unsigned*>(&s_edge[j]) + (i >> 5), 1u << (i & 31));
+                    }
+                    j = j + 1 == P ? 0 : j + 1;
+                }
+            }
+        }
+        __syncthreads();
+        DET_MARK(5);
+        const float off = trick ? (float)c * span : 0.0f;  // idxs.to(boxes) * (max_coordinate + 1)
+        auto class_box = [&](int p) -> float4 {
+            float4 b = pbox[p];
+            if (trick) {
+                b.x += off; b.y += off; b.z += off; b.w += off;
+            }
+            return b;
+        };
         uint64_t mykey[4];
         bool mine_kept[4];
         unsigned base2 = 0u;
@@ -307,159 +372,89 @@ yolo_fast_kernel(const HT* __restrict__ head, const float2* __restrict__ priors,
             shift2 = score_shift(base2);
 #pragma unroll
             for (int k = 0; k < 4; ++k) mine_kept[k] = false;
-            unsigned char* my = cls_region + (size_t)(cls_warp ? c : 0) * lay.cls_stride;
-            unsigned* skey = reinterpret_cast<unsigned*>(my + Pp * 36);
-            unsigned char* spred = my + Pp * 40;
-            int m = 0;
             if (cls_warp) {
-                float4* sbox = reinterpret_cast<float4*>(my);
-                uint4* rows4 = reinterpret_cast<uint4*>(my + Pp * 16);
-                unsigned* rows = reinterpret_cast<unsigned*>(rows4);
-                float* sarea = reinterpret_cast<float*>(my + Pp * 32);
-                unsigned* ckey = rows;  // unsorted candidates live in the row storage until the rows are needed
-                unsigned char* cp = reinterpret_cast<unsigned char*>(rows + Pp);
-                // ---- C: order-preserving compaction (predictor ascending)
+                // ---- R: the class's tier candidates (bit p = predictor p), and those with an edge to another of them
+                unsigned kept[4], open[4];
+#pragma unroll
+                for (int k = 0; k < 4; ++k) kept[k] = __ballot_sync(FULL, pass[k] && __float_as_uint(sc[k]) >= cut_bits);
 #pragma unroll
                 for (int k = 0; k < 4; ++k) {
-                    const bool in = pass[k] && __float_as_uint(sc[k]) >= cut_bits;
-                    const unsigned bal = __ballot_sync(FULL, in);
-                    if (in) {
-                        const int pos = m + __popc(bal & lt_mask);
-                        ckey[pos] = __float_as_uint(sc[k]);  // scores are >= +0: bit patterns order like the values
-                        cp[pos] = (unsigned char)(lane + 32 * k);
+                    bool touched = false;
+                    if ((kept[k] >> lane) & 1u) {
+                        const uint4 e = s_edge[lane + 32 * k];
+                        touched = ((e.x & kept[0]) | (e.y & kept[1]) | (e.z & kept[2]) | (e.w & kept[3])) != 0u;
                     }
-                    m += __popc(bal);
+                    open[k] = __ballot_sync(FULL, touched);
                 }
-                __syncwarp();
-                DET_MARK(5);
-                // ---- D: rank by counting -> sorted order (score descending, predictor ascending)
-                const float off = trick ? (float)c * span : 0.0f;  // idxs.to(boxes) * (max_coordinate + 1)
-                for (int i0 = 0; i0 < m; i0 += 32) {
-                    const int i = i0 + lane;
-                    const bool has = i < m;
-                    const unsigned si = has ? ckey[i] : 0u;
-                    int rank = 0;
-#pragma unroll 4
-                    for (int j = 0; j < m; ++j) {
-                        const unsigned sj = ckey[j];
-                        rank += ((sj > si) || (sj == si && j < i)) ? 1 : 0;
-                    }
-                    if (has) {
-                        const int p = (int)cp[i];
-                        float4 b = pbox[p];
-                        if (trick) {
-                            b.x += off; b.y += off; b.z += off; b.w += off;
-                        }
-                        sbox[rank] = b;
-                        sarea[rank] = box_area(b);
-                        skey[rank] = si;
-                        spred[rank] = (unsigned char)p;
-                    }
-                }
-                __syncwarp();
-                for (int r = lane; r < m; r += 32) rows4[r] = make_uint4(0u, 0u, 0u, 0u);
-                if (lane < 4) s_nz[c][lane] = 0u;
-                if (lane == 0) {
-                    // the class's pair items (m * floor(m/2), see E) in chunks of 32 for the CTA-wide sweep below
-                    const int half = m >> 1;
-                    s_work[c] = make_int4(m, m >= 2 ? (m * half + 31) >> 5 : 0,
-                                          half > 1 ? (int)((0xFFFFFFFFu / (unsigned)half) + 1u) : 0, 0);
-                }
-                DET_MARK(6);
-            } else if (wid < kFastMaxC && lane == 0) {
-                s_work[wid] = make_int4(0, 0, 0, 0);
-            }
-            __syncthreads();
-            // ---- E: every unordered pair of every class exactly once.  A class of m candidates has m * floor(m/2) items
-            // (item q -> row r = q / half, distance d = q % half + 1, partner (r + d) mod m), cut into chunks of 32; the
-            // chunks of ALL classes are dealt round-robin to the warps of the CTA, so a class with many candidates no
-            // longer holds up the image (the classes' sizes differ by 2-3x and the work is quadratic in them).
-            {
-                const int nw = T >> 5;
-                const int4 wk = lane < C ? s_work[lane] : make_int4(0, 0, 0, 0);
-                int incl = wk.y;  // inclusive scan of the chunk counts over the classes (lane = class)
+                // greedy over the open candidates: the best one (score descending, predictor ascending) is kept, and the
+                // open candidates it shares an edge with are tested against it exactly.  Scores are >= +0: bit patterns
+                // order like the values.
+                while (open[0] | open[1] | open[2] | open[3]) {
+                    unsigned best = 0u;
+                    int bp = -1;
 #pragma unroll
-                for (int o = 1; o < 32; o <<= 1) {
-                    const int v = __shfl_up_sync(FULL, incl, o);
-                    if (lane >= o) incl += v;
-                }
-                const int chunks = __shfl_sync(FULL, incl, 31);
-                for (int g = wid; g < chunks; g += nw) {
-                    const int cls = __popc(__ballot_sync(FULL, incl <= g));  // classes that end at or before chunk g
-                    const int first = __shfl_sync(FULL, incl - wk.y, cls);
-                    const int mm = __shfl_sync(FULL, wk.x, cls);
-                    const unsigned inv = (unsigned)__shfl_sync(FULL, wk.z, cls);
-                    const int half = mm >> 1, items = mm * half;
-                    const int q = ((g - first) << 5) + lane;
-                    if (q >= items) continue;
-                    unsigned char* cm = cls_region + (size_t)cls * lay.cls_stride;
-                    const float4* cbox = reinterpret_cast<const float4*>(cm);
-                    unsigned* crows = reinterpret_cast<unsigned*>(cm + Pp * 16);
-                    const float* carea = reinterpret_cast<const float*>(cm + Pp * 32);
-                    const int r = half > 1 ? (int)__umulhi((unsigned)q, inv) : q;
-                    const int d = q - r * half + 1;
-                    if (((mm & 1) == 0) && d == half && r >= half) continue;  // distance-m/2 pairs: from the lower half only
-                    int j = r + d;
-                    j = (j >= mm) ? j - mm : j;
-                    const int lo = min(r, j), hi = max(r, j);
-                    const float4 ba = cbox[lo], bb = cbox[hi];
-                    const float aa = carea[lo], ab = carea[hi];
-                    const bool hit = nonan ? nms_suppresses<true>(ba, aa, bb, ab, thr_f)
-                                           : nms_suppresses<false>(ba, aa, bb, ab, thr_f);
-                    if (hit) {
-                        atomicOr(crows + lo * 4 + (hi >> 5), 1u << (hi & 31));
-                        atomicOr(&s_nz[cls][lo >> 5], 1u << (lo & 31));
-                    }
-                }
-            }
-            __syncthreads();
-            DET_MARK(7);
-            if (cls_warp) {
-                const uint4* rows4 = reinterpret_cast<const uint4*>(my + Pp * 16);
-                // ---- F: greedy resolution on the bit rows (uniform across the warp), only non-empty rows matter
-                unsigned alive[4];
-#pragma unroll
-                for (int w = 0; w < 4; ++w) {
-                    const int bits = min(32, max(0, m - 32 * w));
-                    alive[w] = bits == 32 ? 0xffffffffu : ((1u << bits) - 1u);
-                }
-#pragma unroll
-                for (int w = 0; w < 4; ++w) {
-                    unsigned nzw = s_nz[c][w];
-                    while (nzw) {
-                        const int b = __ffs(nzw) - 1;
-                        nzw &= nzw - 1;
-                        if ((alive[w] >> b) & 1u) {
-                            const uint4 rw = rows4[w * 32 + b];
-                            alive[0] &= ~rw.x; alive[1] &= ~rw.y; alive[2] &= ~rw.z; alive[3] &= ~rw.w;
+                    for (int k = 0; k < 4; ++k) {
+                        const unsigned sb = __float_as_uint(sc[k]);
+                        if (((open[k] >> lane) & 1u) && (bp < 0 || sb > best)) {
+                            best = sb;
+                            bp = lane + 32 * k;
                         }
                     }
-                }
-                int kc = __popc(alive[0]) + __popc(alive[1]) + __popc(alive[2]) + __popc(alive[3]);
-                while (kc > K) {  // only the first K survivors of a class can reach the output
+                    const unsigned top = __reduce_max_sync(FULL, bp >= 0 ? best : 0u);
+                    const int w = (int)__reduce_min_sync(FULL, (bp >= 0 && best == top) ? (unsigned)bp : 0xffffffffu);
 #pragma unroll
-                    for (int w = 3; w >= 0; --w)
-                        if (alive[w]) {
-                            alive[w] &= ~(0x80000000u >> __clz(alive[w]));
-                            break;
+                    for (int k = 0; k < 4; ++k)  // (a constant index keeps the masks in registers)
+                        if (k == (w >> 5)) open[k] &= ~(1u << (w & 31));
+                    const uint4 ew = s_edge[w];
+                    const float4 bw = class_box(w);
+                    const float aw = box_area(bw);
+#pragma unroll
+                    for (int k = 0; k < 4; ++k) {
+                        const unsigned ek = (k == 0 ? ew.x : k == 1 ? ew.y : k == 2 ? ew.z : ew.w) & open[k];
+                        bool dead = false;
+                        if ((ek >> lane) & 1u) {
+                            const float4 bb = class_box(lane + 32 * k);
+                            dead = nonan ? nms_suppresses<true>(bw, aw, bb, box_area(bb), thr_f)
+                                         : nms_suppresses<false>(bw, aw, bb, box_area(bb), thr_f);
                         }
+                        const unsigned dm = __ballot_sync(FULL, dead);
+                        open[k] &= ~dm;
+                        kept[k] &= ~dm;
+                    }
+                }
+                int kc = __popc(kept[0]) + __popc(kept[1]) + __popc(kept[2]) + __popc(kept[3]);
+                while (kc > K) {  // only the first K survivors of a class can reach the output: drop the last one
+                    unsigned worst = 0u;
+                    int wp = -1;
+#pragma unroll
+                    for (int k = 0; k < 4; ++k) {
+                        const unsigned sb = __float_as_uint(sc[k]);
+                        if (((kept[k] >> lane) & 1u) && (wp < 0 || sb <= worst)) {
+                            worst = sb;
+                            wp = lane + 32 * k;
+                        }
+                    }
+                    const unsigned low = __reduce_min_sync(FULL, wp >= 0 ? worst : 0xffffffffu);
+                    const int w = (int)__reduce_max_sync(FULL, (wp >= 0 && worst == low) ? (unsigned)wp : 0u);
+#pragma unroll
+                    for (int k = 0; k < 4; ++k)
+                        if (k == (w >> 5)) kept[k] &= ~(1u << (w & 31));
                     --kc;
                 }
                 // ---- G: the lane's kept keys (descending-score bits | predictor * C + class) and their histogram
 #pragma unroll
-                for (int w = 0; w < 4; ++w) {
-                    if ((alive[w] >> lane) & 1u) {
-                        const int i = lane + 32 * w;
-                        const unsigned sb = skey[i];
-                        mine_kept[w] = true;
-                        mykey[w] = ((uint64_t)(~sb) << 32) | (uint64_t)((unsigned)spred[i] * (unsigned)C + (unsigned)c);
+                for (int k = 0; k < 4; ++k) {
+                    if ((kept[k] >> lane) & 1u) {
+                        const unsigned sb = __float_as_uint(sc[k]);
+                        mine_kept[k] = true;
+                        mykey[k] = ((uint64_t)(~sb) << 32) | (uint64_t)((unsigned)(lane + 32 * k) * (unsigned)C + (unsigned)c);
                         atomicAdd(&s_hist2[score_bin(sb, base2, shift2)], 1);
                     }
                 }
                 if (lane == 0 && kc) atomicAdd(&s_total, kc);
                 DET_MARK(8);
             }
-            __syncthreads();  // every class is done with its scratch: the merge buffers may now overwrite it
+            __syncthreads();  // every class has emitted its kept keys
             if (tier == 2 || s_total >= K) break;  // enough: the first K kept detections all lie above this cut
             __syncthreads();                       // heavy suppression: redo on every candidate
             for (int i = tid; i < kFastBins; i += T) s_hist2[i] = 0;

@@ -23,9 +23,9 @@ for i in range(4):
 torch.cuda.synchronize()
 buf = (ctypes.c_longlong * 32)()
 assert N.lib().det_debug_read_phases(buf) == 0
-names = {0: "start", 1: "A staged+decoded", 2: "B scores/stats/tier", 5: "C compaction (class 0)", 6: "D rank sort", 7: "E pair tests",
-         8: "F/G resolve", 3: "all classes done", 4: "counting-sort merge", 15: "output"}
-order = [0, 1, 2, 5, 6, 7, 8, 3, 4, 15]
+names = {0: "start", 1: "A staged+decoded", 2: "B scores/stats/tier", 5: "E pair filter", 8: "R resolve (class 0)",
+         3: "all classes done", 4: "counting-sort merge", 15: "output"}
+order = [0, 1, 2, 5, 8, 3, 4, 15]
 prev = buf[0]
 for i in order:
     if buf[i]:
